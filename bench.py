@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- BASELINE.json's metric (input GB/s + tokens/s of batch encode) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2b|c2a|c3|c4a|c4b|c5a|c5b] [--size-mib M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2b|c2a|c3|c4a|c4b|c5a|c5b] [--size-mib M] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      the reference's algorithm (C restatement, oracle/) on the host cores
 
@@ -42,6 +42,13 @@ WORKLOADS = {
 }
 DEFAULT_MIB = {"c2b": 1024, "c2a": 1024, "c3": 1600, "c4b": 2048, "c4a": 2048, "c5b": 1024, "c5a": 256}
 VERIFY_MIB = 64           # per workload: the GPU encoding of this much text is compared with the oracle, every array
+DUMP_BYTES = 60 << 20     # --dump-outputs: all sampled arrays of one step together, float64 (under 64 MB with the .npy headers)
+DUMP_DOC_ROWS = 1 << 18   # CSR entries (doc_tok_off) of the sample; the token slots share what the CSR and wide rows leave
+DUMP_WIDE_ROWS = 1 << 16  # wide-offset records (only with packed offsets)
+DUMP_SEED = 1234
+# per-token-slot arrays of tkz_batch_result: (field, values per slot, element type as the C ABI writes it)
+SLOT_ARRAYS = (("ids", 1, "u4"), ("ids16", 1, "u2"), ("offsets", 2, "u4"), ("offsets_packed", 1, "u2"), ("attention_mask", 1, "u4"),
+               ("type_ids", 1, "u4"), ("special_tokens_mask", 1, "u4"), ("span_tokens", 4, "u4"))
 
 
 def env_int(k, d):
@@ -195,6 +202,75 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+class DeviceArray:
+    """A (rows, cols) array the C ABI returned in device memory, seen by torch.as_tensor without a copy (CUDA array interface).
+    It is typed as the signed integer of the same width: torch gathers no unsigned type wider than a byte."""
+
+    def __init__(self, ptr, rows, cols, utype):
+        self.__cuda_array_interface__ = {"shape": (rows, cols), "typestr": "<" + utype.replace("u", "i"), "data": (ptr, False), "version": 3}
+
+
+class OutputSample:
+    """--dump-outputs: a fixed, seeded sample of what the timed path hands its caller in its last step, i.e. the device result of
+    every sub-batch, read right after its call because the next call on the context reuses the buffers.  Written as
+    DIR/<name>.npy in float64: one file per array of tkz_batch_result, and slot_rows / doc_rows / wide_rows holding the row
+    numbers of the sample counted over the whole step (doc_tok_off is made step-wide the same way).  A shard no larger than
+    the budget is written whole."""
+
+    def __init__(self, n_batches, stream):
+        self.n_batches, self.stream = n_batches, stream
+        self.parts = {}
+        self.slot0 = self.wide0 = 0
+        self.ms = 0.0                  # device-timeline time spent here; the caller takes it out of the timed window
+
+    @staticmethod
+    def pick(rng, n, k):
+        return np.arange(n, dtype=np.int64) if n <= k else np.unique(rng.integers(0, n, size=k))
+
+    @staticmethod
+    def gather(ptr, n, cols, utype, rows):
+        import torch
+        if len(rows) == 0:
+            return np.zeros((0, cols) if cols > 1 else 0)
+        t = torch.as_tensor(DeviceArray(ptr, n, cols, utype))
+        v = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy().view("<" + utype).astype(np.float64)
+        return v if cols > 1 else v.ravel()
+
+    def add(self, r, i, doc0):
+        """sub-batch i of the step, whose first document is doc0 of the shard"""
+        import torch
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(self.stream)
+        rng = np.random.default_rng([DUMP_SEED, i])
+        nt, nd = int(r.n_tokens), int(r.n_docs)
+        slot = [(f, c, u) for f, c, u in SLOT_ARRAYS if getattr(r, f)]
+        k = (DUMP_BYTES - 16 * DUMP_DOC_ROWS - 40 * DUMP_WIDE_ROWS) // (8 * (1 + sum(c for _, c, _ in slot))) // self.n_batches
+        rows = self.pick(rng, nt, k)
+        out = {"slot_rows": rows + self.slot0}
+        for f, c, u in slot:
+            out[f] = self.gather(getattr(r, f), nt, c, u, rows)
+        # a sub-batch's closing CSR entry is the next one's first: only the last sub-batch contributes it
+        rows = self.pick(rng, nd + (i == self.n_batches - 1), DUMP_DOC_ROWS // self.n_batches)
+        out["doc_rows"] = rows + doc0
+        out["doc_tok_off"] = self.gather(r.doc_tok_off, nd + 1, 1, "u8", rows) + self.slot0
+        if r.wide_tokens and r.n_wide:
+            rows = self.pick(rng, int(r.n_wide), DUMP_WIDE_ROWS // self.n_batches)
+            out["wide_rows"] = rows + self.wide0
+            out["wide_tokens"] = self.gather(r.wide_tokens, int(r.n_wide), 4, "u4", rows)
+            self.wide0 += int(r.n_wide)
+        self.slot0 += nt
+        for name, a in out.items():
+            self.parts.setdefault(name, []).append(np.asarray(a, dtype=np.float64))
+        e1.record(self.stream)
+        e1.synchronize()
+        self.ms += e0.elapsed_time(e1)
+
+    def save(self, out_dir):
+        os.makedirs(out_dir, exist_ok=True)
+        for name, parts in self.parts.items():
+            np.save(os.path.join(out_dir, name + ".npy"), np.concatenate(parts))
+
+
 class Work:
     """one workload on one rank: corpus in pinned host memory and in HBM, tokenizer, parameters"""
 
@@ -227,9 +303,9 @@ class Work:
         self.tok.close()
         del self.d_text, self.d_offs
 
-    def device_step(self, params, collect=None):
+    def device_step(self, params, collect=None, sink=None):
         tot_tokens = tot_real = 0
-        for (a, b), doff in zip(self.batches, self.d_offs):
+        for i, ((a, b), doff) in enumerate(zip(self.batches, self.d_offs)):
             r = self.tz.BatchResult()
             base = int(self.off[a]); nb = int(self.off[b]) - base
             rc = self.L.tkz_encode_batch_device(self.ctx, C.c_void_p(self.d_text.data_ptr() + base), C.c_void_p(doff.data_ptr()), b - a, nb, C.byref(params), C.byref(r))
@@ -241,12 +317,15 @@ class Work:
                 s = self.stats
                 collect["launches"] += s.kernel_launches; collect["words"] += s.n_words
                 collect["uniq"] = int(s.n_unique_words); collect["long"] = int(s.n_long_words); collect["path"] = int(s.path)
-                for i, k in enumerate(("ms_split", "ms_model", "ms_scan", "ms_emit", "ms_total")):
-                    collect["ms"][i] += getattr(s, k)
+                for j, k in enumerate(("ms_split", "ms_model", "ms_scan", "ms_emit", "ms_total")):
+                    collect["ms"][j] += getattr(s, k)
+            if sink is not None:
+                sink.add(r, i, a)
         return tot_tokens, tot_real
 
-    def time_device(self, outputs, steps, warmup, stream, barrier, params=None):
-        """K steps with everything resident in HBM; returns local ms per step and the counters of the steps"""
+    def time_device(self, outputs, steps, warmup, stream, barrier, params=None, sink=None):
+        """K steps with everything resident in HBM; returns local ms per step and the counters of the steps.  `sink` (an
+        OutputSample) reads the results of the last step; the time it takes is not counted."""
         torch = self.torch
         if params is None:
             params = self.tok.params(outputs)
@@ -256,13 +335,13 @@ class Work:
         barrier(); torch.cuda.synchronize()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record(stream)
-        for _ in range(steps):
+        for s in range(steps):
             agg["words"] = 0
-            tokens, real = self.device_step(params, collect=agg)
+            tokens, real = self.device_step(params, collect=agg, sink=sink if s == steps - 1 else None)
         ev1.record(stream)
         torch.cuda.synchronize(); barrier()
         agg["tokens"], agg["real"] = tokens, real
-        agg["ms_step"] = ev0.elapsed_time(ev1) / steps
+        agg["ms_step"] = (ev0.elapsed_time(ev1) - (sink.ms if sink else 0.0)) / steps
         agg["stage_ms"] = [x / steps for x in agg["ms"]]
         agg["launches_per_step"] = agg["launches"] / steps
         return agg
@@ -451,9 +530,12 @@ def run_ours(args, rank, local_rank, world):
         if headline:
             sampler = ClockSampler(local_rank)
             sampler.start()
-        agg = W.time_device(outputs, steps, warmup, stream, barrier)
+        sink = OutputSample(len(W.batches), stream) if headline and args.dump_outputs and rank == 0 else None
+        agg = W.time_device(outputs, steps, warmup, stream, barrier, sink=sink)
         if sampler:
             sampler.stop_flag.set()
+        if sink:
+            sink.save(args.dump_outputs)
         ms_step = allmax(agg["ms_step"])
         all_bytes, all_real, all_slots = allsum([W.nbytes, agg["real"], agg["tokens"]])
         out = {"value": all_bytes / (ms_step * 1e-3) / 1e9, "unit": "GB/s", "ms_per_step": ms_step, "steps": steps,
@@ -634,7 +716,13 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling / skew measurement (N > 1 only)")
     ap.add_argument("--strong-mib", type=int, default=4096, help="size of the fixed corpus of the strong-scaling measurement")
     ap.add_argument("--multi", type=int, default=0, help="single process: only the strong-scaling measurement over this many GPUs (tkzm_*)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the headline's timed steps, write a seeded sample (at most 64 MB, float64) "
+                    "of what its last step computed to DIR/<name>.npy (rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.multi > 0):
+        ap.error("--dump-outputs samples the device-resident headline; --impl reference and --multi have none")
     if args.size_mib <= 0:
         args.size_mib = DEFAULT_MIB[args.workload]
     if args.warmup < 3 and args.impl == "ours":
