@@ -67,7 +67,8 @@ def ascii_corpus(seed, n_docs, words, long_word_every=0):
 
 @pytest.mark.parametrize("si", [0, 2, 3])
 @pytest.mark.parametrize("trunc,pad", [(None, None), (32, {"length": 40, "pad_id": 0, "pad_type_id": 0, "direction": "right"}),
-                                       (20, {"length": 33, "pad_id": 1, "pad_type_id": 1, "direction": "left"})])
+                                       (20, {"length": 33, "pad_id": 1, "pad_type_id": 1, "direction": "left"}),
+                                       (None, {"length": 256, "pad_id": 1, "pad_type_id": 1, "direction": "left"})])   # (mostly padding: whole-array fill)
 @pytest.mark.parametrize("mode", MODES)
 def test_gpu_hf_mode_equals_oracle_on_random_corpora(si, trunc, pad, mode):
     suite = VEC["suites"][si]

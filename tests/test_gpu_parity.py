@@ -123,7 +123,7 @@ def test_wordpiece_random(seed):
     t.close()
 
 
-@pytest.mark.parametrize("seed", range(16))
+@pytest.mark.parametrize("seed", range(24))
 def test_truncation_and_padding(seed):
     rng = random.Random(900 + seed)
     if seed % 2:
@@ -135,6 +135,8 @@ def test_truncation_and_padding(seed):
     trunc = [None, 0, 1, 5, 8, 64][seed % 6]
     pad = [None, {"length": 8, "pad_id": 7, "pad_type_id": 3, "direction": "right"}, {"length": 5, "pad_id": 0, "direction": "left"},
            {"length": None, "pad_id": 9}][(seed // 2) % 4]
+    if seed >= 16:      # mostly padding: the whole-array fill, in the per-occurrence pipeline at seeds 19 and 23
+        pad = {"length": 256, "pad_id": 4, "pad_type_id": 2, "direction": "left"}
     t.truncation = None if trunc is None else {"max_length": trunc}
     o.truncation = trunc
     t.padding = pad

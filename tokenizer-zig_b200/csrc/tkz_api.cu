@@ -1,11 +1,11 @@
 // tkz_api.cu -- device layer of the C ABI (include/tokzig_b200.h): context, device arenas, model upload, and the
-// batch-encode pipeline that replaces the caller loop over Tokenizer.encode (src/lib.zig:109-160):
+// batch-encode pipelines that replace the caller loop over Tokenizer.encode (src/lib.zig:109-160):
 //
 //   [K0 normalise-compact]  only when the normalizer drops bytes (struct BertNormalizer, normalizer.zig:47-73)
-//   K1 split                byte-class scan -> pre-token spans            (config.zig:364-457, pretokenizer.zig:49-241)
-//   K3 bpe / K4 wordpiece   one warp per pre-token -> tokens in the pool  (bpe.zig:173-263 / wordpiece.zig:141-222)
-//   scans                   tokens per word -> per document -> CSR offsets
-//   K5 emit                 fromTokens + truncate + pad fused in the write (encoding.zig:246-294, 363-463)
+//   encode_slices           any model with a pre-tokenizer: pass A tokenizes 1 KiB slices, pass B writes (tkz_slices.cuh)
+//   encode_words            per-occurrence: K1 pre-token spans (pretokenizer.zig:49-241), K3 bpe / K4 wordpiece per
+//                           pre-token (bpe.zig:173-263 / wordpiece.zig:141-222), scans to CSR offsets, K5 emit
+//   shared epilogue         output arrays, padding + template tokens, stage times, result (encoding.zig:246-294, 363-463)
 //
 // There is no CPU fallback: without a usable CUDA device every entry point fails with TKZ_ERR_CUDA.
 #include <cstdio>
@@ -85,7 +85,6 @@ struct tkz_ctx {
     bool kept_valid = false;              // the table of the previous chunk can be reused
     uint64_t call_bytes = 0;              // text bytes of the whole call (sizes the shared table)
     uint32_t kept_tcap = 0, kept_upool_count = 0; uint64_t kept_upool_cap = 0, call_uniq = 0;
-    bool pad_fill = true;                 // TKZ_PAD_FILL=0: padding slots always by one warp per document (A/B switch)
     bool force_lut = false;               // TKZ_CLASSIFY=lut: per-byte look-up even when the class table fits ranges (A/B switch)
     DevBuf a_huge_w, a_huge_base, a_huge_done, a_grid_state, a_grid_words;   // bpe_grid_kernel (tkz_bpe_grid.cuh)
     bool use_grid = true;                 // TKZ_NO_GRID=1: huge words stay with one block each (A/B switch of the parity tests)
@@ -174,10 +173,10 @@ uint32_t pow2_at_least(uint64_t n) { uint32_t c = 2; while (c < n) c <<= 1; retu
 
 __global__ void ctrl_reset_kernel(unsigned long long* ctrl) {
     // ctrl[0] = error word, ctrl[1] = work counter (u32 view), ctrl[2..4] = read-back scalars,
-    // dedup: ctrl[5] second work counter, [6] n_uniq, [7] n_long, [8] overflow, [9] upool_count, [10] n_words
+    // [11..12], [17], [20..21] block-kernel work counters, [13..15] long-word length classes, [18..19] huge-word list (count, bytes)
     // slice pipeline: [5] entry count, [6] n_uniq | n_uncached << 32, [7] n_long, [8] abort, [9] upool | lscratch << 32,
-    //                [10] n_words, [11..12], [17], [20..21] block-kernel work counters, [13..15] long-word length classes,
-    //                [16] big-copy list, [18..19] huge-word list (count, bytes), [22] tokens of the long words, [23] wide-offset list
+    //                [10] n_words, [16] big-copy list, [22] tokens of the long words, [23] wide-offset list
+    // per-occurrence pipeline: high half of [9] big-copy list
     ctrl[0] = TKZ_ERRW_NONE;
     for (int i = 1; i < 32; i++) ctrl[i] = 0;
 }
@@ -276,7 +275,6 @@ extern "C" int tkz_ctx_create(int device, void* stream, uint64_t arena_hint_byte
     if (const char* e = getenv("TKZ_NO_DEDUP")) ctx->use_dedup = !(e[0] == '1');     // A/B switch for the parity tests
     if (const char* e = getenv("TKZ_CLASSIFY")) ctx->force_lut = (e[0] == 'l');
     if (const char* e = getenv("TKZ_STAGE")) ctx->stage_bulk = !(e[0] == 'l');
-    if (const char* e = getenv("TKZ_PAD_FILL")) ctx->pad_fill = e[0] != '0';
     if (const char* e = getenv("TKZ_KEEP_TABLE")) ctx->keep_table = e[0] != '0';
     if (const char* e = getenv("TKZ_NO_GRID")) ctx->use_grid = !(e[0] == '1');
     if (const char* e = getenv("TKZ_GRID_MIN_LEN")) { const long long v = atoll(e); if (v > (long long)BB_WARP_MAX) ctx->grid_min_len = (uint32_t)v; }
@@ -689,13 +687,105 @@ int launch_bpe(tkz_ctx* ctx, const DevModel& m, const uint8_t* d_text, const uin
     return TKZ_OK;
 }
 
-// hf_compat fields of the emit parameters (tkz_encode_params.hf_flags / tpl_*; validated in encode_device_impl)
-void emit_params_hf(EmitParams& ep, const tkz_encode_params& P) {
-    if (!P.hf_flags) return;
-    ep.hf_flags = P.hf_flags; ep.n_pre = P.tpl_n_prefix; ep.n_suf = P.tpl_n_suffix; ep.seq_type = P.tpl_seq_type;
-    for (uint32_t i = 0; i < TKZ_TPL_MAX; i++) {
-        ep.pre_id[i] = P.tpl_prefix_id[i]; ep.pre_type[i] = P.tpl_prefix_type[i]; ep.suf_id[i] = P.tpl_suffix_id[i]; ep.suf_type[i] = P.tpl_suffix_type[i];
+// ---- epilogue of both device pipelines: everything after each document's token count is known
+
+// (hf_compat fields from tkz_encode_params.hf_flags / tpl_*, validated in encode_device_impl)
+EmitParams emit_params(const tkz_encode_params& P) {
+    EmitParams ep{P.has_truncation, P.max_length, P.has_padding, P.pad_length, P.pad_id, P.pad_type_id, P.pad_left, P.outputs};
+    if (P.hf_flags) {
+        ep.hf_flags = P.hf_flags; ep.n_pre = P.tpl_n_prefix; ep.n_suf = P.tpl_n_suffix; ep.seq_type = P.tpl_seq_type;
+        for (uint32_t i = 0; i < TKZ_TPL_MAX; i++) {
+            ep.pre_id[i] = P.tpl_prefix_id[i]; ep.pre_type[i] = P.tpl_prefix_type[i]; ep.suf_id[i] = P.tpl_suffix_id[i]; ep.suf_type[i] = P.tpl_suffix_type[i];
+        }
     }
+    return ep;
+}
+bool has_frame(const EmitParams& ep) { return (ep.hf_flags & 1u) && ep.n_pre + ep.n_suf; }   // hf_compat: the template's special tokens
+
+// the output arrays of T slots that ep.outputs asks for, and the wide-offset side list, in the context's current output set
+int alloc_outputs(tkz_ctx* ctx, const EmitParams& ep, uint64_t T, uint32_t wide_cap, EmitOut& eo) {
+    auto& O = ctx->O();
+    const uint32_t o = ep.outputs;
+    if (o & TKZ_OUT_IDS_U16) TRY(ensure(ctx, O.ids16, (T + 4) * 2)); else TRY(ensure(ctx, O.ids, (T + 4) * 4));
+    if (o & TKZ_OUT_OFFSETS) TRY(ensure(ctx, O.off, (T + 4) * 8));
+    if (o & TKZ_OUT_ATTENTION) TRY(ensure(ctx, O.attn, (T + 4) * 4));
+    if (o & TKZ_OUT_TYPE_IDS) TRY(ensure(ctx, O.type, (T + 4) * 4));
+    if (o & TKZ_OUT_SPECIAL) TRY(ensure(ctx, O.special, (T + 4) * 4));
+    if (o & TKZ_OUT_OFFSETS_PACKED) TRY(ensure(ctx, O.off16, (T + 4) * 2));
+    if (o & TKZ_OUT_SPAN_TOKENS) TRY(ensure(ctx, O.spans, (T + 4) * 16));
+    if (wide_cap) TRY(ensure(ctx, O.wide, (size_t)wide_cap * 16));
+    eo = EmitOut{(uint32_t*)O.ids.p, (uint32_t*)O.off.p, (uint32_t*)O.attn.p, (uint32_t*)O.type.p, (uint32_t*)O.special.p, (uint16_t*)O.off16.p,
+                 (uint16_t*)O.ids16.p, (uint4*)O.spans.p, (uint4*)O.wide.p, (unsigned int*)((unsigned long long*)ctx->a_ctrl.p + 23), wide_cap};
+    return TKZ_OK;
+}
+
+// before the real tokens are written.  Mostly padding (pad to 512 around a few dozen tokens): every array is filled with its
+// padding value at streaming-store speed and the real tokens overwrite it; else pad_epilogue writes each document's gaps.
+// Returns whether the arrays were filled.
+bool pad_prologue(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, uint32_t nd, uint64_t T, uint64_t T_real, uint64_t& launches) {
+    if (!ep.has_pad || !nd || T < 2 * T_real) return false;
+    const unsigned fg = (unsigned)ctx->sm_count * 8;
+    auto fill = [&](void* p, uint64_t bytes, uint4 v) { fill16_kernel<<<fg, 256, 0, ctx->stream>>>((uint4*)p, bytes, v); launches++; };
+    auto rep = [](uint32_t x) { return make_uint4(x, x, x, x); };
+    const uint32_t o = ep.outputs;
+    if (o & TKZ_OUT_IDS_U16) fill(eo.ids16, T * 2, rep(ep.pad_id | (ep.pad_id << 16))); else fill(eo.ids, T * 4, rep(ep.pad_id));
+    if (o & TKZ_OUT_OFFSETS) fill(eo.offsets, T * 8, rep(0u));
+    if (o & TKZ_OUT_ATTENTION) fill(eo.attention, T * 4, rep(0u));
+    if (o & TKZ_OUT_TYPE_IDS) fill(eo.type_ids, T * 4, rep(ep.pad_type_id));
+    if (o & TKZ_OUT_SPECIAL) fill(eo.special, T * 4, rep(1u));
+    if (o & TKZ_OUT_OFFSETS_PACKED) fill(eo.offsets16, T * 2, rep(0u));
+    if (o & TKZ_OUT_SPAN_TOKENS) fill(eo.spans, T * 16, make_uint4(ep.pad_id, 0u, 0u, 0x0400u));
+    return true;
+}
+
+// after the real tokens are written: the template's special tokens, and the padding slots unless pad_prologue filled them
+// (doc_real: real tokens per document)
+void pad_epilogue(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, uint32_t nd, const uint32_t* doc_real, const unsigned long long* doc_tok_off,
+                  bool filled, uint64_t& launches) {
+    if (!nd) return;
+    if (ep.has_pad && !filled) {
+        emit_pad_real_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off); launches++;
+    } else if (has_frame(ep)) {
+        emit_frame_kernel<<<(nd + 255) / 256, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off); launches++;
+    }
+}
+
+// the eight per-token arrays of a result in TKZ_OUT_* bit order (ids, offsets, attention, type ids, special, packed offsets,
+// ids16, span tokens), nullptr where not delivered
+using ResultArrays = std::array<const void*, 8>;
+void set_result(tkz_batch_result* out, uint64_t n_docs, uint64_t T, uint64_t T_real, const uint64_t* doc_tok_off, const ResultArrays& a,
+                uint64_t n_wide, const void* wide) {
+    out->n_docs = n_docs; out->n_tokens = T; out->n_real_tokens = T_real;
+    out->doc_tok_off = doc_tok_off;
+    out->ids = (const uint32_t*)a[0]; out->offsets = (const uint32_t*)a[1]; out->attention_mask = (const uint32_t*)a[2];
+    out->type_ids = (const uint32_t*)a[3]; out->special_tokens_mask = (const uint32_t*)a[4]; out->offsets_packed = (const uint16_t*)a[5];
+    out->ids16 = (const uint16_t*)a[6]; out->span_tokens = (const uint32_t*)a[7];
+    out->n_wide = n_wide; out->wide_tokens = n_wide ? (const uint32_t*)wide : nullptr;
+}
+
+// device-resident result of an encode, its launch count and its stage times (events ev[0..4])
+void finish(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, const unsigned long long* doc_tok_off, uint64_t n_docs, uint64_t T, uint64_t T_real,
+            uint64_t n_wide, uint64_t launches, tkz_batch_result* out) {
+    ctx->stats.kernel_launches = launches;
+    cudaEventElapsedTime(&ctx->stats.ms_split, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&ctx->stats.ms_model, ctx->ev[1], ctx->ev[2]);
+    cudaEventElapsedTime(&ctx->stats.ms_scan, ctx->ev[2], ctx->ev[3]);
+    cudaEventElapsedTime(&ctx->stats.ms_emit, ctx->ev[3], ctx->ev[4]);
+    cudaEventElapsedTime(&ctx->stats.ms_total, ctx->ev[0], ctx->ev[4]);
+    const uint32_t o = ep.outputs;
+    ResultArrays a = {eo.ids, eo.offsets, eo.attention, eo.type_ids, eo.special, eo.offsets16, eo.ids16, eo.spans};
+    for (uint32_t i = 0; i < 8; i++) if (!(o & (1u << i))) a[i] = nullptr;
+    if (o & TKZ_OUT_IDS_U16) a[0] = nullptr;                          // exactly one of ids / ids16
+    set_result(out, n_docs, T, T_real, (const uint64_t*)doc_tok_off, a, n_wide, eo.wide);
+}
+
+// a failed word: its document to err_doc, the message and the return code of the error word's code
+int report_error(tkz_ctx* ctx, unsigned long long errw, uint64_t err_doc, uint64_t launches, tkz_batch_result* out) {
+    out->err_doc = (int64_t)err_doc;
+    const uint32_t code = (uint32_t)(errw & 0xFF);
+    ctx->err = code == TKZ_ECODE_UTF8 ? "invalid UTF-8 in a BPE pre-token (reference behaviour undefined)" : "MissingUnkToken";
+    ctx->stats.kernel_launches = launches;
+    return code == TKZ_ECODE_UTF8 ? TKZ_ERR_INVALID_UTF8 : TKZ_ERR_MISSING_UNK;
 }
 
 // The slice pipeline (tkz_slices.cuh).  Capacities that depend on the text (token stream, record pool, word table) are
@@ -835,8 +925,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     CK(cudaEventRecord(ctx->ev[2], st));
 
     // ---- tokens per tile -> token base per tile; CSR offsets
-    EmitParams ep{P.has_truncation, P.max_length, P.has_padding, P.pad_length, P.pad_id, P.pad_type_id, P.pad_left, P.outputs};
-    emit_params_hf(ep, P);
+    EmitParams ep = emit_params(P);
     launches += exclusive_scan<uint32_t>(ta.slice_ntok, n_slices, ta.slice_ntok, (unsigned long long*)ctx->a_scan_tmp.p, st);
     unsigned long long* doc_tok_off = (unsigned long long*)ctx->O().doc_tok_off.p;
     if (!plain) {
@@ -860,31 +949,18 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
         if (lt > T_real / 8 + 4096 || lt > (4u << 20)) { P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS; ep.outputs = P.outputs; }
         else wide_cap = (uint32_t)lt;
     }
-    auto fail = [&](unsigned long long errw) -> int {
+    auto fail = [&]() -> int {        // (the error word holds a byte position)
         err_doc_kernel<<<1, 1, 0, st>>>(ctrl, d_doc_off, nd); launches++;
         readback(ctx, hctrl + 4, ctrl + 4, 8);
         cudaStreamSynchronize(st);
-        out->err_doc = (int64_t)hctrl[4];
-        const uint32_t code = (uint32_t)(errw & 0xFF);
-        ctx->err = code == TKZ_ECODE_UTF8 ? "invalid UTF-8 in a BPE pre-token (reference behaviour undefined)" : "MissingUnkToken";
-        ctx->stats.kernel_launches = launches;
-        return code == TKZ_ECODE_UTF8 ? TKZ_ERR_INVALID_UTF8 : TKZ_ERR_MISSING_UNK;
+        return report_error(ctx, hctrl[0], hctrl[4], launches, out);
     };
-    if (hctrl[0] != TKZ_ERRW_NONE && n_long == 0) return fail(hctrl[0]);   // (errors of long words surface in pass B)
+    if (hctrl[0] != TKZ_ERRW_NONE && n_long == 0) return fail();   // (errors of long words surface in pass B)
     CK(cudaEventRecord(ctx->ev[3], st));
 
     // ---- pass B
-    if (P.outputs & TKZ_OUT_IDS_U16) TRY(ensure(ctx, ctx->O().ids16, (T + 4) * 2)); else TRY(ensure(ctx, ctx->O().ids, (T + 4) * 4));
-    if (P.outputs & TKZ_OUT_OFFSETS) TRY(ensure(ctx, ctx->O().off, (T + 4) * 8));
-    if (P.outputs & TKZ_OUT_ATTENTION) TRY(ensure(ctx, ctx->O().attn, (T + 4) * 4));
-    if (P.outputs & TKZ_OUT_TYPE_IDS) TRY(ensure(ctx, ctx->O().type, (T + 4) * 4));
-    if (P.outputs & TKZ_OUT_SPECIAL) TRY(ensure(ctx, ctx->O().special, (T + 4) * 4));
-    if (P.outputs & TKZ_OUT_OFFSETS_PACKED) TRY(ensure(ctx, ctx->O().off16, (T + 4) * 2));
-    if (P.outputs & TKZ_OUT_SPAN_TOKENS) TRY(ensure(ctx, ctx->O().spans, (T + 4) * 16));
-    if (wide_cap) TRY(ensure(ctx, ctx->O().wide, (size_t)wide_cap * 16));
-    EmitOut eo{(uint32_t*)ctx->O().ids.p, (uint32_t*)ctx->O().off.p, (uint32_t*)ctx->O().attn.p, (uint32_t*)ctx->O().type.p,
-               (uint32_t*)ctx->O().special.p, (uint16_t*)ctx->O().off16.p, (uint16_t*)ctx->O().ids16.p, (uint4*)ctx->O().spans.p,
-               (uint4*)ctx->O().wide.p, (unsigned int*)(ctrl + 23), wide_cap};
+    EmitOut eo;
+    TRY(alloc_outputs(ctx, ep, T, wide_cap, eo));
     const uint32_t big_cap = (uint32_t)(N / EMIT_BIG + 16);
     TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
     SliceEmitArgs ea{};
@@ -896,58 +972,147 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ea.doc_tok_local = ta.doc_tok_local; ea.doc_tok_start = (const uint32_t*)ctx->a_doc_tok_start.p;
     ea.doc_tok_off = doc_tok_off; ea.errw = ctrl; ea.err_code = m.kind == TKZ_MODEL_BPE ? TKZ_ECODE_UTF8 : TKZ_ECODE_UNK;
     ea.big = BigList{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 16), big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
-    // mostly padding (pad to 512 around a few dozen tokens): fill every array with its padding value first, at streaming-store
-    // speed, and let pass B overwrite the real tokens; else one warp per document fills the gaps afterwards
-    const bool pad_fill = P.has_padding && nd && ctx->pad_fill && T >= 2 * T_real;
-    if (pad_fill) {
-        const unsigned fg = (unsigned)ctx->sm_count * 8;
-        auto fill = [&](void* p, uint64_t bytes, uint4 v) { fill16_kernel<<<fg, 256, 0, st>>>((uint4*)p, bytes, v); launches++; };
-        auto rep = [](uint32_t x) { return make_uint4(x, x, x, x); };
-        if (P.outputs & TKZ_OUT_IDS_U16) fill(eo.ids16, T * 2, rep(P.pad_id | (P.pad_id << 16))); else fill(eo.ids, T * 4, rep(P.pad_id));
-        if (P.outputs & TKZ_OUT_OFFSETS) fill(eo.offsets, T * 8, rep(0u));
-        if (P.outputs & TKZ_OUT_ATTENTION) fill(eo.attention, T * 4, rep(0u));
-        if (P.outputs & TKZ_OUT_TYPE_IDS) fill(eo.type_ids, T * 4, rep(P.pad_type_id));
-        if (P.outputs & TKZ_OUT_SPECIAL) fill(eo.special, T * 4, rep(1u));
-        if (P.outputs & TKZ_OUT_OFFSETS_PACKED) fill(eo.offsets16, T * 2, rep(0u));
-        if (P.outputs & TKZ_OUT_SPAN_TOKENS) fill(eo.spans, T * 16, make_uint4(P.pad_id, 0u, 0u, 0x0400u));
-    }
+    const bool filled = pad_prologue(ctx, ep, eo, nd, T, T_real, launches);
     const uint32_t egrid = (uint32_t)std::min<uint64_t>(((uint64_t)n_slices + TW_WARPS - 1) / TW_WARPS, (uint64_t)ctx->sm_count * 16);
     if (plain) launch_slice_emit<true>(ea, ep, eo, egrid, st);
     else launch_slice_emit<false>(ea, ep, eo, egrid, st);
     launches++;
     if (n_long) { emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, ea.big, ea.pool_id, ea.pool_s, ea.pool_e); launches++; }
-    const bool frame = (ep.hf_flags & 1u) && ep.n_pre + ep.n_suf;                     // hf_compat: the template's special tokens
-    if (frame && !(P.has_padding && !pad_fill) && nd) {
-        emit_frame_kernel<<<(nd + 255) / 256, 256, 0, st>>>(ep, eo, nd, (const uint32_t*)ctx->a_doc_real.p, doc_tok_off); launches++;
-    } else if (P.has_padding && !pad_fill && nd) {
-        emit_pad_real_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, st>>>(ep, eo, nd, (const uint32_t*)ctx->a_doc_real.p, doc_tok_off, true); launches++;
-    }
+    pad_epilogue(ctx, ep, eo, nd, (const uint32_t*)ctx->a_doc_real.p, doc_tok_off, filled, launches);
     CK(cudaGetLastError());
     CK(cudaEventRecord(ctx->ev[4], st));
     TRY(readback(ctx, hctrl, ctrl, 11 * 8));
     if (wide_cap) TRY(readback(ctx, hctrl + 23, ctrl + 23, 8));
     CK(cudaStreamSynchronize(st));
-    if (hctrl[0] != TKZ_ERRW_NONE) return fail(hctrl[0]);
+    if (hctrl[0] != TKZ_ERRW_NONE) return fail();
     if (wide_cap && (uint32_t)hctrl[23] > wide_cap) { ctx->err = "internal: more wide offsets than tokens of long pre-tokens"; return TKZ_ERR_CUDA; }
     ctx->stats.n_words = hctrl[10];
     if (N) ctx->tw_tok_per_byte = std::max(ctx->tw_tok_per_byte, (double)T_real / (double)N);
-    ctx->stats.kernel_launches = launches;
-    cudaEventElapsedTime(&ctx->stats.ms_split, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&ctx->stats.ms_model, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&ctx->stats.ms_scan, ctx->ev[2], ctx->ev[3]);
-    cudaEventElapsedTime(&ctx->stats.ms_emit, ctx->ev[3], ctx->ev[4]);
-    cudaEventElapsedTime(&ctx->stats.ms_total, ctx->ev[0], ctx->ev[4]);
-    out->n_docs = n_docs; out->n_tokens = T; out->n_real_tokens = T_real;
-    out->doc_tok_off = (const uint64_t*)doc_tok_off;
-    out->ids = (P.outputs & TKZ_OUT_IDS_U16) ? nullptr : eo.ids;
-    out->ids16 = (P.outputs & TKZ_OUT_IDS_U16) ? eo.ids16 : nullptr;
-    out->offsets = (P.outputs & TKZ_OUT_OFFSETS) ? eo.offsets : nullptr;
-    out->attention_mask = (P.outputs & TKZ_OUT_ATTENTION) ? eo.attention : nullptr;
-    out->type_ids = (P.outputs & TKZ_OUT_TYPE_IDS) ? eo.type_ids : nullptr;
-    out->special_tokens_mask = (P.outputs & TKZ_OUT_SPECIAL) ? eo.special : nullptr;
-    out->offsets_packed = (P.outputs & TKZ_OUT_OFFSETS_PACKED) ? eo.offsets16 : nullptr;
-    out->n_wide = wide_cap ? (uint32_t)hctrl[23] : 0; out->wide_tokens = out->n_wide ? (const uint32_t*)eo.wide : nullptr;
-    out->span_tokens = (P.outputs & TKZ_OUT_SPAN_TOKENS) ? (const uint32_t*)eo.spans : nullptr;
+    finish(ctx, ep, eo, doc_tok_off, n_docs, T, T_real, wide_cap ? (uint32_t)hctrl[23] : 0, launches, out);
+    return TKZ_OK;
+}
+
+// The per-occurrence pipeline: models without a pre-tokenizer (every document is one pre-token), the FastTokenizer mode and
+// TKZ_NO_DEDUP=1.  K1 pre-token spans, K3 / K4 one warp (or block) per pre-token, scans to CSR offsets, K5 emit.
+int encode_words(tkz_ctx* ctx, const DevModel& m, const uint8_t* d_text, const uint64_t* d_doc_off, uint32_t nd, uint64_t N,
+                 tkz_encode_params P, tkz_batch_result* out, uint64_t& launches) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long* ctrl = (unsigned long long*)ctx->a_ctrl.p;
+    unsigned long long* hctrl = (unsigned long long*)ctx->h_ctrl.p;
+    const uint64_t n_docs = nd;
+    // a pre-token can have any length: offsets are delivered as 32-bit pairs
+    if (P.outputs & TKZ_OUT_OFFSETS_PACKED) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
+
+    // ---- K1: pre-token spans
+    uint64_t W = 0;
+    TRY(ensure(ctx, ctx->a_doc_word_off, (n_docs + 1) * 4));
+    uint32_t* doc_word_off = (uint32_t*)ctx->a_doc_word_off.p;
+    if (m.has_pretok) {
+        const uint64_t n_tiles = N / SPLIT_TILE + 1;
+        TRY(ensure(ctx, ctx->a_tiles, (n_tiles + 1) * 8));
+        TRY(ensure(ctx, ctx->a_scan_tmp, scan_tmp_elems(n_tiles) * 8));
+        unsigned long long* tiles = (unsigned long long*)ctx->a_tiles.p;
+        split_count_kernel<<<(unsigned)n_tiles, SPLIT_THREADS, 0, st>>>(m, d_text, N, d_doc_off, nd, tiles); launches++;
+        launches += exclusive_scan<unsigned long long>(tiles, n_tiles, tiles, (unsigned long long*)ctx->a_scan_tmp.p, st);
+        TRY(readback(ctx, hctrl + 8, tiles + n_tiles, 8));
+        CK(cudaStreamSynchronize(st));
+        const unsigned long long tot = hctrl[8];
+        W = tot >> 32;
+        if ((tot & 0xFFFFFFFFull) != W) { ctx->err = "internal: word start/end counts differ"; return TKZ_ERR_CUDA; }
+        TRY(ensure(ctx, ctx->a_word_start, (W + 1) * 4));
+        TRY(ensure(ctx, ctx->a_word_end, (W + 1) * 4));
+        TRY(ensure(ctx, ctx->a_word_doc, (W + 1) * 4));
+        split_write_kernel<<<(unsigned)n_tiles, SPLIT_THREADS, 0, st>>>(m, d_text, N, d_doc_off, nd, tiles, (uint32_t*)ctx->a_word_start.p,
+                                                                        (uint32_t*)ctx->a_word_end.p, (uint32_t*)ctx->a_word_doc.p, doc_word_off); launches++;
+    } else {
+        W = n_docs;
+        TRY(ensure(ctx, ctx->a_word_start, (W + 1) * 4));
+        TRY(ensure(ctx, ctx->a_word_end, (W + 1) * 4));
+        TRY(ensure(ctx, ctx->a_word_doc, (W + 1) * 4));
+        words_from_docs_kernel<<<(unsigned)((n_docs + 1 + 255) / 256), 256, 0, st>>>(d_doc_off, nd, (uint32_t*)ctx->a_word_start.p,
+                                                                                     (uint32_t*)ctx->a_word_end.p, (uint32_t*)ctx->a_word_doc.p, doc_word_off); launches++;
+    }
+    const uint32_t nw = (uint32_t)W;
+    uint32_t* word_start = (uint32_t*)ctx->a_word_start.p;
+    uint32_t* word_end = (uint32_t*)ctx->a_word_end.p;
+    uint32_t* word_doc = (uint32_t*)ctx->a_word_doc.p;
+
+    CK(cudaEventRecord(ctx->ev[1], st));
+    // ---- K3 / K4: model, one warp per pre-token
+    TRY(ensure(ctx, ctx->a_word_ntok, (W + 2) * 4));
+    TRY(ensure(ctx, ctx->a_pool_id, N * 4));
+    TRY(ensure(ctx, ctx->a_pool_s, N * 4));
+    TRY(ensure(ctx, ctx->a_pool_e, N * 4));
+    uint32_t* word_ntok = (uint32_t*)ctx->a_word_ntok.p;
+    unsigned int* work_counter = (unsigned int*)(ctrl + 1);
+    if (nw && P.fast) {
+        // FastTokenizer mode: one thread per pre-token replays tokenizeFast (tkz_fast.cuh)
+        TRY(ensure(ctx, ctx->a_pool_rk, N * 4));
+        TRY(ensure(ctx, ctx->a_fast_heap, N * 16 + 64));
+        TRY(ensure(ctx, ctx->a_word_aux, (W + 2) * 4));
+        FastArgs fa{d_text, word_start, word_end, word_doc, doc_word_off, nw, P.fast_max_sequence_length, P.fast_max_tokens,
+                    (uint32_t*)ctx->a_pool_id.p, (uint32_t*)ctx->a_pool_s.p, (uint32_t*)ctx->a_pool_e.p, (uint32_t*)ctx->a_pool_rk.p,
+                    (unsigned long long*)ctx->a_fast_heap.p, word_ntok, (uint32_t*)ctx->a_word_aux.p, ctrl};
+        if (m.kind == TKZ_MODEL_BPE) { fast_bpe_kernel<<<(nw + 127) / 128, 128, 0, st>>>(m, fa); launches++; }
+        else {
+            fast_wp_kernel<<<(nw + 127) / 128, 128, 0, st>>>(m, fa); launches++;
+            if (nd) { fast_wp_fix_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, st>>>(fa, nd); launches++; }
+        }
+    } else if (nw) {
+        if (m.kind == TKZ_MODEL_BPE) {
+            len_class_count_kernel<<<128, 256, 0, st>>>(word_start, word_end, nw, nullptr, ctrl + 13); launches++;
+            TRY(readback(ctx, hctrl + 24, ctrl + 13, 3 * 8));
+            CK(cudaStreamSynchronize(st));
+            TRY(launch_bpe(ctx, m, d_text, word_start, word_end, nw, word_ntok, ctrl, 1, 0, hctrl + 24, N, launches));
+        } else {
+            WpArgs a{d_text, word_start, word_end, nw, (uint32_t*)ctx->a_pool_id.p, (uint32_t*)ctx->a_pool_s.p, (uint32_t*)ctx->a_pool_e.p,
+                     word_ntok, work_counter, ctrl, 0};
+            uint64_t blocks = (W + WP_WARPS - 1) / WP_WARPS;
+            const uint64_t cap = (uint64_t)ctx->sm_count * 8;
+            if (blocks > cap) blocks = cap;
+            wordpiece_warp_kernel<<<(unsigned)blocks, WP_WARPS * 32, 0, st>>>(m, a); launches++;
+        }
+    }
+
+    CK(cudaEventRecord(ctx->ev[2], st));
+    // ---- scans: tokens per word -> per document -> CSR
+    TRY(ensure(ctx, ctx->a_scan_tmp, (scan_tmp_elems(W) + scan_tmp_elems(n_docs)) * 8));
+    launches += exclusive_scan<uint32_t>(word_ntok, W, word_ntok, (unsigned long long*)ctx->a_scan_tmp.p, st);
+    const uint32_t* word_tok_off = word_ntok;
+    TRY(ensure(ctx, ctx->O().doc_tok_off, (n_docs + 1) * 8));
+    unsigned long long* doc_tok_off = (unsigned long long*)ctx->O().doc_tok_off.p;
+    const EmitParams ep = emit_params(P);
+    uint32_t* doc_real = nullptr;                           // (only the padding / template kernels read it)
+    if (ep.has_pad || has_frame(ep)) { TRY(ensure(ctx, ctx->a_doc_real, (n_docs + 2) * 4)); doc_real = (uint32_t*)ctx->a_doc_real.p; }
+    if (nd) { doc_len_kernel<<<(nd + 255) / 256, 256, 0, st>>>(ep, word_tok_off, doc_word_off, nd, doc_tok_off, doc_real); launches++; }
+    launches += exclusive_scan<unsigned long long>(doc_tok_off, n_docs, doc_tok_off, (unsigned long long*)ctx->a_scan_tmp.p, st);
+    gather_scalars_kernel<<<1, 1, 0, st>>>(ctrl, word_tok_off, nw, doc_tok_off, nd, word_doc); launches++;
+    TRY(readback(ctx, hctrl, ctrl, 5 * 8));
+    CK(cudaStreamSynchronize(st));
+    const uint64_t T_real = hctrl[2], T = hctrl[3];
+    ctx->stats.n_words = W; ctx->stats.n_unique_words = W; ctx->stats.n_long_words = 0;
+    if (hctrl[0] != TKZ_ERRW_NONE) return report_error(ctx, hctrl[0], hctrl[4], launches, out);   // (the error word holds a word index)
+
+    CK(cudaEventRecord(ctx->ev[3], st));
+    // ---- K5: emit
+    EmitOut eo;
+    TRY(alloc_outputs(ctx, ep, T, 0, eo));
+    const bool filled = pad_prologue(ctx, ep, eo, nd, T, T_real, launches);
+    if (nw) {
+        const uint32_t big_cap = (uint32_t)(N / EMIT_BIG + 16);
+        TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
+        BigList bl{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 9) + 1, big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
+        emit_words_kernel<<<(nw + 255) / 256, 256, 0, st>>>(ep, eo, nw, word_start, word_doc, word_tok_off, doc_word_off, doc_tok_off,
+                                                            (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
+                                                            (const uint32_t*)ctx->a_pool_e.p, bl, d_doc_off); launches++;
+        emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, bl, (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
+                                                           (const uint32_t*)ctx->a_pool_e.p); launches++;
+    }
+    pad_epilogue(ctx, ep, eo, nd, doc_real, doc_tok_off, filled, launches);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->ev[4], st));
+    CK(cudaStreamSynchronize(st));
+    finish(ctx, ep, eo, doc_tok_off, n_docs, T, T_real, 0, launches, out);
     return TKZ_OK;
 }
 
@@ -1021,7 +1186,7 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
     }
 
     // ---- slice pipeline (tkz_slices.cuh) whenever there is a pre-tokenizer; TKZ_NO_DEDUP=1 keeps the per-occurrence
-    //      pipeline below for A/B tests
+    //      pipeline for A/B tests
     ctx->stats.path = 0;
     if (m.has_pretok && ctx->use_dedup && !P.fast) {
         const ClassRanges& cr = ctx->dm.norm_has_drop ? ctx->cr_post : ctx->cr;      // (K0 ran: the text is already normalised)
@@ -1031,148 +1196,7 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
         ctrl_reset_kernel<<<1, 1, 0, st>>>(ctrl); launches++;
         return encode_slices(ctx, m, cr, d_text, d_doc_off, nd, N, P, true, out, launches);
     }
-    // no pre-tokenizer: a pre-token can have any length, offsets are delivered as 32-bit pairs
-    if (P.outputs & TKZ_OUT_OFFSETS_PACKED) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
-
-    // ---- K1: pre-token spans
-    uint64_t W = 0;
-    TRY(ensure(ctx, ctx->a_doc_word_off, (n_docs + 1) * 4));
-    uint32_t* doc_word_off = (uint32_t*)ctx->a_doc_word_off.p;
-    if (m.has_pretok) {
-        const uint64_t n_tiles = N / SPLIT_TILE + 1;
-        TRY(ensure(ctx, ctx->a_tiles, (n_tiles + 1) * 8));
-        TRY(ensure(ctx, ctx->a_scan_tmp, scan_tmp_elems(n_tiles) * 8));
-        unsigned long long* tiles = (unsigned long long*)ctx->a_tiles.p;
-        split_count_kernel<<<(unsigned)n_tiles, SPLIT_THREADS, 0, st>>>(m, d_text, N, d_doc_off, nd, tiles); launches++;
-        launches += exclusive_scan<unsigned long long>(tiles, n_tiles, tiles, (unsigned long long*)ctx->a_scan_tmp.p, st);
-        TRY(readback(ctx, hctrl + 8, tiles + n_tiles, 8));
-        CK(cudaStreamSynchronize(st));
-        const unsigned long long tot = hctrl[8];
-        W = tot >> 32;
-        if ((tot & 0xFFFFFFFFull) != W) { ctx->err = "internal: word start/end counts differ"; return TKZ_ERR_CUDA; }
-        TRY(ensure(ctx, ctx->a_word_start, (W + 1) * 4));
-        TRY(ensure(ctx, ctx->a_word_end, (W + 1) * 4));
-        TRY(ensure(ctx, ctx->a_word_doc, (W + 1) * 4));
-        split_write_kernel<<<(unsigned)n_tiles, SPLIT_THREADS, 0, st>>>(m, d_text, N, d_doc_off, nd, tiles, (uint32_t*)ctx->a_word_start.p,
-                                                                        (uint32_t*)ctx->a_word_end.p, (uint32_t*)ctx->a_word_doc.p, doc_word_off); launches++;
-    } else {
-        W = n_docs;
-        TRY(ensure(ctx, ctx->a_word_start, (W + 1) * 4));
-        TRY(ensure(ctx, ctx->a_word_end, (W + 1) * 4));
-        TRY(ensure(ctx, ctx->a_word_doc, (W + 1) * 4));
-        words_from_docs_kernel<<<(unsigned)((n_docs + 1 + 255) / 256), 256, 0, st>>>(d_doc_off, nd, (uint32_t*)ctx->a_word_start.p,
-                                                                                     (uint32_t*)ctx->a_word_end.p, (uint32_t*)ctx->a_word_doc.p, doc_word_off); launches++;
-    }
-    const uint32_t nw = (uint32_t)W;
-    uint32_t* word_start = (uint32_t*)ctx->a_word_start.p;
-    uint32_t* word_end = (uint32_t*)ctx->a_word_end.p;
-    uint32_t* word_doc = (uint32_t*)ctx->a_word_doc.p;
-
-    CK(cudaEventRecord(ctx->ev[1], st));
-    // ---- K3 / K4: model, one warp per pre-token
-    TRY(ensure(ctx, ctx->a_word_ntok, (W + 2) * 4));
-    TRY(ensure(ctx, ctx->a_pool_id, N * 4));
-    TRY(ensure(ctx, ctx->a_pool_s, N * 4));
-    TRY(ensure(ctx, ctx->a_pool_e, N * 4));
-    uint32_t* word_ntok = (uint32_t*)ctx->a_word_ntok.p;
-    unsigned int* work_counter = (unsigned int*)(ctrl + 1);
-    if (nw && P.fast) {
-        // FastTokenizer mode: one thread per pre-token replays tokenizeFast (tkz_fast.cuh)
-        TRY(ensure(ctx, ctx->a_pool_rk, N * 4));
-        TRY(ensure(ctx, ctx->a_fast_heap, N * 16 + 64));
-        TRY(ensure(ctx, ctx->a_word_aux, (W + 2) * 4));
-        FastArgs fa{d_text, word_start, word_end, word_doc, doc_word_off, nw, P.fast_max_sequence_length, P.fast_max_tokens,
-                    (uint32_t*)ctx->a_pool_id.p, (uint32_t*)ctx->a_pool_s.p, (uint32_t*)ctx->a_pool_e.p, (uint32_t*)ctx->a_pool_rk.p,
-                    (unsigned long long*)ctx->a_fast_heap.p, word_ntok, (uint32_t*)ctx->a_word_aux.p, ctrl};
-        if (m.kind == TKZ_MODEL_BPE) { fast_bpe_kernel<<<(nw + 127) / 128, 128, 0, st>>>(m, fa); launches++; }
-        else {
-            fast_wp_kernel<<<(nw + 127) / 128, 128, 0, st>>>(m, fa); launches++;
-            if (nd) { fast_wp_fix_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, st>>>(fa, nd); launches++; }
-        }
-    } else     if (nw) {
-        if (m.kind == TKZ_MODEL_BPE) {
-            len_class_count_kernel<<<128, 256, 0, st>>>(word_start, word_end, nw, nullptr, ctrl + 13); launches++;
-            TRY(readback(ctx, hctrl + 24, ctrl + 13, 3 * 8));
-            CK(cudaStreamSynchronize(st));
-            TRY(launch_bpe(ctx, m, d_text, word_start, word_end, nw, word_ntok, ctrl, 1, 0, hctrl + 24, N, launches));
-        } else {
-            WpArgs a{d_text, word_start, word_end, nw, (uint32_t*)ctx->a_pool_id.p, (uint32_t*)ctx->a_pool_s.p, (uint32_t*)ctx->a_pool_e.p,
-                     word_ntok, work_counter, ctrl, 0};
-            uint64_t blocks = (W + WP_WARPS - 1) / WP_WARPS;
-            const uint64_t cap = (uint64_t)ctx->sm_count * 8;
-            if (blocks > cap) blocks = cap;
-            wordpiece_warp_kernel<<<(unsigned)blocks, WP_WARPS * 32, 0, st>>>(m, a); launches++;
-        }
-    }
-
-    CK(cudaEventRecord(ctx->ev[2], st));
-    // ---- scans: tokens per word -> per document -> CSR
-    TRY(ensure(ctx, ctx->a_scan_tmp, (scan_tmp_elems(W) + scan_tmp_elems(n_docs)) * 8));
-    launches += exclusive_scan<uint32_t>(word_ntok, W, word_ntok, (unsigned long long*)ctx->a_scan_tmp.p, st);
-    const uint32_t* word_tok_off = word_ntok;
-    TRY(ensure(ctx, ctx->O().doc_tok_off, (n_docs + 1) * 8));
-    unsigned long long* doc_tok_off = (unsigned long long*)ctx->O().doc_tok_off.p;
-    EmitParams ep{P.has_truncation, P.max_length, P.has_padding, P.pad_length, P.pad_id, P.pad_type_id, P.pad_left, P.outputs};
-    emit_params_hf(ep, P);
-    if (nd) { doc_len_kernel<<<(nd + 255) / 256, 256, 0, st>>>(ep, word_tok_off, doc_word_off, nd, doc_tok_off); launches++; }
-    launches += exclusive_scan<unsigned long long>(doc_tok_off, n_docs, doc_tok_off, (unsigned long long*)ctx->a_scan_tmp.p, st);
-    gather_scalars_kernel<<<1, 1, 0, st>>>(ctrl, word_tok_off, nw, doc_tok_off, nd, word_doc); launches++;
-    TRY(readback(ctx, hctrl, ctrl, 5 * 8));
-    CK(cudaStreamSynchronize(st));
-    const unsigned long long errw = hctrl[0];
-    const uint64_t T_real = hctrl[2], T = hctrl[3];
-    ctx->stats.n_words = W; ctx->stats.n_unique_words = W; ctx->stats.n_long_words = 0;
-    if (errw != TKZ_ERRW_NONE) {
-        out->err_doc = (int64_t)hctrl[4];
-        const uint32_t code = (uint32_t)(errw & 0xFF);
-        ctx->err = code == TKZ_ECODE_UTF8 ? "invalid UTF-8 in a BPE pre-token (reference behaviour undefined)" : "MissingUnkToken";
-        ctx->stats.kernel_launches = launches;
-        return code == TKZ_ECODE_UTF8 ? TKZ_ERR_INVALID_UTF8 : TKZ_ERR_MISSING_UNK;
-    }
-
-    CK(cudaEventRecord(ctx->ev[3], st));
-    // ---- K5: emit
-    if (P.outputs & TKZ_OUT_IDS_U16) TRY(ensure(ctx, ctx->O().ids16, T * 2)); else TRY(ensure(ctx, ctx->O().ids, T * 4));
-    if (P.outputs & TKZ_OUT_OFFSETS) TRY(ensure(ctx, ctx->O().off, T * 8));
-    if (P.outputs & TKZ_OUT_ATTENTION) TRY(ensure(ctx, ctx->O().attn, T * 4));
-    if (P.outputs & TKZ_OUT_TYPE_IDS) TRY(ensure(ctx, ctx->O().type, T * 4));
-    if (P.outputs & TKZ_OUT_SPECIAL) TRY(ensure(ctx, ctx->O().special, T * 4));
-    if (P.outputs & TKZ_OUT_SPAN_TOKENS) TRY(ensure(ctx, ctx->O().spans, T * 16));
-    EmitOut eo{(uint32_t*)ctx->O().ids.p, (uint32_t*)ctx->O().off.p, (uint32_t*)ctx->O().attn.p, (uint32_t*)ctx->O().type.p,
-               (uint32_t*)ctx->O().special.p, nullptr, (uint16_t*)ctx->O().ids16.p, (uint4*)ctx->O().spans.p, nullptr, nullptr, 0u};
-    if (nw) {
-        const uint32_t big_cap = (uint32_t)(N / EMIT_BIG + 16);
-        TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
-        BigList bl{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 9) + 1, big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
-        emit_words_kernel<<<(nw + 255) / 256, 256, 0, st>>>(ep, eo, nw, word_start, word_doc, word_tok_off, doc_word_off, doc_tok_off,
-                                                            (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
-                                                            (const uint32_t*)ctx->a_pool_e.p, bl, d_doc_off); launches++;
-        emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, bl, (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
-                                                           (const uint32_t*)ctx->a_pool_e.p); launches++;
-    }
-    if ((P.has_padding || ((ep.hf_flags & 1u) && ep.n_pre + ep.n_suf)) && nd) {
-        emit_pad_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, st>>>(ep, eo, nd, word_tok_off, doc_word_off, doc_tok_off); launches++;
-    }
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(ctx->ev[4], st));
-    CK(cudaStreamSynchronize(st));
-    ctx->stats.kernel_launches = launches;
-    cudaEventElapsedTime(&ctx->stats.ms_split, ctx->ev[0], ctx->ev[1]);
-    cudaEventElapsedTime(&ctx->stats.ms_model, ctx->ev[1], ctx->ev[2]);
-    cudaEventElapsedTime(&ctx->stats.ms_scan, ctx->ev[2], ctx->ev[3]);
-    cudaEventElapsedTime(&ctx->stats.ms_emit, ctx->ev[3], ctx->ev[4]);
-    cudaEventElapsedTime(&ctx->stats.ms_total, ctx->ev[0], ctx->ev[4]);
-    out->n_docs = n_docs; out->n_tokens = T; out->n_real_tokens = T_real;
-    out->doc_tok_off = (const uint64_t*)doc_tok_off;
-    out->ids = (P.outputs & TKZ_OUT_IDS_U16) ? nullptr : eo.ids;
-    out->ids16 = (P.outputs & TKZ_OUT_IDS_U16) ? eo.ids16 : nullptr;
-    out->offsets = (P.outputs & TKZ_OUT_OFFSETS) ? eo.offsets : nullptr;
-    out->attention_mask = (P.outputs & TKZ_OUT_ATTENTION) ? eo.attention : nullptr;
-    out->type_ids = (P.outputs & TKZ_OUT_TYPE_IDS) ? eo.type_ids : nullptr;
-    out->special_tokens_mask = (P.outputs & TKZ_OUT_SPECIAL) ? eo.special : nullptr;
-    out->offsets_packed = nullptr;
-    out->span_tokens = (P.outputs & TKZ_OUT_SPAN_TOKENS) ? (const uint32_t*)eo.spans : nullptr;
-    return TKZ_OK;
+    return encode_words(ctx, m, d_text, d_doc_off, nd, N, P, out, launches);
 }
 
 }  // namespace
@@ -1207,6 +1231,14 @@ void wide_finish(WideRec* w, uint64_t n_total, const std::vector<std::array<uint
     std::sort(w, w + n_total, [](const WideRec& a, const WideRec& b) { return a.hi != b.hi ? a.hi < b.hi : a.lo < b.lo; });
 }
 
+// the per-token arrays of a device result (ResultArrays order), the pinned host arrays they are copied to, bytes per slot
+struct ResultCopy { const void* dev; HostBuf* host; size_t elem; };
+std::array<ResultCopy, 8> result_copies(tkz_ctx* ctx, const tkz_batch_result& r) {
+    return {{{r.ids, &ctx->h_ids, 4}, {r.offsets, &ctx->h_off, 8}, {r.attention_mask, &ctx->h_attn, 4}, {r.type_ids, &ctx->h_type, 4},
+             {r.special_tokens_mask, &ctx->h_special, 4}, {r.offsets_packed, &ctx->h_off16, 2}, {r.ids16, &ctx->h_ids16, 2},
+             {r.span_tokens, &ctx->h_spans, 16}}};
+}
+
 // one shot: H2D everything, encode, D2H everything (small batches)
 int encode_host_single(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_off, uint64_t n_docs, uint64_t N,
                        const tkz_encode_params* params, tkz_batch_result* out) {
@@ -1218,33 +1250,27 @@ int encode_host_single(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_of
     tkz_batch_result dev{};
     int rc = encode_device_impl(ctx, (const uint8_t*)ctx->a_text.p, (const uint64_t*)ctx->a_doc_off.p, n_docs, N, params, &dev);
     *out = dev;
-    out->doc_tok_off = nullptr; out->ids = nullptr; out->offsets = nullptr; out->attention_mask = nullptr; out->type_ids = nullptr;
-    out->special_tokens_mask = nullptr; out->offsets_packed = nullptr; out->ids16 = nullptr; out->span_tokens = nullptr;
+    set_result(out, dev.n_docs, dev.n_tokens, dev.n_real_tokens, nullptr, {}, 0, nullptr);    // (no device pointer leaves)
     if (rc != TKZ_OK) return rc;
     const uint64_t T = dev.n_tokens;
     cudaStream_t st = ctx->stream;
     TRY(ensure_host(ctx, ctx->h_doc_tok_off, (n_docs + 1) * 8));
     CK(cudaMemcpyAsync(ctx->h_doc_tok_off.p, dev.doc_tok_off, (n_docs + 1) * 8, cudaMemcpyDeviceToHost, st));
-    out->doc_tok_off = (const uint64_t*)ctx->h_doc_tok_off.p;
-    struct { const void* src; HostBuf* hb; const void** dst; size_t elem; } cp[] = {
-        {dev.ids, &ctx->h_ids, (const void**)&out->ids, 4}, {dev.offsets, &ctx->h_off, (const void**)&out->offsets, 8},
-        {dev.attention_mask, &ctx->h_attn, (const void**)&out->attention_mask, 4}, {dev.type_ids, &ctx->h_type, (const void**)&out->type_ids, 4},
-        {dev.special_tokens_mask, &ctx->h_special, (const void**)&out->special_tokens_mask, 4},
-        {dev.offsets_packed, &ctx->h_off16, (const void**)&out->offsets_packed, 2}, {dev.ids16, &ctx->h_ids16, (const void**)&out->ids16, 2},
-        {dev.span_tokens, &ctx->h_spans, (const void**)&out->span_tokens, 16}};
-    for (auto& c : cp) {
-        if (!c.src) continue;
-        TRY(ensure_host(ctx, *c.hb, T * c.elem));
-        if (T) CK(cudaMemcpyAsync(c.hb->p, c.src, T * c.elem, cudaMemcpyDeviceToHost, st));
-        *c.dst = c.hb->p;
+    const auto cp = result_copies(ctx, dev);
+    ResultArrays host{};
+    for (uint32_t i = 0; i < 8; i++) {
+        if (!cp[i].dev) continue;
+        TRY(ensure_host(ctx, *cp[i].host, T * cp[i].elem));
+        if (T) CK(cudaMemcpyAsync(cp[i].host->p, cp[i].dev, T * cp[i].elem, cudaMemcpyDeviceToHost, st));
+        host[i] = cp[i].host->p;
     }
-    out->n_wide = 0; out->wide_tokens = nullptr;
     if (dev.n_wide) {
         TRY(ensure_host(ctx, ctx->h_wide, dev.n_wide * 16));
         CK(cudaMemcpyAsync(ctx->h_wide.p, dev.wide_tokens, dev.n_wide * 16, cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
-    if (dev.n_wide) { wide_finish((WideRec*)ctx->h_wide.p, dev.n_wide, {}); out->n_wide = dev.n_wide; out->wide_tokens = (const uint32_t*)ctx->h_wide.p; }
+    if (dev.n_wide) wide_finish((WideRec*)ctx->h_wide.p, dev.n_wide, {});
+    set_result(out, dev.n_docs, T, dev.n_real_tokens, (const uint64_t*)ctx->h_doc_tok_off.p, host, dev.n_wide, ctx->h_wide.p);
     ctx->stats.ms_call_kernels = ctx->stats.ms_total;
     return TKZ_OK;
 }
@@ -1290,7 +1316,7 @@ int encode_host_chunked(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_o
         CK(cudaEventRecord(ctx->ev_h2d[b], ctx->s_h2d));
         return TKZ_OK;
     };
-    bool used_ids16 = false;
+    ResultArrays host{};
 restart:
     cb.resize(2); chunk_target = ctx->chunk_bytes; ctx->kept_valid = false; ctx->call_uniq = 0;
     uint64_t W_total = 0; std::vector<std::array<uint64_t, 3>> wide_parts;
@@ -1336,20 +1362,19 @@ restart:
         ms_kernels += ctx->stats.ms_total;
         // kernel-bound chunk (its device time exceeds what ~45 GB/s of PCIe needs for its text): larger chunks from now on
         if ((double)ctx->stats.ms_total * 1e-3 > (double)nb / 45e9 && chunk_target < chunk_max) chunk_target *= 2;
-        used_ids16 = dev.ids16 != nullptr;                      // (the same decision in every chunk: it depends on the model and the parameters)
         const uint64_t T = dev.n_tokens;
         // size the host arrays from the first chunk's token density
         uint64_t est = T_total + T;
         if (i == 0 && nb) est = (uint64_t)((double)T * ((double)N / (double)nb) * 1.03) + 4096;
         if (est < T_total + T) est = T_total + T;
-        struct { const void* src; HostBuf* hb; size_t elem; } cp[] = {
-            {dev.ids, &ctx->h_ids, 4}, {dev.offsets, &ctx->h_off, 8}, {dev.attention_mask, &ctx->h_attn, 4},
-            {dev.type_ids, &ctx->h_type, 4}, {dev.special_tokens_mask, &ctx->h_special, 4}, {dev.offsets_packed, &ctx->h_off16, 2},
-            {dev.ids16, &ctx->h_ids16, 2}, {dev.span_tokens, &ctx->h_spans, 16}};
-        for (auto& c : cp) {
-            if (!c.src) continue;
-            TRY(ensure_host_keep(ctx, *c.hb, est * c.elem, T_total * c.elem));
-            if (T) CK(cudaMemcpyAsync((uint8_t*)c.hb->p + T_total * c.elem, c.src, T * c.elem, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        // (every chunk delivers the same arrays: they depend on the model and the parameters)
+        const auto cp = result_copies(ctx, dev);
+        for (uint32_t k = 0; k < 8; k++) {
+            host[k] = nullptr;
+            if (!cp[k].dev) continue;
+            TRY(ensure_host_keep(ctx, *cp[k].host, est * cp[k].elem, T_total * cp[k].elem));
+            if (T) CK(cudaMemcpyAsync((uint8_t*)cp[k].host->p + T_total * cp[k].elem, cp[k].dev, T * cp[k].elem, cudaMemcpyDeviceToHost, ctx->s_d2h));
+            host[k] = cp[k].host->p;
         }
         if (dev.n_wide) {
             TRY(ensure_host_keep(ctx, ctx->h_wide, (W_total + dev.n_wide) * 16, W_total * 16));
@@ -1369,19 +1394,7 @@ restart:
     if (W_total) wide_finish((WideRec*)ctx->h_wide.p, W_total, wide_parts);
     ctx->out_sel = 0;
     ctx->stats.ms_call_kernels = ms_kernels;
-    uint32_t outputs = P.outputs;
-    if ((outputs & TKZ_OUT_IDS_U16) && !used_ids16) outputs &= ~TKZ_OUT_IDS_U16;
-    out->n_docs = n_docs; out->n_tokens = T_total; out->n_real_tokens = T_real;
-    out->doc_tok_off = h_dto;
-    out->ids = (outputs & TKZ_OUT_IDS_U16) ? nullptr : (const uint32_t*)ctx->h_ids.p;
-    out->ids16 = (outputs & TKZ_OUT_IDS_U16) ? (const uint16_t*)ctx->h_ids16.p : nullptr;
-    out->offsets = (outputs & TKZ_OUT_OFFSETS) ? (const uint32_t*)ctx->h_off.p : nullptr;
-    out->attention_mask = (outputs & TKZ_OUT_ATTENTION) ? (const uint32_t*)ctx->h_attn.p : nullptr;
-    out->type_ids = (outputs & TKZ_OUT_TYPE_IDS) ? (const uint32_t*)ctx->h_type.p : nullptr;
-    out->special_tokens_mask = (outputs & TKZ_OUT_SPECIAL) ? (const uint32_t*)ctx->h_special.p : nullptr;
-    out->offsets_packed = (outputs & TKZ_OUT_OFFSETS_PACKED) ? (const uint16_t*)ctx->h_off16.p : nullptr;
-    out->span_tokens = (outputs & TKZ_OUT_SPAN_TOKENS) ? (const uint32_t*)ctx->h_spans.p : nullptr;
-    out->n_wide = (outputs & TKZ_OUT_OFFSETS_PACKED) ? W_total : 0; out->wide_tokens = out->n_wide ? (const uint32_t*)ctx->h_wide.p : nullptr;
+    set_result(out, n_docs, T_total, T_real, h_dto, host, W_total, ctx->h_wide.p);
     return TKZ_OK;
 }
 

@@ -16,7 +16,7 @@ struct EmitParams {
     uint32_t pad_id, pad_type_id; int pad_left;
     uint32_t outputs;
     // hf_compat (tkz_encode_params.hf_flags; 0 = the reference): single-sequence template -- what processor.zig:41-152 declares
-    // and leaves as TODO -- and offsets relative to the document.  Only the per-occurrence pipeline serves it.
+    // and leaves as TODO -- and offsets relative to the document.  Both device pipelines serve it.
     uint32_t hf_flags;
     uint32_t n_pre, n_suf, pre_id[4], pre_type[4], suf_id[4], suf_type[4], seq_type;
 };
@@ -33,12 +33,14 @@ __device__ __forceinline__ unsigned long long doc_out_len(const EmitParams& p, u
     return (p.has_pad && k + add < p.pad_length) ? p.pad_length : k + add;
 }
 
-// per document: real token count -> output slot count
+// per document: real token count -> output slot count; the real count also to doc_real when the padding / template
+// kernels need it (doc_real != nullptr)
 __global__ void doc_len_kernel(EmitParams p, const uint32_t* __restrict__ word_tok_off, const uint32_t* __restrict__ doc_word_off, uint32_t n_docs,
-                               unsigned long long* __restrict__ doc_len) {
+                               unsigned long long* __restrict__ doc_len, uint32_t* __restrict__ doc_real) {
     const uint32_t d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d >= n_docs) return;
     const unsigned long long t = word_tok_off[doc_word_off[d + 1]] - word_tok_off[doc_word_off[d]];
+    if (doc_real) doc_real[d] = (uint32_t)t;
     unsigned long long kept;
     doc_len[d] = doc_out_len(p, t, &kept);
 }
@@ -147,36 +149,6 @@ __global__ void __launch_bounds__(256) emit_big_kernel(EmitParams p, EmitOut o, 
         const unsigned long long dst = (unsigned long long)it.z | ((unsigned long long)it.w << 32);
         for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < it.y; i += gridDim.x * blockDim.x)
             emit_real(p, o, dst + i, pool_id[it.x + i], pool_s[it.x + i] + sh, pool_e[it.x + i] + sh);
-    }
-}
-
-// padding slots, one warp per document (src/encoding.zig:407-414, 418-425)
-__global__ void __launch_bounds__(256) emit_pad_kernel(EmitParams p, EmitOut o, uint32_t n_docs, const uint32_t* __restrict__ word_tok_off,
-                                                       const uint32_t* __restrict__ doc_word_off, const unsigned long long* __restrict__ doc_tok_off) {
-    const uint32_t d = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint32_t lane = lane_id();
-    if (d >= n_docs) return;
-    const unsigned long long t = word_tok_off[doc_word_off[d + 1]] - word_tok_off[doc_word_off[d]];
-    unsigned long long kept;
-    const unsigned long long olen = doc_out_len(p, t, &kept);
-    const unsigned long long full = kept + tpl_added(p);
-    if (p.hf_flags & 1u) {
-        // the template's special tokens around the kept tokens
-        const unsigned long long b0 = doc_tok_off[d] + ((p.has_pad && p.pad_left) ? olen - full : 0);
-        if (lane < p.n_pre) emit_special(p, o, b0 + lane, p.pre_id[lane], p.pre_type[lane]);
-        if (lane >= 8 && lane - 8 < p.n_suf) emit_special(p, o, b0 + p.n_pre + kept + (lane - 8), p.suf_id[lane - 8], p.suf_type[lane - 8]);
-    }
-    if (olen == full) return;
-    const unsigned long long base = doc_tok_off[d] + (p.pad_left ? 0 : full);
-    const unsigned long long npad = olen - full;
-    for (unsigned long long k = lane; k < npad; k += 32) {
-        const unsigned long long dst = base + k;
-        emit_id(p, o, dst, p.pad_id);
-        if (p.outputs & 2u) reinterpret_cast<uint2*>(o.offsets)[dst] = make_uint2(0u, 0u);
-        if (p.outputs & 4u) o.attention[dst] = 0u;
-        if (p.outputs & 8u) o.type_ids[dst] = p.pad_type_id;
-        if (p.outputs & 16u) o.special[dst] = 1u;
-        if (p.outputs & 128u) o.spans[dst] = make_uint4(p.pad_id, 0u, 0u, 0x0400u);     // initPadding: flags.is_padding (bit 2)
     }
 }
 

@@ -1195,7 +1195,7 @@ __device__ __forceinline__ void warp_fill_u32(uint32_t* p, unsigned long long n,
 
 // padding slots from per-document real counts (src/encoding.zig:407-414, 418-425), one warp per document
 __global__ void __launch_bounds__(256) emit_pad_real_kernel(EmitParams p, EmitOut o, uint32_t n_docs, const uint32_t* __restrict__ doc_real,
-                                                            const unsigned long long* __restrict__ doc_tok_off, bool pads) {
+                                                            const unsigned long long* __restrict__ doc_tok_off) {
     const uint32_t d = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (d >= n_docs) return;
     unsigned long long kept;
@@ -1208,7 +1208,7 @@ __global__ void __launch_bounds__(256) emit_pad_real_kernel(EmitParams p, EmitOu
         if (lane < p.n_pre) emit_special(p, o, b0 + lane, p.pre_id[lane], p.pre_type[lane]);
         if (lane >= 8 && lane - 8 < p.n_suf) emit_special(p, o, b0 + p.n_pre + kept + (lane - 8), p.suf_id[lane - 8], p.suf_type[lane - 8]);
     }
-    if (olen == full || !pads) return;
+    if (olen == full) return;
     const unsigned long long base = doc_tok_off[d] + (p.pad_left ? 0 : full);
     const unsigned long long npad = olen - full;
     if (p.outputs & 64u) { uint16_t* q = o.ids16 + base; for (unsigned long long i = lane_id(); i < npad; i += 32) q[i] = (uint16_t)p.pad_id; }
