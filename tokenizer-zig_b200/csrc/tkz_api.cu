@@ -77,6 +77,7 @@ struct tkz_ctx {
     bool has_iso = false;                 // the class table isolates some byte (punctuation split)
     ClassRanges cr{}, cr_post{};          // byte classes as ranges (raw bytes / bytes already normalised by K0)
     bool stage_bulk = true;               // TKZ_STAGE=ldg: pass A stages its slices with plain loads instead of bulk copies (A/B switch)
+    bool narrow_records = true;           // TKZ_TOK_RECORD=wide: u32 ids in the token stream even for 16-bit vocabularies (A/B switch)
     // chunks of ONE host-buffer call share the word table and the record pool of the slice pipeline: the first chunk starts from an
     // empty table, the later ones find the call's frequent words already tokenized (every call starts cold; TKZ_KEEP_TABLE=0
     // gives every chunk its own table)
@@ -219,6 +220,23 @@ __global__ void gather_scalars_kernel(unsigned long long* ctrl, const uint32_t* 
     ctrl[4] = (ew != TKZ_ERRW_NONE && n_words) ? word_doc[(uint32_t)(ew >> 8)] : 0;
 }
 
+// pass A's shared memory (above the 48 KB default) for every class mode and record kind of a model
+template <int MODEL, int REC>
+void slice_words_smem_rec() {
+    const int sm = (int)sizeof(BlockShared);
+    cudaFuncSetAttribute(slice_words_kernel<MODEL, 0, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
+    cudaFuncSetAttribute(slice_words_kernel<MODEL, 1, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
+    cudaFuncSetAttribute(slice_words_kernel<MODEL, 2, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
+    cudaFuncSetAttribute(slice_words_kernel<MODEL, 3, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
+}
+template <int MODEL>
+void slice_words_smem() {
+    slice_words_smem_rec<MODEL, TW_REC_ID32>();
+    slice_words_smem_rec<MODEL, TW_REC_WIDE>();
+    slice_words_smem_rec<MODEL, TW_REC_ID16>();
+    slice_words_smem_rec<MODEL, TW_REC4>();
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------ context
@@ -247,17 +265,8 @@ extern "C" int tkz_ctx_create(int device, void* stream, uint64_t arena_hint_byte
     }
     cudaFuncSetAttribute(bpe_block_kernel<1024, 12288>, cudaFuncAttributeMaxDynamicSharedMemorySize, 12288 * 15);
     cudaFuncSetAttribute(bpe_block_kernel<512, 4096, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4096 * 15);
-    {
-        const int sm = (int)sizeof(BlockShared);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_BPE, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_BPE, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_BPE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_BPE, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_WORDPIECE, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_WORDPIECE, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_WORDPIECE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-        cudaFuncSetAttribute(slice_words_kernel<TKZ_MODEL_WORDPIECE, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-    }
+    slice_words_smem<TKZ_MODEL_BPE>();
+    slice_words_smem<TKZ_MODEL_WORDPIECE>();
     e = cudaFuncSetAttribute(bpe_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BPE_SMEM_BYTES);
     if (e != cudaSuccess) {
         g_create_error = std::string("kernel image not usable on this device (built for sm_100a): ") + cudaGetErrorString(e);
@@ -275,6 +284,7 @@ extern "C" int tkz_ctx_create(int device, void* stream, uint64_t arena_hint_byte
     if (const char* e = getenv("TKZ_NO_DEDUP")) ctx->use_dedup = !(e[0] == '1');     // A/B switch for the parity tests
     if (const char* e = getenv("TKZ_CLASSIFY")) ctx->force_lut = (e[0] == 'l');
     if (const char* e = getenv("TKZ_STAGE")) ctx->stage_bulk = !(e[0] == 'l');
+    if (const char* e = getenv("TKZ_TOK_RECORD")) ctx->narrow_records = !(e[0] == 'w');
     if (const char* e = getenv("TKZ_KEEP_TABLE")) ctx->keep_table = e[0] != '0';
     if (const char* e = getenv("TKZ_NO_GRID")) ctx->use_grid = !(e[0] == '1');
     if (const char* e = getenv("TKZ_GRID_MIN_LEN")) { const long long v = atoll(e); if (v > (long long)BB_WARP_MAX) ctx->grid_min_len = (uint32_t)v; }
@@ -792,23 +802,37 @@ int report_error(tkz_ctx* ctx, unsigned long long errw, uint64_t err_doc, uint64
 // estimated from the batch and from what earlier batches of the context needed; when pass A runs out of one of them the
 // call returns TKZ_RETRY_WORST and the caller runs it again with worst-case capacities (tokens <= bytes), never truncated.
 #define TKZ_RETRY_WORST 2
-template <int MODEL>
-void launch_slice_words(const DevModel& m, const SliceArgs& ta, int cls, uint32_t blocks, cudaStream_t st) {
+template <int MODEL, int REC>
+void launch_slice_words_rec(const DevModel& m, const SliceArgs& ta, int cls, uint32_t blocks, cudaStream_t st) {
     const size_t sm = sizeof(BlockShared);
-    if (cls == 0) slice_words_kernel<MODEL, 0><<<blocks, TW_THREADS, sm, st>>>(m, ta);
-    else if (cls == 1) slice_words_kernel<MODEL, 1><<<blocks, TW_THREADS, sm, st>>>(m, ta);
-    else if (cls == 2) slice_words_kernel<MODEL, 2><<<blocks, TW_THREADS, sm, st>>>(m, ta);
-    else slice_words_kernel<MODEL, 3><<<blocks, TW_THREADS, sm, st>>>(m, ta);
+    if (cls == 0) slice_words_kernel<MODEL, 0, REC><<<blocks, TW_THREADS, sm, st>>>(m, ta);
+    else if (cls == 1) slice_words_kernel<MODEL, 1, REC><<<blocks, TW_THREADS, sm, st>>>(m, ta);
+    else if (cls == 2) slice_words_kernel<MODEL, 2, REC><<<blocks, TW_THREADS, sm, st>>>(m, ta);
+    else slice_words_kernel<MODEL, 3, REC><<<blocks, TW_THREADS, sm, st>>>(m, ta);
 }
+template <int MODEL>
+void launch_slice_words(const DevModel& m, const SliceArgs& ta, int cls, int rec, uint32_t blocks, cudaStream_t st) {
+    if (rec == TW_REC_ID32) launch_slice_words_rec<MODEL, TW_REC_ID32>(m, ta, cls, blocks, st);
+    else if (rec == TW_REC_WIDE) launch_slice_words_rec<MODEL, TW_REC_WIDE>(m, ta, cls, blocks, st);
+    else if (rec == TW_REC_ID16) launch_slice_words_rec<MODEL, TW_REC_ID16>(m, ta, cls, blocks, st);
+    else launch_slice_words_rec<MODEL, TW_REC4>(m, ta, cls, blocks, st);
+}
+// the output forms with offsets read TW_REC_WIDE or TW_REC4 records, the ids-only forms TW_REC_ID32 or TW_REC_ID16
 template <bool PLAIN>
-void launch_slice_emit(const SliceEmitArgs& ea, const EmitParams& ep, const EmitOut& eo, uint32_t blocks, cudaStream_t st) {
+void launch_slice_emit(const SliceEmitArgs& ea, const EmitParams& ep, const EmitOut& eo, int rec, uint32_t blocks, cudaStream_t st) {
     const uint32_t o = ep.outputs;
-    if (o == TKZ_OUT_IDS) slice_emit_kernel<PLAIN, 1u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
-    else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS | TKZ_OUT_ATTENTION)) slice_emit_kernel<PLAIN, 7u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
-    else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS_PACKED)) slice_emit_kernel<PLAIN, 33u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
-    else if (o == (TKZ_OUT_IDS | TKZ_OUT_IDS_U16 | TKZ_OUT_OFFSETS_PACKED)) slice_emit_kernel<PLAIN, 97u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
-    else if (o == (TKZ_OUT_IDS | TKZ_OUT_IDS_U16)) slice_emit_kernel<PLAIN, 65u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
-    else slice_emit_kernel<PLAIN, 0u><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo);
+    const bool narrow = rec == TW_REC4 || rec == TW_REC_ID16;
+#define TKZ_SLICE_EMIT(OUTS, REC) slice_emit_kernel<PLAIN, OUTS, REC><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo)
+    if (o == TKZ_OUT_IDS) { if (narrow) TKZ_SLICE_EMIT(1u, TW_REC_ID16); else TKZ_SLICE_EMIT(1u, TW_REC_ID32); }
+    else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS | TKZ_OUT_ATTENTION)) { if (narrow) TKZ_SLICE_EMIT(7u, TW_REC4); else TKZ_SLICE_EMIT(7u, TW_REC_WIDE); }
+    else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS_PACKED)) { if (narrow) TKZ_SLICE_EMIT(33u, TW_REC4); else TKZ_SLICE_EMIT(33u, TW_REC_WIDE); }
+    else if (o == (TKZ_OUT_IDS | TKZ_OUT_IDS_U16 | TKZ_OUT_OFFSETS_PACKED)) { if (narrow) TKZ_SLICE_EMIT(97u, TW_REC4); else TKZ_SLICE_EMIT(97u, TW_REC_WIDE); }
+    else if (o == (TKZ_OUT_IDS | TKZ_OUT_IDS_U16)) { if (narrow) TKZ_SLICE_EMIT(65u, TW_REC_ID16); else TKZ_SLICE_EMIT(65u, TW_REC_ID32); }
+    else if (rec == TW_REC_ID32) TKZ_SLICE_EMIT(0u, TW_REC_ID32);
+    else if (rec == TW_REC_WIDE) TKZ_SLICE_EMIT(0u, TW_REC_WIDE);
+    else if (rec == TW_REC_ID16) TKZ_SLICE_EMIT(0u, TW_REC_ID16);
+    else TKZ_SLICE_EMIT(0u, TW_REC4);
+#undef TKZ_SLICE_EMIT
 }
 
 int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const uint8_t* d_text, const uint64_t* d_doc_off, uint32_t nd, uint64_t N,
@@ -843,10 +867,15 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     if (tok_cap > 0xFFFFF000ull) tok_cap = 0xFFFFF000ull;
     const uint32_t long_cap = (uint32_t)(N / 256 + 16);                        // a long word has more than 255 bytes: always enough
     const bool want_of = (P.outputs & (TKZ_OUT_OFFSETS | TKZ_OUT_OFFSETS_PACKED)) != 0;
+    // token stream records: 16-bit ids when every id of the model fits, with the two offset bytes beside them in 4 bytes --
+    // unless the offsets are document-relative (hf_compat), which needs the word's position in the slice as well
+    const bool narrow = ctx->narrow_records && ctx->ids16_ok && !(want_of && (P.hf_flags & TKZ_HF_DOC_OFFSETS));
+    const int rec = want_of ? (narrow ? TW_REC4 : TW_REC_WIDE) : (narrow ? TW_REC_ID16 : TW_REC_ID32);
+    const size_t rec_bytes = rec == TW_REC_WIDE ? 8 : (rec == TW_REC_ID16 ? 2 : 4);
     TRY(ensure(ctx, ctx->a_wtable, ((size_t)tcap + mcap) * sizeof(WordSlot) + (size_t)m32cap * sizeof(WordSlot32)));
     TRY(ensure(ctx, ctx->a_upool, (size_t)upool_cap * 8));
     TRY(ensure(ctx, ctx->a_lscratch, (size_t)warps * 4 * 256 * 4));
-    TRY(ensure(ctx, ctx->a_tok_id, (size_t)tok_cap * (want_of ? 8 : 4)));
+    TRY(ensure(ctx, ctx->a_tok_id, (size_t)tok_cap * rec_bytes));
     TRY(ensure(ctx, ctx->a_tile_tok_off, ((size_t)n_slices + 2) * 4));
     TRY(ensure(ctx, ctx->a_tile_ntok_inline, ((size_t)n_slices + 2) * 4));
     TRY(ensure(ctx, ctx->a_tile_ntok, ((size_t)n_slices + 2) * 4));
@@ -868,7 +897,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ta.table32 = (WordSlot32*)((WordSlot*)ctx->a_wtable.p + tcap + mcap); ta.table32_mask = m32cap - 1;
     ta.upool = (unsigned long long*)ctx->a_upool.p; ta.upool_cap = (uint32_t)upool_cap; ta.upool_count = (unsigned int*)(ctrl + 9);
     ta.lscratch = (uint32_t*)ctx->a_lscratch.p;
-    ta.tok_id = (uint32_t*)ctx->a_tok_id.p; ta.tok2 = want_of ? (uint2*)ctx->a_tok_id.p : nullptr;
+    ta.tok = ctx->a_tok_id.p;
     ta.tok_cap = (uint32_t)tok_cap; ta.tok_count = (unsigned int*)(ctrl + 5);
     ta.slice_tok_off = (uint32_t*)ctx->a_tile_tok_off.p; ta.slice_ntok_inline = (uint32_t*)ctx->a_tile_ntok_inline.p;
     ta.slice_ntok = (uint32_t*)ctx->a_tile_ntok.p; ta.slice_long = (uint32_t*)ctx->a_tile_long.p;
@@ -882,8 +911,8 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ta.stage_bulk = ctx->stage_bulk ? 1 : 0;
     ta.has_iso = ctx->has_iso ? 1 : 0;
     const int cls = (cr.usable && !ctx->force_lut) ? (cr.norm_lower ? 1 : 0) : (m.norm_identity ? 2 : 3);
-    if (m.kind == TKZ_MODEL_BPE) launch_slice_words<TKZ_MODEL_BPE>(m, ta, cls, grid, st);
-    else launch_slice_words<TKZ_MODEL_WORDPIECE>(m, ta, cls, grid, st);
+    if (m.kind == TKZ_MODEL_BPE) launch_slice_words<TKZ_MODEL_BPE>(m, ta, cls, rec, grid, st);
+    else launch_slice_words<TKZ_MODEL_WORDPIECE>(m, ta, cls, rec, grid, st);
     launches++;
     if (m.kind == TKZ_MODEL_BPE) { len_class_count_kernel<<<128, 256, 0, st>>>(ta.long_start, ta.long_end, 0, ta.n_long, ctrl + 13); launches++; }
     TRY(readback(ctx, hctrl, ctrl, 16 * 8));
@@ -965,7 +994,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
     SliceEmitArgs ea{};
     ea.doc_off = d_doc_off; ea.n_docs = nd; ea.n_slices = n_slices; ea.slice_doc_lo = ta.slice_doc_lo;
-    ea.tok_id = ta.tok_id; ea.tok2 = ta.tok2;
+    ea.tok = ta.tok;
     ea.slice_tok_off = ta.slice_tok_off; ea.slice_ntok_inline = ta.slice_ntok_inline; ea.slice_long = ta.slice_long; ea.slice_tokbase = ta.slice_ntok;
     ea.long_start = ta.long_start; ea.long_ins = ta.long_ins; ea.long_ntok = (const uint32_t*)ctx->a_long_ntok.p;
     ea.pool_id = (const uint32_t*)ctx->a_pool_id.p; ea.pool_s = (const uint32_t*)ctx->a_pool_s.p; ea.pool_e = (const uint32_t*)ctx->a_pool_e.p;
@@ -974,8 +1003,8 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ea.big = BigList{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 16), big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
     const bool filled = pad_prologue(ctx, ep, eo, nd, T, T_real, launches);
     const uint32_t egrid = (uint32_t)std::min<uint64_t>(((uint64_t)n_slices + TW_WARPS - 1) / TW_WARPS, (uint64_t)ctx->sm_count * 16);
-    if (plain) launch_slice_emit<true>(ea, ep, eo, egrid, st);
-    else launch_slice_emit<false>(ea, ep, eo, egrid, st);
+    if (plain) launch_slice_emit<true>(ea, ep, eo, rec, egrid, st);
+    else launch_slice_emit<false>(ea, ep, eo, rec, egrid, st);
     launches++;
     if (n_long) { emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, ea.big, ea.pool_id, ea.pool_s, ea.pool_e); launches++; }
     pad_epilogue(ctx, ep, eo, nd, (const uint32_t*)ctx->a_doc_real.p, doc_tok_off, filled, launches);

@@ -14,8 +14,9 @@
 //              symbols in shared memory) and publishes the value; a word whose owner is still computing is polled after
 //              the warp has published its own words (owners never wait, so polling cannot deadlock).  Words of 16..31
 //              bytes go the same way through 64-byte slots.  Result: the TOKENS of the slice's words, in text order, in
-//              a compact per-slice run of the token stream (id u32 + offsets u8,u8), the token count of the slice and the
-//              token prefix at every document start.
+//              a compact per-slice run of the token stream (one record per token, TW_REC_*: 4 bytes = id u16 + offsets
+//              u8,u8 when every id of the model fits 16 bits, else id u32 + offsets; ids only: u16 or u32), the token
+//              count of the slice and the token prefix at every document start.
 //   [word-list kernels on the few pre-tokens longer than TW_MAX_INLINE bytes (tkz_bpe.cuh / tkz_bpe_block.cuh /
 //    tkz_wordpiece.cuh), long_fix_kernel adds their token counts]
 //   scan over slices
@@ -61,6 +62,13 @@ constexpr uint32_t TW_LONGF = 0x20000000u;        // in registers only: the word
 constexpr uint32_t TW_NONE = 0xFFFFFFFFu;
 constexpr uint32_t TW_MAX_SLICE_LONG = 4;         // long words (> 255 bytes) that can START in one 1 KiB slice
 
+// token stream records, chosen per call (encode_slices) and compiled into both passes.  Offsets fit a byte each (a word of
+// pass A has <= 255 bytes); ids fit 16 bits when every id the model can emit is below 65536.
+constexpr int TW_REC_ID32 = 0;                    // u32 id (ids only)
+constexpr int TW_REC_WIDE = 1;                    // {u32 id, start | end << 8 | the word's position in the slice << 16}
+constexpr int TW_REC_ID16 = 2;                    // u16 id (ids only, 16-bit vocabulary)
+constexpr int TW_REC4 = 3;                        // u32: id | start << 16 | end << 24 (16-bit vocabulary, pre-token offsets)
+
 // 32-byte slot = one L2 sector.  Short words (<= 15 bytes): k0..k3 = the normalised bytes, length in the top byte of k3
 // (so a used key is never all zero).  Medium words live in their own slot range: k0,k1 = 64-bit tag (top bit set),
 // k2,k3 = representative occurrence (text position, length), published after the tag.
@@ -100,7 +108,7 @@ struct SliceArgs {
     WordSlot32* table32; uint32_t table32_mask;
     unsigned long long* upool; uint32_t upool_cap; unsigned int* upool_count;     // token records: id | start << 32 | end << 48
     uint32_t* lscratch;                           // per warp of the grid: 4 * 256 u32, symbol arrays of words of 65..255 bytes
-    uint32_t* tok_id; uint2* tok2; uint32_t tok_cap; unsigned int* tok_count;     // token stream: ids only, or {id, start | end << 8} records (tok2) when the call wants offsets
+    void* tok; uint32_t tok_cap; unsigned int* tok_count;                         // token stream: tok_cap records of the kind TW_REC_*
     uint32_t* slice_tok_off; uint32_t* slice_ntok_inline; uint32_t* slice_ntok;   // slice_ntok (+ long words) is scanned -> token base
     uint32_t* slice_long;                         // first long-list index << 3 | count of the long words that start in the slice
     uint32_t* doc_tok_local;                      // per document: tokens of its slice before its first word
@@ -591,9 +599,19 @@ __device__ __forceinline__ WholeWarpOut tw_own_word(const DevModel& m, const Sli
     return out;
 }
 
+// one token into the stream at index i: of = start | end << 8, ph = the word's position in the slice << 16
+template <int REC>
+__device__ __forceinline__ void tw_put_token(void* tok, uint32_t i, uint32_t id, uint32_t of, uint32_t ph) {
+    if (REC == TW_REC_WIDE) static_cast<uint2*>(tok)[i] = make_uint2(id, of | ph);
+    else if (REC == TW_REC4) static_cast<uint32_t*>(tok)[i] = id | (of << 16);
+    else if (REC == TW_REC_ID16) static_cast<uint16_t*>(tok)[i] = (uint16_t)id;
+    else static_cast<uint32_t*>(tok)[i] = id;
+}
+
 // copies the token records of the listed words (three or more tokens each) from the pool into the token stream: four lanes
 // per word, eight words per step, so that the L2 round trips of a whole slice overlap (one at a time they were 17 % of the
 // kernel's stall samples)
+template <int REC>
 __device__ __forceinline__ void tw_flush_pooled(const SliceArgs& a, const uint4* plist, uint32_t n) {
     const uint32_t lane = lane_id();
     __syncwarp();
@@ -601,17 +619,17 @@ __device__ __forceinline__ void tw_flush_pooled(const SliceArgs& a, const uint4*
         const uint4 q = plist[e];
         for (uint32_t i = lane & 3u; i < q.y; i += 4) {
             const unsigned long long r = __ldcg(a.upool + q.x + i);       // written in THIS launch by the word's owner: L2, not the read-only path
-            const uint32_t of = ((uint32_t)(r >> 32) & 0xFFu) | (((uint32_t)(r >> 48) & 0xFFu) << 8) | q.w;
-            if (a.tok2) a.tok2[q.z + i] = make_uint2((uint32_t)r, of);
-            else a.tok_id[q.z + i] = (uint32_t)r;
+            const uint32_t of = ((uint32_t)(r >> 32) & 0xFFu) | (((uint32_t)(r >> 48) & 0xFFu) << 8);
+            tw_put_token<REC>(a.tok, q.z + i, (uint32_t)r, of, q.w);
         }
     }
     __syncwarp();
 }
 
 // CLS: 0 byte ranges + identity byte map, 1 byte ranges + ASCII lower-case, 2 LUT + identity, 3 LUT + arbitrary byte map
-// pass A: one warp per 1 KiB slice, slices strided over all warps of the grid (4 blocks of 8 warps per SM)
-template <int MODEL, int CLS>
+// REC: the token stream's record kind (TW_REC_*)
+// pass A: one warp per 1 KiB slice, slices strided over all warps of the grid (3 blocks of 8 warps per SM)
+template <int MODEL, int CLS, int REC>
 __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kernel(const __grid_constant__ DevModel m, const __grid_constant__ SliceArgs a) {
     extern __shared__ __align__(128) unsigned char tw_smem_raw[];
     BlockShared& bs = *reinterpret_cast<BlockShared*>(tw_smem_raw);
@@ -918,16 +936,16 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             else { const uint32_t inc = warp_incl_scan(nt); ex = inc - nt; tot = __shfl_sync(FULL, inc, 31); }
             const uint32_t dst = tbase + run + ex;                  // stream position of the word's first token
             if (can_store && nt && !(flags & TW_POOLF)) {
-                // (record: id, start | end << 8 | the word's position in the slice << 16 -- the position is only read by the hf_compat
-                // mode of pass B, which reports offsets relative to the document)
-                if (a.tok2) { const uint32_t ph = p << 16; a.tok2[dst] = make_uint2(v.a, (v.b & 0xFFFFu) | ph); if (nt == 2) a.tok2[dst + 1] = make_uint2(v.c, (v.d & 0xFFFFu) | ph); }
-                else { a.tok_id[dst] = v.a; if (nt == 2) a.tok_id[dst + 1] = v.c; }
+                // (the word's position in the slice goes into TW_REC_WIDE records only: it is read by the hf_compat mode of pass B
+                // that reports offsets relative to the document)
+                tw_put_token<REC>(a.tok, dst, v.a, v.b & 0xFFFFu, p << 16);
+                if (nt == 2) tw_put_token<REC>(a.tok, dst + 1, v.c, v.d & 0xFFFFu, p << 16);
             }
             // words with three or more tokens: listed now, copied from the pool at the end of the slice
             const uint32_t pooled = __ballot_sync(FULL, can_store && nt && (flags & TW_POOLF));
             if (pooled) {
                 const uint32_t np = __popc(pooled);
-                if (n_pl + np > 32) { tw_flush_pooled(a, sh.plist, n_pl); n_pl = 0; }
+                if (n_pl + np > 32) { tw_flush_pooled<REC>(a, sh.plist, n_pl); n_pl = 0; }
                 if ((pooled >> lane) & 1u) sh.plist[n_pl + __popc(pooled & lt_mask)] = make_uint4(v.a, nt, dst, p << 16);
                 n_pl += np;
             }
@@ -944,7 +962,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             if (have) sh.wlist[k] = (uint16_t)(run + ex);      // (the round's wlist entries were read at its top, before the votes)
             run += tot;
         }
-        if (n_pl) tw_flush_pooled(a, sh.plist, n_pl);
+        if (n_pl) tw_flush_pooled<REC>(a, sh.plist, n_pl);
         if (can_store) tcur += run;
         // long words -> one contiguous run of the long list
         uint32_t lfirst = 0;
@@ -1002,7 +1020,7 @@ __global__ void long_fix_kernel(const uint32_t* __restrict__ long_start, const u
 // ------------------------------------------------------------------ pass B
 struct SliceEmitArgs {
     const uint64_t* doc_off; uint32_t n_docs; uint32_t n_slices; const uint32_t* slice_doc_lo;
-    const uint32_t* tok_id; const uint2* tok2;     // ids only, or {id, start | end << 8} records
+    const void* tok;                              // the token stream (records of the kind TW_REC_*)
     const uint32_t* slice_tok_off; const uint32_t* slice_ntok_inline; const uint32_t* slice_long;
     const uint32_t* slice_tokbase;                // exclusive scan of the slice token counts (n_slices + 1)
     const uint32_t* long_start; const uint32_t* long_ins; const uint32_t* long_ntok;
@@ -1036,13 +1054,12 @@ __device__ __forceinline__ void te_put(const EmitParams& p, const EmitOut& o, un
 #ifndef TKZ_TE_UNROLL
 #define TKZ_TE_UNROLL 4
 #endif
-// copies the stream tokens [j0, j1) of a slice (stream position src + j) to dst0 + (j - j0); TKZ_TE_UNROLL loads in flight per lane
-template <uint32_t OUTS>
+// copies the stream tokens [j0, j1) of a slice (stream position src + j) to dst0 + (j - j0); TKZ_TE_UNROLL loads in flight per lane.
+// Every record kind decodes to the (id, start | end << 8 [| position << 16]) that te_put takes.
+template <uint32_t OUTS, int REC>
 __device__ __forceinline__ void te_copy(const SliceEmitArgs& a, const EmitParams& p, const EmitOut& o, size_t src, uint32_t j0, uint32_t j1,
                                         unsigned long long dst0, uint32_t hs = 0) {
     const uint32_t lane = lane_id();
-    const uint32_t outputs = OUTS ? OUTS : p.outputs;
-    const bool want_of = (outputs & (2u | 32u)) != 0;
     constexpr int TE_U = TKZ_TE_UNROLL;
     for (uint32_t j = j0 + lane; j < j1; j += 32 * TE_U) {
         uint32_t id[TE_U], of[TE_U];
@@ -1050,8 +1067,11 @@ __device__ __forceinline__ void te_copy(const SliceEmitArgs& a, const EmitParams
         for (int u = 0; u < TE_U; u++) { id[u] = 0; of[u] = 0; }
 #pragma unroll
         for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) {
-            if (want_of) { const uint2 r = __ldg(a.tok2 + src + j + 32 * u); id[u] = r.x; of[u] = r.y; }
-            else id[u] = __ldg(a.tok_id + src + j + 32 * u);
+            const size_t i = src + j + 32 * u;
+            if (REC == TW_REC_WIDE) { const uint2 r = __ldg(static_cast<const uint2*>(a.tok) + i); id[u] = r.x; of[u] = r.y; }
+            else if (REC == TW_REC4) { const uint32_t r = __ldg(static_cast<const uint32_t*>(a.tok) + i); id[u] = r & 0xFFFFu; of[u] = r >> 16; }
+            else if (REC == TW_REC_ID16) id[u] = __ldg(static_cast<const uint16_t*>(a.tok) + i);
+            else id[u] = __ldg(static_cast<const uint32_t*>(a.tok) + i);
         }
 #pragma unroll
         for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) te_put<OUTS>(p, o, dst0 + (j + 32 * u - j0), id[u], of[u], hs);
@@ -1060,7 +1080,8 @@ __device__ __forceinline__ void te_copy(const SliceEmitArgs& a, const EmitParams
 
 // PLAIN = no truncation and no padding: the output is the plain concatenation of all tokens in text order, so a token's
 // destination is its global index.  Otherwise the tokens of the slice are cut by the documents that meet the slice.
-template <bool PLAIN, uint32_t OUTS>
+// REC: the token stream's record kind, as pass A wrote it.
+template <bool PLAIN, uint32_t OUTS, int REC>
 __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(const __grid_constant__ SliceEmitArgs a, const __grid_constant__ EmitParams p,
                                                                 const __grid_constant__ EmitOut o) {
     const uint32_t FULL = 0xFFFFFFFFu;
@@ -1083,14 +1104,14 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
         const uint32_t d_lo = __shfl_sync(FULL, meta, 5), d_hi = __shfl_sync(FULL, meta, 6);
         meta = load_meta(s + stride);
         if (PLAIN) {
-            if (lg == 0) te_copy<OUTS>(a, p, o, src, 0, ntok, base);
+            if (lg == 0) te_copy<OUTS, REC>(a, p, o, src, 0, ntok, base);
             else {
                 // pieces: inline tokens up to the next long word's insertion index, then the long word (from the pool)
                 uint32_t j = 0; unsigned long long g = base;
                 const uint32_t lf = lg >> 3, ln = lg & 7u;
                 for (uint32_t i = 0; i <= ln; i++) {
                     const uint32_t jn = i < ln ? __ldg(a.long_ins + lf + i) : ntok;
-                    te_copy<OUTS>(a, p, o, src, j, jn, g);
+                    te_copy<OUTS, REC>(a, p, o, src, j, jn, g);
                     g += jn - j; j = jn;
                     if (i < ln) {
                         uint32_t cnt = __ldg(a.long_ntok + lf + i);
@@ -1129,7 +1150,7 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
                     const unsigned long long dbase = dto + shift;                                    // destination of the document's token 0
                     const uint32_t dbyte = __shfl_sync(FULL, my_dbyte, e);
                     const uint32_t hs = s * TW_SLICE - dbyte;                                        // (mod 2^32) slice start relative to the document
-                    if (ln == 0) te_copy<OUTS>(a, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs);
+                    if (ln == 0) te_copy<OUTS, REC>(a, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs);
                     else {
                         // slice-local real index r = g - base; pieces as in the PLAIN case, cut to [g0, g1)
                         uint32_t j = 0, r = 0;
@@ -1137,7 +1158,7 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
                             const uint32_t jn = i < ln ? __ldg(a.long_ins + lf + i) : ntok;
                             {   // inline piece: stream tokens [j, jn) = real indices [r, r + jn - j)
                                 const uint32_t lo = max(g0 - base, r), hi2 = min(g1 - base, r + (jn - j));
-                                if (lo < hi2) te_copy<OUTS>(a, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs);
+                                if (lo < hi2) te_copy<OUTS, REC>(a, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs);
                             }
                             r += jn - j; j = jn;
                             if (i < ln) {
