@@ -33,14 +33,12 @@ def assert_same(got: tz.BatchEncoding, ref: orc.BatchEncoding, what=""):
 MODES = ("slices", "lut", "occurrence")
 
 
-def pair(js, dedup=True, mode=None):
+def pair(js, mode="slices"):
     """(GPU tokenizer, oracle).  The context reads its pipeline switches when it is created: mode "slices" = the slice
     pipeline (tkz_slices.cuh, default: byte classes by packed range compares when the class table allows it), "lut" = the
     same pipeline with the per-byte class look-up forced (TKZ_CLASSIFY=lut), "occurrence" = the per-occurrence pipeline
-    (TKZ_NO_DEDUP=1; dedup=False is the older spelling).  All device pipelines are held to the same oracle."""
+    (TKZ_NO_DEDUP=1).  All device pipelines are held to the same oracle."""
     import os
-    if mode is None:
-        mode = "slices" if dedup else "occurrence"
     os.environ["TKZ_NO_DEDUP"] = "1" if mode == "occurrence" else "0"
     os.environ["TKZ_CLASSIFY"] = "lut" if mode == "lut" else "auto"
     try:
@@ -130,7 +128,7 @@ def test_truncation_and_padding(seed):
         js, alpha = rand_wp_json(rng)
     else:
         js, alpha = rand_bpe_json(rng, n_merges=30, pretok="Whitespace")
-    t, o = pair(js, dedup=seed % 4 != 3)
+    t, o = pair(js, mode="slices" if seed % 4 != 3 else "occurrence")
     docs = rand_docs(rng, alpha, 300, max_len=60)
     trunc = [None, 0, 1, 5, 8, 64][seed % 6]
     pad = [None, {"length": 8, "pad_id": 7, "pad_type_id": 3, "direction": "right"}, {"length": 5, "pad_id": 0, "direction": "left"},
@@ -160,7 +158,7 @@ def test_struct_chains(seed):
         js, alpha = rand_wp_json(rng, pretok=None, normalizer=None)
     else:
         js, alpha = rand_bpe_json(rng, n_merges=30, unk="<unk>" if seed % 4 == 0 else None)
-    t, o = pair(js, dedup=seed % 3 != 1)
+    t, o = pair(js, mode="slices" if seed % 3 != 1 else "occurrence")
     nn = [rng.choice(list(tzn)) for _ in range(rng.randint(0, 3))]
     fl = [rng.randint(0, 3) for _ in nn]
     pn = [rng.choice(list(tzp)) for _ in range(rng.randint(0, 3))]

@@ -76,12 +76,9 @@ struct tkz_ctx {
     DevBuf a_wtable, a_lscratch, a_tok_id;
     bool has_iso = false;                 // the class table isolates some byte (punctuation split)
     ClassRanges cr{}, cr_post{};          // byte classes as ranges (raw bytes / bytes already normalised by K0)
-    bool stage_bulk = true;               // TKZ_STAGE=ldg: pass A stages its slices with plain loads instead of bulk copies (A/B switch)
     bool narrow_records = true;           // TKZ_TOK_RECORD=wide: u32 ids in the token stream even for 16-bit vocabularies (A/B switch)
     // chunks of ONE host-buffer call share the word table and the record pool of the slice pipeline: the first chunk starts from an
-    // empty table, the later ones find the call's frequent words already tokenized (every call starts cold; TKZ_KEEP_TABLE=0
-    // gives every chunk its own table)
-    bool keep_table = true;               // switch
+    // empty table, the later ones find the call's frequent words already tokenized (every call starts cold)
     bool call_keep = false;               // inside a chunked host-buffer call
     bool kept_valid = false;              // the table of the previous chunk can be reused
     uint64_t call_bytes = 0;              // text bytes of the whole call (sizes the shared table)
@@ -283,9 +280,7 @@ extern "C" int tkz_ctx_create(int device, void* stream, uint64_t arena_hint_byte
     (void)arena_hint_bytes;
     if (const char* e = getenv("TKZ_NO_DEDUP")) ctx->use_dedup = !(e[0] == '1');     // A/B switch for the parity tests
     if (const char* e = getenv("TKZ_CLASSIFY")) ctx->force_lut = (e[0] == 'l');
-    if (const char* e = getenv("TKZ_STAGE")) ctx->stage_bulk = !(e[0] == 'l');
     if (const char* e = getenv("TKZ_TOK_RECORD")) ctx->narrow_records = !(e[0] == 'w');
-    if (const char* e = getenv("TKZ_KEEP_TABLE")) ctx->keep_table = e[0] != '0';
     if (const char* e = getenv("TKZ_NO_GRID")) ctx->use_grid = !(e[0] == '1');
     if (const char* e = getenv("TKZ_GRID_MIN_LEN")) { const long long v = atoll(e); if (v > (long long)BB_WARP_MAX) ctx->grid_min_len = (uint32_t)v; }
     {
@@ -500,30 +495,23 @@ extern "C" int tkz_model_upload(tkz_ctx* ctx, const tkz_model_desc* d) {
                 // r, i.e. entries (X, a) / (b, Z) with a rank below r (X, Z are then built by merges of even lower rank).  Window
                 // of the entry: wl = max nsym(X) over (X, a) with rank < r, wr = max nsym(Z) over (b, Z) with rank < r.  Early
                 // merges involve short symbols, so the pairs that merge in the first, populous steps get windows of 1-3 symbols
-                // (a rank-blind window is as wide as the longest token that ever joins the symbol: TKZ_WINDOWS=blind).
-                const bool blind = [] { const char* e = getenv("TKZ_WINDOWS"); return e && e[0] == 'b'; }();
-                const bool no_local_aa = [] { const char* e = getenv("TKZ_LOCAL_AA"); return e && e[0] == '0'; }();
-                m.local_aa = no_local_aa ? 0 : 1;
+                // (a rank-blind window would be as wide as the longest token that ever joins the symbol).
                 std::unordered_map<uint32_t, uint32_t> WL, WR;  // running max while the entries are visited in rank order
-                for (uint32_t sl : order) {
-                    const MergeEnt& e = mtab[sl];
-                    if (blind) { uint32_t& l = WL[e.second]; l = std::max(l, ns(e.first)); uint32_t& r = WR[e.first]; r = std::max(r, ns(e.second)); }
-                }
                 for (uint32_t sl : order) {                    // ascending rank: WL / WR hold exactly the entries of lower rank
                     const MergeEnt& e = mtab[sl];
                     auto get = [](std::unordered_map<uint32_t, uint32_t>& mp, uint32_t k) { auto it = mp.find(k); return it == mp.end() ? 0u : it->second; };
                     uint32_t wl = get(WL, e.first), wr = get(WR, e.second);     // threats to `first` from its left, to `second` from its right
                     // (A, A): the window is laid around the whole RUN of A and must also see an A that could still appear next
                     // to the run (it would change which A pairs with which): such an A is built from at most nsym(A) symbols
-                    if (e.first == e.second && !no_local_aa) { wl = std::max(wl, ns(e.first)); wr = std::max(wr, ns(e.first)); }
+                    if (e.first == e.second) { wl = std::max(wl, ns(e.first)); wr = std::max(wr, ns(e.first)); }
                     if (wl > 250 || wr > 250) { proper = false; break; }
                     win[sl] = (uint16_t)(wl | (wr << 8));
-                    if (!blind) { uint32_t& l = WL[e.second]; l = std::max(l, ns(e.first)); uint32_t& r = WR[e.first]; r = std::max(r, ns(e.second)); }
+                    uint32_t& l = WL[e.second]; l = std::max(l, ns(e.first)); uint32_t& r = WR[e.first]; r = std::max(r, ns(e.second));
                 }
                 if (getenv("TKZ_GRID_DEBUG") && !order.empty()) {
                     double sl_ = 0, sr_ = 0; uint32_t ml = 0, mr = 0;
                     for (uint32_t sl : order) { sl_ += win[sl] & 0xFF; sr_ += win[sl] >> 8; ml = std::max<uint32_t>(ml, win[sl] & 0xFF); mr = std::max<uint32_t>(mr, win[sl] >> 8); }
-                    fprintf(stderr, "[tkz upload] %zu merges, windows: mean left %.2f right %.2f, max left %u right %u (%s)\n", order.size(), sl_ / order.size(), sr_ / order.size(), ml, mr, blind ? "rank-blind" : "rank-aware");
+                    fprintf(stderr, "[tkz upload] %zu merges, windows: mean left %.2f right %.2f, max left %u right %u\n", order.size(), sl_ / order.size(), sr_ / order.size(), ml, mr);
                 }
             }
             TRY(upload(ctx, ctx->t_merge_win, win.data(), win.size() * 2));
@@ -626,9 +614,8 @@ int launch_bpe(tkz_ctx* ctx, const DevModel& m, const uint8_t* d_text, const uin
         if (ok) {
             GridBpeArgs ga{};
             ga.text = d_text; ga.word_start = word_start; ga.word_end = word_end;
-            ga.sparse_div = BG_SPARSE_DIV; ga.sparse_walk = BG_SPARSE_WALK;
+            ga.sparse_walk = BG_SPARSE_WALK;
             if (const char* e = getenv("TKZ_GRID_SPARSE_WALK")) ga.sparse_walk = (uint32_t)atoll(e);
-            if (const char* e = getenv("TKZ_GRID_SPARSE_DIV")) ga.sparse_div = (uint32_t)atoll(e);
             ga.hw = (const uint32_t*)ctx->a_huge_w.p; ga.hbase = (const uint32_t*)ctx->a_huge_base.p; ga.n_huge = (uint32_t)n_huge; ga.M = (uint32_t)M;
             uint8_t* p = (uint8_t*)ctx->a_grid_state.p;
             auto take = [&](size_t bytes) { uint8_t* r = p; p += bytes; return r; };
@@ -908,7 +895,6 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ta.n_words = ctrl + 10; ta.n_uniq = (unsigned int*)(ctrl + 6); ta.n_uncached = (unsigned int*)(ctrl + 6) + 1;
     ta.cr = cr;
     ta.n_bulk = N >= (uint64_t)(TW_SLICE + TW_POST) ? (uint32_t)std::min<uint64_t>(n_slices, (N - (TW_SLICE + TW_POST)) / TW_SLICE + 1) : 0u;
-    ta.stage_bulk = ctx->stage_bulk ? 1 : 0;
     ta.has_iso = ctx->has_iso ? 1 : 0;
     const int cls = (cr.usable && !ctx->force_lut) ? (cr.norm_lower ? 1 : 0) : (m.norm_identity ? 2 : 3);
     if (m.kind == TKZ_MODEL_BPE) launch_slice_words<TKZ_MODEL_BPE>(m, ta, cls, rec, grid, st);
@@ -1324,7 +1310,7 @@ int encode_host_chunked(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_o
     uint64_t chunk_target = ctx->chunk_bytes;
     const uint64_t chunk_max = std::min<uint64_t>(ctx->chunk_bytes * 8, 1ull << 30);
     struct KeepGuard { tkz_ctx* c; ~KeepGuard() { c->call_keep = false; c->kept_valid = false; c->call_bytes = 0; } } keep_guard{ctx};
-    ctx->call_keep = ctx->keep_table; ctx->kept_valid = false; ctx->call_bytes = N; ctx->call_uniq = 0;
+    ctx->call_keep = true; ctx->kept_valid = false; ctx->call_bytes = N; ctx->call_uniq = 0;
     cb.push_back(next_boundary(0, chunk_target));
     tkz_encode_params P{};
     if (params_in) P = *params_in;

@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(NT, MINB) bpe_block_kernel(DevModel m, BlockBp
                         for (uint32_t j = lo; j < i && head; j++) head = rk[j] >= r;
                         for (uint32_t j = i + 1; j <= hi && head; j++) head = rk[j] >= r;
                         // an equal rank inside the window is another occurrence of the same pair: it cannot overlap (a != b)
-                    } else if (r != TKZ_NONE && m.local_aa) {
+                    } else if (r != TKZ_NONE) {
                         // (A, A): the window goes around the whole run of A (its extent is part of the decision: the run
                         // pairs up from its start).  Nothing of lower rank left of the run within wl pairs, nor from the pair
                         // of its last A on within wr pairs => no A of the run is consumed and no A joins it before round r

@@ -48,7 +48,6 @@ struct GridBpeArgs {
     const uint32_t* hbase;                // huge word h -> first byte in the concatenation   (n_huge + 1, last = M)
     uint32_t n_huge, M;
     uint32_t sparse_walk;                 // longest run walk of the sparse phase (TKZ_GRID_SPARSE_WALK)
-    uint32_t sparse_div;                  // sparse phase below n / sparse_div ranked pairs (0: dense steps only; TKZ_GRID_SPARSE_DIV)
     uint32_t* id[2]; uint32_t* s[2]; uint32_t* e[2]; uint32_t* rk[2]; uint32_t* wid[2]; uint16_t* win[2];
     uint32_t* hn;                         // per symbol: TKZ_NONE, BG_PENDING, or the new id of the pair it heads
     uint32_t* wmin[2];                    // per huge word: smallest pair rank (double-buffered by step parity)
@@ -285,7 +284,7 @@ __global__ void __launch_bounds__(BG_NT, 1) bpe_grid_kernel(const __grid_constan
                             c = 0;
                             while (c < BG_WALK && e0 < n && rk[e0 - 1] != TKZ_BOUNDARY && ids[e0] == x) { e0++; c++; }
                             const bool ropen = e0 < n && rk[e0 - 1] != TKZ_BOUNDARY && ids[e0] == x;
-                            if (m.local_aa && !lopen && !ropen) {
+                            if (!lopen && !ropen) {
                                 if (((i - s0) & 1u) == 0) {
                                     const uint32_t wv = ((k < 2 ? w2.x : w2.y) >> ((k & 1) * 16)) & 0xFFFFu, wl = wv & 0xFFu, wr = wv >> 8;
                                     const uint32_t jlo = s0 > wl ? s0 - wl : 0;
@@ -465,7 +464,7 @@ __global__ void __launch_bounds__(BG_NT, 1) bpe_grid_kernel(const __grid_constan
         // Scratch = the arrays of the other buffer: pair lists, dstep, hstep (step in which hn[i] was written).
         const uint32_t n_live = *(volatile uint32_t*)(a.gs + 22 + (par ^ 1u));
         if (gt == 0 && step < 256) a.dbg[1024 + step] = n_live;
-        if (a.sparse_div != 0u && (unsigned long long)n_live * a.sparse_div < n && n_live != 0u) {
+        if ((unsigned long long)n_live * BG_SPARSE_DIV < n && n_live != 0u) {
             const uint32_t nxt = cur ^ 1u;
             uint32_t* const ids2 = a.id[cur]; uint32_t* const rk2 = a.rk[cur]; uint32_t* const wd2 = a.wid[cur]; uint16_t* const win2 = a.win[cur];
             uint32_t* const ev2 = a.e[cur];
@@ -525,7 +524,7 @@ __global__ void __launch_bounds__(BG_NT, 1) bpe_grid_kernel(const __grid_constan
                             if (c2 == BG_WALK) { ropen = true; break; }
                             last = nq; c2++;
                         }
-                        if (m.local_aa && !lopen && !ropen) {
+                        if (!lopen && !ropen) {
                             if ((c & 1u) == 0) {
                                 const uint32_t wv = win2[i], wl = wv & 0xFFu, wr = wv >> 8;
                                 head = true;

@@ -69,7 +69,6 @@ struct DevModel {
     // windowed schedule (tkz_bpe_block.cuh): per merge-table slot, how far a competing merge can reach: low byte = WL of the
     // pair's first symbol, high byte = WR of its second symbol; valid only when windowed_ok (table proven "proper" at upload)
     const uint16_t* merge_win; int windowed_ok;
-    int local_aa;                    // equal-symbol pairs may merge by the run-window rule (tkz_bpe_block.cuh); 0: only at the word's minimum rank
     int has_unk; uint32_t unk_id;
     // WordPiece
     const WpEnt* wp_tab; uint32_t wp_mask;

@@ -44,12 +44,9 @@ namespace tkz {
 
 constexpr int TW_THREADS = 256, TW_WARPS = 8, TW_SEG = 32, TW_SLICE = 32 * TW_SEG;      // slice = 1 KiB = one 32-byte segment per lane
 constexpr int TW_PRE = 16, TW_POST = 48, TW_STAGE = TW_PRE + TW_SLICE + TW_POST;         // staged window: 16 B before, 48 B behind the slice
-#ifndef TKZ_BPS
-#define TKZ_BPS 3
-#endif
-constexpr int TW_BLOCKS_PER_SM = TKZ_BPS;          // pass A: 3 blocks of 8 warps -> 80 registers per thread and ~150 KB of shared memory per SM, which leaves
+constexpr int TW_BLOCKS_PER_SM = 3;                // pass A: 3 blocks of 8 warps -> 80 registers per thread and ~150 KB of shared memory per SM, which leaves
                                                    // ~90 KB of L1 for the table probes; 4 blocks -> 64 registers: the round loop spills (B200, c2b 1 GiB: 4.93 ms
-                                                   // against 4.25; build-time A/B: TKZ_NVCC_FLAGS=-DTKZ_BPS=4)
+                                                   // against 4.25)
 constexpr uint32_t TW_TOK_CHUNK = 16384;           // tokens a warp claims from the token stream with one atomic (then sub-allocates)
 constexpr uint32_t TW_SLICE_TOK_MAX = TW_SLICE + 256;   // tokens the words that start in one slice can have (<= their bytes)
 constexpr uint32_t TW_MAX_SHORT = 15;             // bytes next to the length byte in the 128-bit key
@@ -118,7 +115,6 @@ struct SliceArgs {
     unsigned long long* n_words; unsigned int* n_uniq; unsigned int* n_uncached;
     ClassRanges cr;
     int has_iso;                                  // some byte is its own pre-token (punctuation split)
-    int stage_bulk;                               // 1: slices arrive by cp.async.bulk (default); 0: 16-byte loads per lane (TKZ_STAGE=ldg, A/B switch)
 };
 
 // first document that starts at or after each tile (slice) start; entry n_tiles = n_docs + 1.  One thread per tile.
@@ -173,12 +169,6 @@ __device__ __forceinline__ void tw_ld256(const WordSlot* s, uint32_t (&r)[8]) {
 __device__ __forceinline__ void tw_ld256_cg(const void* s, uint32_t (&r)[8]) {
     asm volatile("ld.global.cg.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "l"(s) : "memory");
-}
-// text read by plain loads (A/B path, tails): 16 bytes that do not allocate in L1
-__device__ __forceinline__ uint4 tw_ld_text16(const uint4* p) {
-    uint4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-    return v;
 }
 __device__ __forceinline__ uint4 tw_ld_value(const WordSlot* s) {
     uint4 v;
@@ -672,7 +662,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
     uint32_t tcur = 0, tend = 0;                                // the warp's current chunk of the token stream
     uint32_t buf = 0, phase = 0;                                // staging window in use, parity bits of the two mbarriers
     uint32_t words_total = 0;
-    if (lane == 0 && a.stage_bulk && bulk_ok(s)) issue(s, 0);
+    if (lane == 0 && bulk_ok(s)) issue(s, 0);
     for (; s < a.n_slices; s += stride, buf ^= 1u) {
         const uint64_t slice_base = (uint64_t)s * TW_SLICE;
         const uint32_t d_lo = __shfl_sync(FULL, meta, 0);
@@ -682,7 +672,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
         uint32_t* const tw = rawb + TW_PRE / 4;                    // word 0 = bytes 0..3 of the slice
         uint8_t* const tb = reinterpret_cast<uint8_t*>(tw);
         // the warp's next slice goes into the other window now (its readers finished at the end of the previous iteration)
-        if (lane == 0 && a.stage_bulk && bulk_ok(s + stride)) {
+        if (lane == 0 && bulk_ok(s + stride)) {
             if (!NORM_ID) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the window was normalised in place
             issue(s + stride, buf ^ 1u);
         }
@@ -696,18 +686,8 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             atomicOr(&sh.docbits[p >> 5], 1u << (p & 31));
         }
         const bool tail = !bulk_ok(s);
-        if (!tail && a.stage_bulk) { tw_mbar_wait(&sh.bar[buf], (phase >> buf) & 1u); phase ^= 1u << buf; }
-        else if (!tail) {
-            // A/B path: the window by 16-byte loads (two per lane for the slice, lanes 0..3 the 16 bytes before and 48 behind)
-            const uint4* g = reinterpret_cast<const uint4*>(a.text + slice_base);
-            uint4* d4 = reinterpret_cast<uint4*>(tw);
-            const uint4 v0 = tw_ld_text16(g + 2 * lane), v1 = tw_ld_text16(g + 2 * lane + 1);
-            uint4 hv = make_uint4(0, 0, 0, 0);
-            if (lane < 4 && (lane > 0 || slice_base > 0)) hv = tw_ld_text16(lane == 0 ? g - 1 : g + 63 + lane);
-            d4[2 * lane] = v0; d4[2 * lane + 1] = v1;
-            if (lane < 4) d4[lane == 0 ? -1 : 63 + (int)lane] = hv;
-            __syncwarp();
-        } else {
+        if (!tail) { tw_mbar_wait(&sh.bar[buf], (phase >> buf) & 1u); phase ^= 1u << buf; }
+        else {
             // bytes at or beyond n read as 0 and are masked out of the class bits below
             for (uint32_t i = lane; i < TW_STAGE / 4; i += 32) {
                 uint32_t v = 0;
@@ -1051,16 +1031,13 @@ __device__ __forceinline__ void te_put(const EmitParams& p, const EmitOut& o, un
     if (outputs & 128u) o.spans[dst] = make_uint4(id, s, e, ty & 0xFFu);
 }
 
-#ifndef TKZ_TE_UNROLL
-#define TKZ_TE_UNROLL 4
-#endif
-// copies the stream tokens [j0, j1) of a slice (stream position src + j) to dst0 + (j - j0); TKZ_TE_UNROLL loads in flight per lane.
+// copies the stream tokens [j0, j1) of a slice (stream position src + j) to dst0 + (j - j0); TE_U loads in flight per lane.
 // Every record kind decodes to the (id, start | end << 8 [| position << 16]) that te_put takes.
 template <uint32_t OUTS, int REC>
 __device__ __forceinline__ void te_copy(const SliceEmitArgs& a, const EmitParams& p, const EmitOut& o, size_t src, uint32_t j0, uint32_t j1,
                                         unsigned long long dst0, uint32_t hs = 0) {
     const uint32_t lane = lane_id();
-    constexpr int TE_U = TKZ_TE_UNROLL;
+    constexpr int TE_U = 4;                     // B200, c2b 1 GiB: pass B 1.42 ms with 2, 1.25 ms with 4 or 8
     for (uint32_t j = j0 + lane; j < j1; j += 32 * TE_U) {
         uint32_t id[TE_U], of[TE_U];
 #pragma unroll
