@@ -862,7 +862,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     TRY(ensure(ctx, ctx->a_wtable, ((size_t)tcap + mcap) * sizeof(WordSlot) + (size_t)m32cap * sizeof(WordSlot32)));
     TRY(ensure(ctx, ctx->a_upool, (size_t)upool_cap * 8));
     TRY(ensure(ctx, ctx->a_lscratch, (size_t)warps * 4 * 256 * 4));
-    TRY(ensure(ctx, ctx->a_tok_id, (size_t)tok_cap * rec_bytes));
+    TRY(ensure(ctx, ctx->a_tok_id, (size_t)tok_cap * rec_bytes + 16));     // (pass B copies whole 16-byte units around each run)
     TRY(ensure(ctx, ctx->a_tile_tok_off, ((size_t)n_slices + 2) * 4));
     TRY(ensure(ctx, ctx->a_tile_ntok_inline, ((size_t)n_slices + 2) * 4));
     TRY(ensure(ctx, ctx->a_tile_ntok, ((size_t)n_slices + 2) * 4));

@@ -1031,40 +1031,181 @@ __device__ __forceinline__ void te_put(const EmitParams& p, const EmitOut& o, un
     if (outputs & 128u) o.spans[dst] = make_uint4(id, s, e, ty & 0xFFu);
 }
 
-// copies the stream tokens [j0, j1) of a slice (stream position src + j) to dst0 + (j - j0); TE_U loads in flight per lane.
-// Every record kind decodes to the (id, start | end << 8 [| position << 16]) that te_put takes.
-template <uint32_t OUTS, int REC>
-__device__ __forceinline__ void te_copy(const SliceEmitArgs& a, const EmitParams& p, const EmitOut& o, size_t src, uint32_t j0, uint32_t j1,
-                                        unsigned long long dst0, uint32_t hs = 0) {
-    const uint32_t lane = lane_id();
-    constexpr int TE_U = 4;                     // B200, c2b 1 GiB: pass B 1.42 ms with 2, 1.25 ms with 4 or 8
-    for (uint32_t j = j0 + lane; j < j1; j += 32 * TE_U) {
-        uint32_t id[TE_U], of[TE_U];
-#pragma unroll
-        for (int u = 0; u < TE_U; u++) { id[u] = 0; of[u] = 0; }
-#pragma unroll
-        for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) {
-            const size_t i = src + j + 32 * u;
-            if (REC == TW_REC_WIDE) { const uint2 r = __ldg(static_cast<const uint2*>(a.tok) + i); id[u] = r.x; of[u] = r.y; }
-            else if (REC == TW_REC4) { const uint32_t r = __ldg(static_cast<const uint32_t*>(a.tok) + i); id[u] = r & 0xFFFFu; of[u] = r >> 16; }
-            else if (REC == TW_REC_ID16) id[u] = __ldg(static_cast<const uint16_t*>(a.tok) + i);
-            else id[u] = __ldg(static_cast<const uint32_t*>(a.tok) + i);
+// Pass B reads the token stream through two windows of TE_WIN bytes per warp in shared memory, filled by bulk copies
+// (cp.async.bulk + mbarrier, as pass A stages its text).  While the warp writes the tokens of one window the next one is
+// in flight: the rest of the slice's run, else the first window of the warp's next slice.  A window starts at the 16-byte
+// boundary at or below the first record asked for, so a run needs no alignment in the stream; the neighbouring records a
+// window holds as well are never written out.  (B200, c2b 1 GiB: per-lane loads of 4 records, 4 in flight, issued only
+// after the previous slice was written, took 1.20 ms of pass B; see DESIGN 4.1 for this version.)
+constexpr uint32_t TE_WIN = 1024;
+
+__shared__ __align__(128) unsigned char te_smem[TW_WARPS][2 * TE_WIN + 16];   // per warp: two windows, their mbarriers
+
+template <int REC>
+struct TeWindows {
+    static constexpr uint32_t RB = REC == TW_REC_WIDE ? 8 : (REC == TW_REC_ID16 ? 2 : 4);   // bytes per record
+    static constexpr uint32_t RPG = 16 / RB, RPW = TE_WIN / RB;                             // records per 16 bytes, per window
+    uint32_t cur, clo, chi;              // the window being read and the records [clo, chi) it holds
+    uint32_t nlo, nhi, npend;            // the other window: its records, whether its copy is in flight
+    uint32_t phase;                      // parity bits of the two mbarriers
+    uint32_t run_end, next_lo, next_hi;  // end of the current slice's run; the run of the warp's next slice
+
+    __device__ __forceinline__ unsigned char* win() const { return te_smem[threadIdx.x >> 5]; }
+    __device__ __forceinline__ unsigned long long* bar() const { return reinterpret_cast<unsigned long long*>(win() + 2 * TE_WIN); }
+    // records [lo, hi) of the stream tok (as many as fit) into the other window; warp-uniform, that window is idle
+    __device__ __forceinline__ void issue(const void* tok, uint32_t lo, uint32_t hi) {
+        const uint32_t b = cur ^ 1u, a0 = lo & ~(RPG - 1u), a1 = min(a0 + RPW, (hi + RPG - 1u) & ~(RPG - 1u));
+        nlo = a0; nhi = a1; npend = 1;
+        __syncwarp();                    // every lane is done reading the window
+        if (lane_id() == 0) tw_bulk_load(win() + b * TE_WIN, static_cast<const unsigned char*>(tok) + (size_t)a0 * RB, (a1 - a0) * RB, bar() + b);
+    }
+    // the copy in flight becomes the window being read; then the next window this warp will need goes in flight
+    __device__ __forceinline__ void advance(const void* tok) {
+        const uint32_t b = cur ^ 1u;
+        tw_mbar_wait(bar() + b, (phase >> b) & 1u);
+        phase ^= 1u << b;
+        cur = b; clo = nlo; chi = nhi; npend = 0;
+        if (chi < run_end) issue(tok, chi, run_end);
+        else if (next_lo < next_hi) issue(tok, next_lo, next_hi);
+    }
+    // make the window being read hold record r of the current slice's run (warp-uniform)
+    __device__ __forceinline__ void ensure(const void* tok, uint32_t r) {
+        if (r - clo < chi - clo) return;
+        if (npend && r - nlo < nhi - nlo) { advance(tok); return; }
+        if (npend) {                     // a window that is not needed: drained.  (The plain kernel asks for a slice's records
+                                         // in increasing order, starting at its run, so it never gets here; kept so that any
+                                         // order of requests stays correct.)
+            const uint32_t b = cur ^ 1u;
+            tw_mbar_wait(bar() + b, (phase >> b) & 1u);
+            phase ^= 1u << b; npend = 0;
         }
+        issue(tok, r, run_end);
+        advance(tok);
+    }
+    __device__ __forceinline__ void drain() {
+        if (npend) { const uint32_t b = cur ^ 1u; tw_mbar_wait(bar() + b, (phase >> b) & 1u); npend = 0; }
+        __syncwarp();
+    }
+};
+
+// record q of a window -> (id, start | end << 8 [| position << 16]), the form te_put takes
+template <int REC>
+__device__ __forceinline__ void te_rec(const unsigned char* w, uint32_t q, uint32_t& id, uint32_t& of) {
+    if (REC == TW_REC_WIDE) { const uint2 r = reinterpret_cast<const uint2*>(w)[q]; id = r.x; of = r.y; }
+    else if (REC == TW_REC4) { const uint32_t r = reinterpret_cast<const uint32_t*>(w)[q]; id = r & 0xFFFFu; of = r >> 16; }
+    else if (REC == TW_REC_ID16) { id = reinterpret_cast<const uint16_t*>(w)[q]; of = 0; }
+    else { id = reinterpret_cast<const uint32_t*>(w)[q]; of = 0; }
+}
+
+// ids + offsets + attention of 4 tokens at a 4-aligned destination slot: 16-byte stores (offsets: two of them)
+__device__ __forceinline__ void te_put4(const EmitParams& p, const EmitOut& o, unsigned long long dst, const uint32_t (&id)[4], const uint32_t (&of)[4],
+                                        uint32_t hs) {
+    uint32_t s[4], e[4];
 #pragma unroll
-        for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) te_put<OUTS>(p, o, dst0 + (j + 32 * u - j0), id[u], of[u], hs);
+    for (int u = 0; u < 4; u++) {
+        s[u] = of[u] & 0xFFu; e[u] = (of[u] >> 8) & 0xFFu;
+        if (p.hf_flags & 2u) { const uint32_t b = hs + (of[u] >> 16); s[u] += b; e[u] += b; }
+    }
+    *reinterpret_cast<uint4*>(o.ids + dst) = make_uint4(id[0], id[1], id[2], id[3]);
+    reinterpret_cast<uint4*>(o.offsets + 2 * dst)[0] = make_uint4(s[0], e[0], s[1], e[1]);
+    reinterpret_cast<uint4*>(o.offsets + 2 * dst)[1] = make_uint4(s[2], e[2], s[3], e[3]);
+    *reinterpret_cast<uint4*>(o.attention + dst) = make_uint4(1u, 1u, 1u, 1u);
+}
+
+// n tokens whose records start at index q0 of window w -> destination slots d0 .. d0 + n - 1.  Ids + offsets + attention:
+// 4 tokens per lane at 4-aligned slots, the head and tail groups that the range only partly covers token by token (source
+// and destination alignment differ freely: the records are read from shared memory at any index).  The generic form:
+// te_put per token.
+template <uint32_t OUTS, int REC>
+__device__ __forceinline__ void te_store(const EmitParams& p, const EmitOut& o, const unsigned char* w, uint32_t q0, uint32_t n, unsigned long long d0,
+                                         uint32_t hs) {
+    constexpr bool VEC = OUTS == 7u;
+    constexpr uint32_t U = 4;
+    const uint32_t lane = lane_id();
+    if (!VEC) {
+        for (uint32_t k = lane; k < n; k += 32) { uint32_t id, of; te_rec<REC>(w, q0 + k, id, of); te_put<OUTS>(p, o, d0 + k, id, of, hs); }
+        return;
+    }
+    const uint32_t head = (uint32_t)d0 & (U - 1u);          // slots of the first group before d0
+    const uint32_t ng = (head + n + U - 1u) / U;
+    for (uint32_t g = lane; g < ng; g += 32) {
+        const uint32_t k0 = g * U - head;                   // (mod 2^32) token of the group's first slot
+        if ((g > 0 || head == 0) && k0 + U <= n) {
+            uint32_t id[U], of[U];
+#pragma unroll
+            for (uint32_t u = 0; u < U; u++) te_rec<REC>(w, q0 + k0 + u, id[u], of[u]);
+            te_put4(p, o, d0 + k0, id, of, hs);
+        } else {
+#pragma unroll
+            for (uint32_t u = 0; u < U; u++) {
+                const uint32_t k = k0 + u;
+                if (k < n) { uint32_t id, of; te_rec<REC>(w, q0 + k, id, of); te_put<OUTS>(p, o, d0 + k, id, of, hs); }
+            }
+        }
+    }
+}
+
+// which kernels take the staged copy: without truncation / padding, ids + offsets + attention (16 B per token) and the
+// generic form.  The rest keep per-lane loads at 8 (5) blocks per SM, which measured faster for them (B200, 1000 W):
+// c2b 1 GiB pass B ids only 0.345 ms against 0.384 staged, ids16 + packed offsets 0.466 against 0.526; the c3 hf_compat
+// step 32.6 ms against 33.4 with the staged truncation / padding form (4 blocks per SM, 8-byte records spill there)
+template <bool PLAIN, uint32_t OUTS>
+__host__ __device__ constexpr bool te_staged() { return PLAIN && (OUTS == 7u || OUTS == 0u); }
+
+// copies the stream tokens [j0, j1) of a slice whose run starts at stream position src to dst0 + (j - j0): window by
+// window, or with TE_U loads in flight per lane for the forms that are not staged
+template <bool STAGED, uint32_t OUTS, int REC>
+__device__ __forceinline__ void te_copy(TeWindows<REC>& w, const void* tok, const EmitParams& p, const EmitOut& o, uint32_t src, uint32_t j0, uint32_t j1,
+                                        unsigned long long dst0, uint32_t hs = 0) {
+    if (!STAGED) {
+        const uint32_t lane = lane_id();
+        constexpr int TE_U = 4;                     // B200, c2b 1 GiB: pass B 1.42 ms with 2, 1.25 ms with 4 or 8 (8-byte records)
+        for (uint32_t j = j0 + lane; j < j1; j += 32 * TE_U) {
+            uint32_t id[TE_U], of[TE_U];
+#pragma unroll
+            for (int u = 0; u < TE_U; u++) { id[u] = 0; of[u] = 0; }
+#pragma unroll
+            for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) {
+                const size_t i = (size_t)src + j + 32 * u;
+                if (REC == TW_REC_WIDE) { const uint2 r = __ldg(static_cast<const uint2*>(tok) + i); id[u] = r.x; of[u] = r.y; }
+                else if (REC == TW_REC4) { const uint32_t r = __ldg(static_cast<const uint32_t*>(tok) + i); id[u] = r & 0xFFFFu; of[u] = r >> 16; }
+                else if (REC == TW_REC_ID16) id[u] = __ldg(static_cast<const uint16_t*>(tok) + i);
+                else id[u] = __ldg(static_cast<const uint32_t*>(tok) + i);
+            }
+#pragma unroll
+            for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) te_put<OUTS>(p, o, dst0 + (j + 32 * u - j0), id[u], of[u], hs);
+        }
+        return;
+    }
+    uint32_t r = src + j0;
+    const uint32_t r1 = src + j1;
+    while (r < r1) {
+        w.ensure(tok, r);
+        const uint32_t re = min(r1, w.chi);
+        te_store<OUTS, REC>(p, o, w.win() + w.cur * TE_WIN, r - w.clo, re - r, dst0 + (r - (src + j0)), hs);
+        r = re;
     }
 }
 
 // PLAIN = no truncation and no padding: the output is the plain concatenation of all tokens in text order, so a token's
 // destination is its global index.  Otherwise the tokens of the slice are cut by the documents that meet the slice.
 // REC: the token stream's record kind, as pass A wrote it.
+// Staged forms: 4 blocks of 8 warps per SM (64 registers, no spill).  At 5 blocks (48 registers) and 6 (40) they spill, and
+// pass B measured 1.11 and 1.17 ms against 0.99 (B200, c2b 1 GiB): the windows in flight hide the loads without more warps.
 template <bool PLAIN, uint32_t OUTS, int REC>
-__global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(const __grid_constant__ SliceEmitArgs a, const __grid_constant__ EmitParams p,
+__global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PLAIN ? 8 : 5)) slice_emit_kernel(const __grid_constant__ SliceEmitArgs a, const __grid_constant__ EmitParams p,
                                                                 const __grid_constant__ EmitOut o) {
+    constexpr bool STAGED = te_staged<PLAIN, OUTS>();
     const uint32_t FULL = 0xFFFFFFFFu;
     const uint32_t lane = lane_id(), wid = threadIdx.x >> 5;
     const uint32_t stride = gridDim.x * TW_WARPS;
-    // slice metadata is fetched one slice ahead: lanes 0..6 hold ntok_inline, tok_off, tokbase, tokbase[+1], long, doc_lo, doc_lo[+1]
+    TeWindows<REC> w;
+    if (STAGED && lane == 0) { tw_mbar_init(w.bar()); tw_mbar_init(w.bar() + 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+    __syncwarp();
+    w.cur = 0; w.clo = w.chi = 0; w.nlo = w.nhi = 0; w.npend = 0; w.phase = 0;
+    // slice metadata is fetched one slice ahead, two for the staged forms (the token window of the next slice is issued while
+    // this one is written):
+    // lanes 0..6 hold ntok_inline, tok_off, tokbase, tokbase[+1], long, doc_lo, doc_lo[+1]
     auto load_meta = [&](uint32_t s) -> uint32_t {
         if (s >= a.n_slices || lane >= 7) return 0u;
         const uint32_t* src = lane == 0 ? a.slice_ntok_inline + s : (lane == 1 ? a.slice_tok_off + s : (lane < 4 ? a.slice_tokbase + s + (lane - 2)
@@ -1072,23 +1213,25 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
         return __ldg(src);
     };
     uint32_t s = blockIdx.x * TW_WARPS + wid;
-    uint32_t meta = load_meta(s);
+    uint32_t meta = load_meta(s), meta_next = STAGED ? load_meta(s + stride) : 0u;
     for (; s < a.n_slices; s += stride) {
         const uint32_t ntok = __shfl_sync(FULL, meta, 0);
-        const size_t src = __shfl_sync(FULL, meta, 1);
+        const uint32_t src = __shfl_sync(FULL, meta, 1);
         const uint32_t base = __shfl_sync(FULL, meta, 2), base_next = __shfl_sync(FULL, meta, 3);
         const uint32_t lg = __shfl_sync(FULL, meta, 4);
         const uint32_t d_lo = __shfl_sync(FULL, meta, 5), d_hi = __shfl_sync(FULL, meta, 6);
-        meta = load_meta(s + stride);
+        if (STAGED) { meta = meta_next; meta_next = load_meta(s + 2 * stride); }
+        else meta = load_meta(s + stride);
+        if (STAGED) { w.run_end = src + ntok; w.next_lo = __shfl_sync(FULL, meta, 1); w.next_hi = w.next_lo + __shfl_sync(FULL, meta, 0); }
         if (PLAIN) {
-            if (lg == 0) te_copy<OUTS, REC>(a, p, o, src, 0, ntok, base);
+            if (lg == 0) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, 0, ntok, base);
             else {
                 // pieces: inline tokens up to the next long word's insertion index, then the long word (from the pool)
                 uint32_t j = 0; unsigned long long g = base;
                 const uint32_t lf = lg >> 3, ln = lg & 7u;
                 for (uint32_t i = 0; i <= ln; i++) {
                     const uint32_t jn = i < ln ? __ldg(a.long_ins + lf + i) : ntok;
-                    te_copy<OUTS, REC>(a, p, o, src, j, jn, g);
+                    te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, j, jn, g);
                     g += jn - j; j = jn;
                     if (i < ln) {
                         uint32_t cnt = __ldg(a.long_ntok + lf + i);
@@ -1127,7 +1270,7 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
                     const unsigned long long dbase = dto + shift;                                    // destination of the document's token 0
                     const uint32_t dbyte = __shfl_sync(FULL, my_dbyte, e);
                     const uint32_t hs = s * TW_SLICE - dbyte;                                        // (mod 2^32) slice start relative to the document
-                    if (ln == 0) te_copy<OUTS, REC>(a, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs);
+                    if (ln == 0) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs);
                     else {
                         // slice-local real index r = g - base; pieces as in the PLAIN case, cut to [g0, g1)
                         uint32_t j = 0, r = 0;
@@ -1135,7 +1278,7 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
                             const uint32_t jn = i < ln ? __ldg(a.long_ins + lf + i) : ntok;
                             {   // inline piece: stream tokens [j, jn) = real indices [r, r + jn - j)
                                 const uint32_t lo = max(g0 - base, r), hi2 = min(g1 - base, r + (jn - j));
-                                if (lo < hi2) te_copy<OUTS, REC>(a, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs);
+                                if (lo < hi2) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs);
                             }
                             r += jn - j; j = jn;
                             if (i < ln) {
@@ -1159,6 +1302,7 @@ __global__ void __launch_bounds__(TW_THREADS, PLAIN ? 8 : 5) slice_emit_kernel(c
             }
         }
     }
+    if (STAGED) w.drain();        // no bulk copy may still write into the block's shared memory when it exits
 }
 
 // per document: global token index of its start, real token count, output slot count (feeds the scan -> CSR offsets)
