@@ -107,6 +107,13 @@ typedef struct tkz_model_desc {
 /* SpanToken records (src/token.zig:11-76): 16 bytes per slot {id u32, start u32, end u32, type_id u8, flags u8, pad u16} in
  * tkz_batch_result.span_tokens; flags bit 2 = is_padding (SpanToken.initPadding), the other flags are never set by the path */
 #define TKZ_OUT_SPAN_TOKENS 128u
+/* Word ids (Hugging Face Encoding.word_ids for a single sequence) in tkz_batch_result.word_ids: for every real token the
+ * ordinal of the pre-token that produced it among the pre-tokens of its document, counting from 0.  A pre-token that yields
+ * no token still uses up its index; without a pre-tokenizer every token has word id 0; template special tokens and padding
+ * slots get 0xFFFFFFFF; truncation keeps the kept tokens' word ids.  Works with any hf_flags (in reference mode the pieces of
+ * the pre-tokenizer are the words).  Not part of TKZ_OUT_ALL.  TKZ_ERR_INVALID_ARG with `fast`, in the compact result
+ * (tkz_encode_batch_compact / tkzm_encode_batch_compact), and with a model whose largest id is 2^22 or more. */
+#define TKZ_OUT_WORD_IDS 256u
 
 /* Per-call knobs = the public fields Tokenizer.truncation / Tokenizer.padding (src/lib.zig:41-42,149-157;
  * src/types.zig:39-45,55-59).  stride / strategy / pad_token are ignored by the reference's encode. */
@@ -167,6 +174,7 @@ typedef struct tkz_batch_result {
      * 32-bit offsets for every token instead, as a call without pre-tokenizer does.) */
     uint64_t n_wide;
     const uint32_t* wide_tokens;
+    const uint32_t* word_ids;           /* n_tokens, see TKZ_OUT_WORD_IDS; 0xFFFFFFFF for special tokens and padding */
 } tkz_batch_result;
 
 /* counters of the last encode (FastTokenizer.arenaMemoryUsage analogue, src/lib.zig:451-453) */

@@ -33,6 +33,8 @@ OUT_IDS, OUT_OFFSETS, OUT_ATTENTION, OUT_TYPE_IDS, OUT_SPECIAL, OUT_ALL = 1, 2, 
 OUT_SPAN_TOKENS = 128            # 16-byte SpanToken records (src/token.zig:19-33)
 OUT_IDS_U16 = 64                 # ids as u16 (ids16) when every id of the vocabulary is < 65536
 OUT_OFFSETS_PACKED = 32          # one u16 per token (start | end << 8); falls back to OUT_OFFSETS when a pre-token has >= 256 bytes
+OUT_WORD_IDS = 256               # word ids: each token's pre-token index in its document, WORD_NONE for specials and padding
+WORD_NONE = 0xFFFFFFFF
 NORM_CFG_LOWER, NORM_BERT_STRUCT, NORM_LOWER_STRUCT = 1, 2, 3
 PT_WS_CFG, PT_BERT_CFG, PT_WS_STRUCT, PT_BERT_STRUCT, PT_BYTELEVEL_STRUCT = 1, 2, 3, 4, 5
 MODEL_BPE, MODEL_WORDPIECE = 0, 1
@@ -112,6 +114,7 @@ class BatchResult(C.Structure):
         ("span_tokens", C.c_void_p),
         ("n_wide", C.c_uint64),
         ("wide_tokens", C.c_void_p),
+        ("word_ids", C.c_void_p),
     ]
 
 
@@ -279,6 +282,7 @@ class BatchEncoding:
     offsets_packed: Optional[np.ndarray] = None     # u16 per token: start | end << 8 (OUT_OFFSETS_PACKED); 0xFFFF = see wide_tokens
     wide_tokens: Optional[np.ndarray] = None        # (n_wide, 4) u32: slot low, slot high, start, end -- tokens of pre-tokens of 256+ bytes
     span_tokens: Optional[np.ndarray] = None        # (n, 4) u32: id, start, end, type_id | flags << 8 (OUT_SPAN_TOKENS)
+    word_ids: Optional[np.ndarray] = None           # u32 per slot: pre-token index in the document, WORD_NONE for specials / padding (OUT_WORD_IDS)
 
     def __len__(self):
         return len(self.doc_tok_off) - 1
@@ -313,6 +317,7 @@ def _result_to_batch(r: BatchResult) -> BatchEncoding:
         offsets_packed=_copy(r.offsets_packed, T, np.uint16) if r.offsets_packed else None,
         wide_tokens=_copy(r.wide_tokens, 4 * int(r.n_wide), np.uint32).reshape(-1, 4) if (r.wide_tokens and r.n_wide) else None,
         span_tokens=_copy(r.span_tokens, 4 * T, np.uint32).reshape(-1, 4) if r.span_tokens else None,
+        word_ids=_copy(r.word_ids, T, np.uint32) if r.word_ids else None,
     )
 
 

@@ -61,7 +61,7 @@ struct tkz_ctx {
     DevBuf a_text, a_doc_off, a_norm_text, a_norm_doc_off, a_chunk, a_tiles, a_word_start, a_word_end, a_word_doc, a_doc_word_off,
         a_word_ntok, a_pool_id, a_pool_s, a_pool_e, a_pool_rk, a_scan_tmp, a_ctrl;
     // output arrays, double-buffered so that the D2H copy of one chunk overlaps the kernels of the next (tkz_encode_batch)
-    struct OutSet { DevBuf doc_tok_off, ids, off, attn, type, special, off16, ids16, spans, wide; } outs[2];
+    struct OutSet { DevBuf doc_tok_off, ids, off, attn, type, special, off16, ids16, spans, wide, wid; } outs[2];
     int out_sel = 0;
     OutSet& O() { return outs[out_sel]; }
     DevBuf in_text[2], in_doc_off[2];
@@ -71,7 +71,8 @@ struct tkz_ctx {
     uint64_t chunk_bytes = 64ull << 20;
     // slice pipeline arenas (tkz_slices.cuh)
     DevBuf a_long_start, a_long_end, a_long_ntok, a_long_slice, a_long_ins, a_tile_ntok, a_tile_ntok_inline, a_tile_tok_off, a_tile_long,
-        a_doc_tok_local, a_doc_tok_start, a_doc_real, a_upool, a_tile_doc_lo, a_g_first, a_g_win, a_g_flag, a_big;
+        a_doc_tok_local, a_doc_tok_start, a_doc_real, a_upool, a_tile_doc_lo, a_g_first, a_g_win, a_g_flag, a_big,
+        a_slice_nword, a_doc_word_local, a_doc_word_base, a_long_k;        // word ids (TKZ_OUT_WORD_IDS)
     bool use_dedup = true;                // TKZ_NO_DEDUP=1: per-occurrence pipeline even with a pre-tokenizer (A/B switch of the parity tests)
     DevBuf a_wtable, a_lscratch, a_tok_id;
     bool has_iso = false;                 // the class table isolates some byte (punctuation split)
@@ -93,9 +94,10 @@ struct tkz_ctx {
     uint64_t tw_uniq_hist = 0;            // most unique words seen in one batch: sizes the next batch's word table
     uint64_t tw_upool_hist = 0;           // most token records used by one batch
     double tw_tok_per_byte = 0.0;         // densest batch so far: sizes the token stream
-    HostBuf h_ctrl, h_doc_tok_off, h_ids, h_off, h_attn, h_type, h_special, h_off16, h_ids16, h_spans, h_wide;
+    HostBuf h_ctrl, h_doc_tok_off, h_ids, h_off, h_attn, h_type, h_special, h_off16, h_ids16, h_spans, h_wide, h_wid;
     DevBuf a_fast_heap, a_word_aux;       // FastTokenizer mode (tkz_fast.cuh)
     bool ids16_ok = false;                // every id the model can emit is below 65536 (TKZ_OUT_IDS_U16)
+    uint32_t max_id = 0;                  // largest id the model can emit (word ids need it below 2^22: TW_REC_WORD)
     // decode direction (tkz_decode.cuh)
     bool has_decode = false;
     DecodeTables dt{};
@@ -232,6 +234,7 @@ void slice_words_smem() {
     slice_words_smem_rec<MODEL, TW_REC_WIDE>();
     slice_words_smem_rec<MODEL, TW_REC_ID16>();
     slice_words_smem_rec<MODEL, TW_REC4>();
+    slice_words_smem_rec<MODEL, TW_REC_WORD>();
 }
 
 }  // namespace
@@ -314,13 +317,14 @@ extern "C" void tkz_ctx_destroy(tkz_ctx* ctx) {
                       &ctx->in_doc_off[1], &ctx->a_ctrl, &ctx->a_long_start, &ctx->a_long_end, &ctx->a_long_ntok, &ctx->a_long_slice, &ctx->a_long_ins,
                       &ctx->a_tile_ntok, &ctx->a_tile_ntok_inline, &ctx->a_tile_tok_off, &ctx->a_tile_long, &ctx->a_doc_tok_local,
                       &ctx->a_doc_tok_start, &ctx->a_doc_real, &ctx->a_upool, &ctx->a_tile_doc_lo, &ctx->a_g_first, &ctx->a_g_win, &ctx->a_g_flag, &ctx->a_big,
+                      &ctx->a_slice_nword, &ctx->a_doc_word_local, &ctx->a_doc_word_base, &ctx->a_long_k,
                       &ctx->a_wtable, &ctx->a_lscratch, &ctx->a_tok_id, &ctx->a_fast_heap, &ctx->a_word_aux,
                       &ctx->a_huge_w, &ctx->a_huge_base, &ctx->a_huge_done, &ctx->a_grid_state, &ctx->a_grid_words,
                       &ctx->t_dec_bytes, &ctx->t_dec_off, &ctx->t_dec_special, &ctx->a_dec_ids, &ctx->a_dec_seq_off, &ctx->a_dec_len, &ctx->a_dec_raw,
                       &ctx->a_dec_out, &ctx->a_dec_olen, &ctx->a_dec_boff};
-    for (auto& os : ctx->outs) for (DevBuf* b : {&os.doc_tok_off, &os.ids, &os.off, &os.attn, &os.type, &os.special, &os.off16, &os.ids16, &os.spans, &os.wide}) release(*b);
+    for (auto& os : ctx->outs) for (DevBuf* b : {&os.doc_tok_off, &os.ids, &os.off, &os.attn, &os.type, &os.special, &os.off16, &os.ids16, &os.spans, &os.wide, &os.wid}) release(*b);
     for (DevBuf* b : bufs) release(*b);
-    HostBuf* hb[] = {&ctx->h_ctrl, &ctx->h_doc_tok_off, &ctx->h_ids, &ctx->h_off, &ctx->h_attn, &ctx->h_type, &ctx->h_special, &ctx->h_off16, &ctx->h_ids16, &ctx->h_spans, &ctx->h_wide,
+    HostBuf* hb[] = {&ctx->h_ctrl, &ctx->h_doc_tok_off, &ctx->h_ids, &ctx->h_off, &ctx->h_attn, &ctx->h_type, &ctx->h_special, &ctx->h_off16, &ctx->h_ids16, &ctx->h_spans, &ctx->h_wide, &ctx->h_wid,
                      &ctx->h_doc_stage[0], &ctx->h_doc_stage[1], &ctx->h_dec_bytes, &ctx->h_dec_off};
     for (HostBuf* b : hb) release_host(*b);
     if (ctx->s_h2d) cudaStreamDestroy(ctx->s_h2d);
@@ -555,6 +559,7 @@ extern "C" int tkz_model_upload(tkz_ctx* ctx, const tkz_model_desc* d) {
         for (uint32_t i = 0; i < d->vocab_n; i++) max_id = std::max(max_id, d->vocab_ids[i]);
         if (d->model_kind == TKZ_MODEL_BPE) for (uint32_t i = 0; i < d->merges_n; i++) max_id = std::max(max_id, d->merge_new[i]);
         ctx->ids16_ok = max_id < 65536u;
+        ctx->max_id = max_id;
     }
     CK(cudaStreamSynchronize(ctx->stream));      // host staging vectors die at return
     ctx->dm = m;
@@ -710,9 +715,11 @@ int alloc_outputs(tkz_ctx* ctx, const EmitParams& ep, uint64_t T, uint32_t wide_
     if (o & TKZ_OUT_SPECIAL) TRY(ensure(ctx, O.special, (T + 4) * 4));
     if (o & TKZ_OUT_OFFSETS_PACKED) TRY(ensure(ctx, O.off16, (T + 4) * 2));
     if (o & TKZ_OUT_SPAN_TOKENS) TRY(ensure(ctx, O.spans, (T + 4) * 16));
+    if (o & TKZ_OUT_WORD_IDS) TRY(ensure(ctx, O.wid, (T + 4) * 4));
     if (wide_cap) TRY(ensure(ctx, O.wide, (size_t)wide_cap * 16));
     eo = EmitOut{(uint32_t*)O.ids.p, (uint32_t*)O.off.p, (uint32_t*)O.attn.p, (uint32_t*)O.type.p, (uint32_t*)O.special.p, (uint16_t*)O.off16.p,
-                 (uint16_t*)O.ids16.p, (uint4*)O.spans.p, (uint4*)O.wide.p, (unsigned int*)((unsigned long long*)ctx->a_ctrl.p + 23), wide_cap};
+                 (uint16_t*)O.ids16.p, (uint4*)O.spans.p, (uint4*)O.wide.p, (unsigned int*)((unsigned long long*)ctx->a_ctrl.p + 23), wide_cap,
+                 (uint32_t*)O.wid.p};
     return TKZ_OK;
 }
 
@@ -732,6 +739,7 @@ bool pad_prologue(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, uint32_
     if (o & TKZ_OUT_SPECIAL) fill(eo.special, T * 4, rep(1u));
     if (o & TKZ_OUT_OFFSETS_PACKED) fill(eo.offsets16, T * 2, rep(0u));
     if (o & TKZ_OUT_SPAN_TOKENS) fill(eo.spans, T * 16, make_uint4(ep.pad_id, 0u, 0u, 0x0400u));
+    if (o & TKZ_OUT_WORD_IDS) fill(eo.word_ids, T * 4, rep(TKZ_NONE));
     return true;
 }
 
@@ -740,23 +748,30 @@ bool pad_prologue(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, uint32_
 void pad_epilogue(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, uint32_t nd, const uint32_t* doc_real, const unsigned long long* doc_tok_off,
                   bool filled, uint64_t& launches) {
     if (!nd) return;
+    const bool wid = (ep.outputs & TKZ_OUT_WORD_IDS) != 0;
     if (ep.has_pad && !filled) {
-        emit_pad_real_kernel<<<(unsigned)(((uint64_t)nd * 32 + 255) / 256), 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off); launches++;
+        const unsigned g = (unsigned)(((uint64_t)nd * 32 + 255) / 256);
+        if (wid) emit_pad_real_kernel<true><<<g, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off);
+        else emit_pad_real_kernel<false><<<g, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off);
+        launches++;
     } else if (has_frame(ep)) {
-        emit_frame_kernel<<<(nd + 255) / 256, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off); launches++;
+        if (wid) emit_frame_kernel<true><<<(nd + 255) / 256, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off);
+        else emit_frame_kernel<false><<<(nd + 255) / 256, 256, 0, ctx->stream>>>(ep, eo, nd, doc_real, doc_tok_off);
+        launches++;
     }
 }
 
-// the eight per-token arrays of a result in TKZ_OUT_* bit order (ids, offsets, attention, type ids, special, packed offsets,
-// ids16, span tokens), nullptr where not delivered
-using ResultArrays = std::array<const void*, 8>;
+// the nine per-token arrays of a result in TKZ_OUT_* bit order (ids, offsets, attention, type ids, special, packed offsets,
+// ids16, span tokens, word ids), nullptr where not delivered
+constexpr uint32_t N_RESULT_ARRAYS = 9;
+using ResultArrays = std::array<const void*, N_RESULT_ARRAYS>;
 void set_result(tkz_batch_result* out, uint64_t n_docs, uint64_t T, uint64_t T_real, const uint64_t* doc_tok_off, const ResultArrays& a,
                 uint64_t n_wide, const void* wide) {
     out->n_docs = n_docs; out->n_tokens = T; out->n_real_tokens = T_real;
     out->doc_tok_off = doc_tok_off;
     out->ids = (const uint32_t*)a[0]; out->offsets = (const uint32_t*)a[1]; out->attention_mask = (const uint32_t*)a[2];
     out->type_ids = (const uint32_t*)a[3]; out->special_tokens_mask = (const uint32_t*)a[4]; out->offsets_packed = (const uint16_t*)a[5];
-    out->ids16 = (const uint16_t*)a[6]; out->span_tokens = (const uint32_t*)a[7];
+    out->ids16 = (const uint16_t*)a[6]; out->span_tokens = (const uint32_t*)a[7]; out->word_ids = (const uint32_t*)a[8];
     out->n_wide = n_wide; out->wide_tokens = n_wide ? (const uint32_t*)wide : nullptr;
 }
 
@@ -770,8 +785,8 @@ void finish(tkz_ctx* ctx, const EmitParams& ep, const EmitOut& eo, const unsigne
     cudaEventElapsedTime(&ctx->stats.ms_emit, ctx->ev[3], ctx->ev[4]);
     cudaEventElapsedTime(&ctx->stats.ms_total, ctx->ev[0], ctx->ev[4]);
     const uint32_t o = ep.outputs;
-    ResultArrays a = {eo.ids, eo.offsets, eo.attention, eo.type_ids, eo.special, eo.offsets16, eo.ids16, eo.spans};
-    for (uint32_t i = 0; i < 8; i++) if (!(o & (1u << i))) a[i] = nullptr;
+    ResultArrays a = {eo.ids, eo.offsets, eo.attention, eo.type_ids, eo.special, eo.offsets16, eo.ids16, eo.spans, eo.word_ids};
+    for (uint32_t i = 0; i < N_RESULT_ARRAYS; i++) if (!(o & (1u << i))) a[i] = nullptr;
     if (o & TKZ_OUT_IDS_U16) a[0] = nullptr;                          // exactly one of ids / ids16
     set_result(out, n_docs, T, T_real, (const uint64_t*)doc_tok_off, a, n_wide, eo.wide);
 }
@@ -800,17 +815,20 @@ void launch_slice_words_rec(const DevModel& m, const SliceArgs& ta, int cls, uin
 template <int MODEL>
 void launch_slice_words(const DevModel& m, const SliceArgs& ta, int cls, int rec, uint32_t blocks, cudaStream_t st) {
     if (rec == TW_REC_ID32) launch_slice_words_rec<MODEL, TW_REC_ID32>(m, ta, cls, blocks, st);
+    else if (rec == TW_REC_WORD) launch_slice_words_rec<MODEL, TW_REC_WORD>(m, ta, cls, blocks, st);
     else if (rec == TW_REC_WIDE) launch_slice_words_rec<MODEL, TW_REC_WIDE>(m, ta, cls, blocks, st);
     else if (rec == TW_REC_ID16) launch_slice_words_rec<MODEL, TW_REC_ID16>(m, ta, cls, blocks, st);
     else launch_slice_words_rec<MODEL, TW_REC4>(m, ta, cls, blocks, st);
 }
-// the output forms with offsets read TW_REC_WIDE or TW_REC4 records, the ids-only forms TW_REC_ID32 or TW_REC_ID16
+// the output forms with offsets read TW_REC_WIDE or TW_REC4 records, the ids-only forms TW_REC_ID32 or TW_REC_ID16; calls
+// with word ids TW_REC_WORD records, always per document (never PLAIN) and through the generic form
 template <bool PLAIN>
 void launch_slice_emit(const SliceEmitArgs& ea, const EmitParams& ep, const EmitOut& eo, int rec, uint32_t blocks, cudaStream_t st) {
     const uint32_t o = ep.outputs;
     const bool narrow = rec == TW_REC4 || rec == TW_REC_ID16;
 #define TKZ_SLICE_EMIT(OUTS, REC) slice_emit_kernel<PLAIN, OUTS, REC><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo)
-    if (o == TKZ_OUT_IDS) { if (narrow) TKZ_SLICE_EMIT(1u, TW_REC_ID16); else TKZ_SLICE_EMIT(1u, TW_REC_ID32); }
+    if (rec == TW_REC_WORD) { if (!PLAIN) slice_emit_kernel<false, 0u, TW_REC_WORD><<<blocks, TW_THREADS, 0, st>>>(ea, ep, eo); }
+    else if (o == TKZ_OUT_IDS) { if (narrow) TKZ_SLICE_EMIT(1u, TW_REC_ID16); else TKZ_SLICE_EMIT(1u, TW_REC_ID32); }
     else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS | TKZ_OUT_ATTENTION)) { if (narrow) TKZ_SLICE_EMIT(7u, TW_REC4); else TKZ_SLICE_EMIT(7u, TW_REC_WIDE); }
     else if (o == (TKZ_OUT_IDS | TKZ_OUT_OFFSETS_PACKED)) { if (narrow) TKZ_SLICE_EMIT(33u, TW_REC4); else TKZ_SLICE_EMIT(33u, TW_REC_WIDE); }
     else if (o == (TKZ_OUT_IDS | TKZ_OUT_IDS_U16 | TKZ_OUT_OFFSETS_PACKED)) { if (narrow) TKZ_SLICE_EMIT(97u, TW_REC4); else TKZ_SLICE_EMIT(97u, TW_REC_WIDE); }
@@ -829,7 +847,9 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     unsigned long long* hctrl = (unsigned long long*)ctx->h_ctrl.p;
     const uint64_t n_docs = nd;
     const uint32_t n_slices = (uint32_t)(N / TW_SLICE + 1);
-    const bool plain = !P.has_truncation && !P.has_padding && !P.hf_flags;        // (hf_compat: per-document destinations and offsets)
+    const bool want_wid = (P.outputs & TKZ_OUT_WORD_IDS) != 0;
+    // (hf_compat and word ids: per-document destinations and offsets / word bases)
+    const bool plain = !P.has_truncation && !P.has_padding && !P.hf_flags && !want_wid;
     // ---- capacities: from the text size and from what earlier batches of this context needed
     const bool keep = ctx->call_keep && ctx->kept_valid && !worst;           // reuse the table + pool of this call's previous chunk
     const uint64_t Nsz = ctx->call_keep ? std::max<uint64_t>(N, ctx->call_bytes) : N;
@@ -857,8 +877,9 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     // token stream records: 16-bit ids when every id of the model fits, with the two offset bytes beside them in 4 bytes --
     // unless the offsets are document-relative (hf_compat), which needs the word's position in the slice as well
     const bool narrow = ctx->narrow_records && ctx->ids16_ok && !(want_of && (P.hf_flags & TKZ_HF_DOC_OFFSETS));
-    const int rec = want_of ? (narrow ? TW_REC4 : TW_REC_WIDE) : (narrow ? TW_REC_ID16 : TW_REC_ID32);
-    const size_t rec_bytes = rec == TW_REC_WIDE ? 8 : (rec == TW_REC_ID16 ? 2 : 4);
+    // (word ids: the word's index in its slice beside the id, with or without offsets)
+    const int rec = want_wid ? TW_REC_WORD : want_of ? (narrow ? TW_REC4 : TW_REC_WIDE) : (narrow ? TW_REC_ID16 : TW_REC_ID32);
+    const size_t rec_bytes = (rec == TW_REC_WIDE || rec == TW_REC_WORD) ? 8 : (rec == TW_REC_ID16 ? 2 : 4);
     TRY(ensure(ctx, ctx->a_wtable, ((size_t)tcap + mcap) * sizeof(WordSlot) + (size_t)m32cap * sizeof(WordSlot32)));
     TRY(ensure(ctx, ctx->a_upool, (size_t)upool_cap * 8));
     TRY(ensure(ctx, ctx->a_lscratch, (size_t)warps * 4 * 256 * 4));
@@ -873,6 +894,12 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     TRY(ensure(ctx, ctx->a_long_end, (size_t)long_cap * 4));
     TRY(ensure(ctx, ctx->a_long_slice, (size_t)long_cap * 4));
     TRY(ensure(ctx, ctx->a_long_ins, (size_t)long_cap * 4));
+    if (want_wid) {
+        TRY(ensure(ctx, ctx->a_slice_nword, ((size_t)n_slices + 2) * 4));
+        TRY(ensure(ctx, ctx->a_doc_word_local, (n_docs + 2) * 4));
+        TRY(ensure(ctx, ctx->a_doc_word_base, (n_docs + 2) * 4));
+        TRY(ensure(ctx, ctx->a_long_k, (size_t)long_cap * 4));
+    }
     TRY(ensure(ctx, ctx->O().doc_tok_off, (n_docs + 1) * 8));
     TRY(ensure(ctx, ctx->a_scan_tmp, (scan_tmp_elems(n_slices) + scan_tmp_elems(n_docs)) * 8));
     if (!keep) CK(cudaMemsetAsync(ctx->a_wtable.p, 0, ((size_t)tcap + mcap) * sizeof(WordSlot) + (size_t)m32cap * sizeof(WordSlot32), st));
@@ -896,6 +923,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ta.cr = cr;
     ta.n_bulk = N >= (uint64_t)(TW_SLICE + TW_POST) ? (uint32_t)std::min<uint64_t>(n_slices, (N - (TW_SLICE + TW_POST)) / TW_SLICE + 1) : 0u;
     ta.has_iso = ctx->has_iso ? 1 : 0;
+    if (want_wid) { ta.slice_nword = (uint32_t*)ctx->a_slice_nword.p; ta.doc_word_local = (uint32_t*)ctx->a_doc_word_local.p; ta.long_k = (uint32_t*)ctx->a_long_k.p; }
     const int cls = (cr.usable && !ctx->force_lut) ? (cr.norm_lower ? 1 : 0) : (m.norm_identity ? 2 : 3);
     if (m.kind == TKZ_MODEL_BPE) launch_slice_words<TKZ_MODEL_BPE>(m, ta, cls, rec, grid, st);
     else launch_slice_words<TKZ_MODEL_WORDPIECE>(m, ta, cls, rec, grid, st);
@@ -942,12 +970,15 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     // ---- tokens per tile -> token base per tile; CSR offsets
     EmitParams ep = emit_params(P);
     launches += exclusive_scan<uint32_t>(ta.slice_ntok, n_slices, ta.slice_ntok, (unsigned long long*)ctx->a_scan_tmp.p, st);
+    // word ids: words per slice -> global index of each slice's first word (in place)
+    if (want_wid) launches += exclusive_scan<uint32_t>(ta.slice_nword, n_slices, ta.slice_nword, (unsigned long long*)ctx->a_scan_tmp.p, st);
     unsigned long long* doc_tok_off = (unsigned long long*)ctx->O().doc_tok_off.p;
     if (!plain) {
         TRY(ensure(ctx, ctx->a_doc_tok_start, (n_docs + 2) * 4));
         TRY(ensure(ctx, ctx->a_doc_real, (n_docs + 2) * 4));
         doc_finish2_kernel<<<(nd + 1 + 255) / 256, 256, 0, st>>>(d_doc_off, nd, ta.slice_ntok, ta.doc_tok_local, ep, (uint32_t*)ctx->a_doc_tok_start.p,
-                                                                  (uint32_t*)ctx->a_doc_real.p, doc_tok_off); launches++;
+                                                                  (uint32_t*)ctx->a_doc_real.p, doc_tok_off, ta.slice_nword, ta.doc_word_local,
+                                                                  want_wid ? (uint32_t*)ctx->a_doc_word_base.p : nullptr); launches++;
         launches += exclusive_scan<unsigned long long>(doc_tok_off, n_docs, doc_tok_off, (unsigned long long*)ctx->a_scan_tmp.p, st);
         TRY(readback(ctx, hctrl + 3, doc_tok_off + n_docs, 8));
     }
@@ -977,7 +1008,7 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     EmitOut eo;
     TRY(alloc_outputs(ctx, ep, T, wide_cap, eo));
     const uint32_t big_cap = (uint32_t)(N / EMIT_BIG + 16);
-    TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
+    TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + 2 * sizeof(uint32_t))));
     SliceEmitArgs ea{};
     ea.doc_off = d_doc_off; ea.n_docs = nd; ea.n_slices = n_slices; ea.slice_doc_lo = ta.slice_doc_lo;
     ea.tok = ta.tok;
@@ -986,13 +1017,19 @@ int encode_slices(tkz_ctx* ctx, const DevModel& m, const ClassRanges& cr, const 
     ea.pool_id = (const uint32_t*)ctx->a_pool_id.p; ea.pool_s = (const uint32_t*)ctx->a_pool_s.p; ea.pool_e = (const uint32_t*)ctx->a_pool_e.p;
     ea.doc_tok_local = ta.doc_tok_local; ea.doc_tok_start = (const uint32_t*)ctx->a_doc_tok_start.p;
     ea.doc_tok_off = doc_tok_off; ea.errw = ctrl; ea.err_code = m.kind == TKZ_MODEL_BPE ? TKZ_ECODE_UTF8 : TKZ_ECODE_UNK;
-    ea.big = BigList{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 16), big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
+    ea.big = BigList{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 16), big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap),
+                     (uint32_t*)((uint4*)ctx->a_big.p + big_cap) + big_cap};
+    if (want_wid) { ea.slice_wordbase = ta.slice_nword; ea.doc_word_base = (const uint32_t*)ctx->a_doc_word_base.p; ea.long_k = ta.long_k; }
     const bool filled = pad_prologue(ctx, ep, eo, nd, T, T_real, launches);
     const uint32_t egrid = (uint32_t)std::min<uint64_t>(((uint64_t)n_slices + TW_WARPS - 1) / TW_WARPS, (uint64_t)ctx->sm_count * 16);
     if (plain) launch_slice_emit<true>(ea, ep, eo, rec, egrid, st);
     else launch_slice_emit<false>(ea, ep, eo, rec, egrid, st);
     launches++;
-    if (n_long) { emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, ea.big, ea.pool_id, ea.pool_s, ea.pool_e); launches++; }
+    if (n_long) {
+        if (want_wid) emit_big_kernel<true><<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, ea.big, ea.pool_id, ea.pool_s, ea.pool_e);
+        else emit_big_kernel<false><<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, ea.big, ea.pool_id, ea.pool_s, ea.pool_e);
+        launches++;
+    }
     pad_epilogue(ctx, ep, eo, nd, (const uint32_t*)ctx->a_doc_real.p, doc_tok_off, filled, launches);
     CK(cudaGetLastError());
     CK(cudaEventRecord(ctx->ev[4], st));
@@ -1115,13 +1152,18 @@ int encode_words(tkz_ctx* ctx, const DevModel& m, const uint8_t* d_text, const u
     const bool filled = pad_prologue(ctx, ep, eo, nd, T, T_real, launches);
     if (nw) {
         const uint32_t big_cap = (uint32_t)(N / EMIT_BIG + 16);
-        TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + sizeof(uint32_t))));
-        BigList bl{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 9) + 1, big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap)};
-        emit_words_kernel<<<(nw + 255) / 256, 256, 0, st>>>(ep, eo, nw, word_start, word_doc, word_tok_off, doc_word_off, doc_tok_off,
-                                                            (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
-                                                            (const uint32_t*)ctx->a_pool_e.p, bl, d_doc_off); launches++;
-        emit_big_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, bl, (const uint32_t*)ctx->a_pool_id.p, (const uint32_t*)ctx->a_pool_s.p,
-                                                           (const uint32_t*)ctx->a_pool_e.p); launches++;
+        TRY(ensure(ctx, ctx->a_big, (size_t)big_cap * (sizeof(uint4) + 2 * sizeof(uint32_t))));
+        BigList bl{(uint4*)ctx->a_big.p, (unsigned int*)(ctrl + 9) + 1, big_cap, (uint32_t*)((uint4*)ctx->a_big.p + big_cap),
+                   (uint32_t*)((uint4*)ctx->a_big.p + big_cap) + big_cap};
+        const uint32_t *pid = (const uint32_t*)ctx->a_pool_id.p, *ps = (const uint32_t*)ctx->a_pool_s.p, *pe = (const uint32_t*)ctx->a_pool_e.p;
+        if (ep.outputs & TKZ_OUT_WORD_IDS) {
+            emit_words_kernel<true><<<(nw + 255) / 256, 256, 0, st>>>(ep, eo, nw, word_start, word_doc, word_tok_off, doc_word_off, doc_tok_off, pid, ps, pe, bl, d_doc_off);
+            emit_big_kernel<true><<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, bl, pid, ps, pe);
+        } else {
+            emit_words_kernel<false><<<(nw + 255) / 256, 256, 0, st>>>(ep, eo, nw, word_start, word_doc, word_tok_off, doc_word_off, doc_tok_off, pid, ps, pe, bl, d_doc_off);
+            emit_big_kernel<false><<<ctx->sm_count * 4, 256, 0, st>>>(ep, eo, bl, pid, ps, pe);
+        }
+        launches += 2;
     }
     pad_epilogue(ctx, ep, eo, nd, doc_real, doc_tok_off, filled, launches);
     CK(cudaGetLastError());
@@ -1164,6 +1206,11 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
                 if ((i < P.tpl_n_prefix && P.tpl_prefix_id[i] > 0xFFFFu) || (i < P.tpl_n_suffix && P.tpl_suffix_id[i] > 0xFFFFu)) { ctx->err = "template id above 65535 with TKZ_OUT_IDS_U16"; return TKZ_ERR_INVALID_ARG; }
         // document-relative offsets do not fit the one-u16-per-token form
         if ((P.hf_flags & TKZ_HF_DOC_OFFSETS) && (P.outputs & TKZ_OUT_OFFSETS_PACKED)) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
+    }
+    if (P.outputs & TKZ_OUT_WORD_IDS) {
+        if (P.fast) { ctx->err = "word ids cannot be combined with the FastTokenizer mode"; return TKZ_ERR_INVALID_ARG; }
+        // (the slice pipeline's token records keep the word's index in the slice above a 22-bit id)
+        if (ctx->max_id >= (1u << 22)) { ctx->err = "word ids need every id of the model below 2^22"; return TKZ_ERR_INVALID_ARG; }
     }
     if ((P.outputs & TKZ_OUT_IDS_U16) && (!ctx->ids16_ok || (P.has_padding && P.pad_id > 0xFFFFu))) P.outputs &= ~TKZ_OUT_IDS_U16;
     const uint32_t nd = (uint32_t)n_docs;
@@ -1248,10 +1295,11 @@ void wide_finish(WideRec* w, uint64_t n_total, const std::vector<std::array<uint
 
 // the per-token arrays of a device result (ResultArrays order), the pinned host arrays they are copied to, bytes per slot
 struct ResultCopy { const void* dev; HostBuf* host; size_t elem; };
-std::array<ResultCopy, 8> result_copies(tkz_ctx* ctx, const tkz_batch_result& r) {
+// (word ids are relative to their document: chunks of the host path copy them as they are)
+std::array<ResultCopy, N_RESULT_ARRAYS> result_copies(tkz_ctx* ctx, const tkz_batch_result& r) {
     return {{{r.ids, &ctx->h_ids, 4}, {r.offsets, &ctx->h_off, 8}, {r.attention_mask, &ctx->h_attn, 4}, {r.type_ids, &ctx->h_type, 4},
              {r.special_tokens_mask, &ctx->h_special, 4}, {r.offsets_packed, &ctx->h_off16, 2}, {r.ids16, &ctx->h_ids16, 2},
-             {r.span_tokens, &ctx->h_spans, 16}}};
+             {r.span_tokens, &ctx->h_spans, 16}, {r.word_ids, &ctx->h_wid, 4}}};
 }
 
 // one shot: H2D everything, encode, D2H everything (small batches)
@@ -1273,7 +1321,7 @@ int encode_host_single(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_of
     CK(cudaMemcpyAsync(ctx->h_doc_tok_off.p, dev.doc_tok_off, (n_docs + 1) * 8, cudaMemcpyDeviceToHost, st));
     const auto cp = result_copies(ctx, dev);
     ResultArrays host{};
-    for (uint32_t i = 0; i < 8; i++) {
+    for (uint32_t i = 0; i < N_RESULT_ARRAYS; i++) {
         if (!cp[i].dev) continue;
         TRY(ensure_host(ctx, *cp[i].host, T * cp[i].elem));
         if (T) CK(cudaMemcpyAsync(cp[i].host->p, cp[i].dev, T * cp[i].elem, cudaMemcpyDeviceToHost, st));
@@ -1384,7 +1432,7 @@ restart:
         if (est < T_total + T) est = T_total + T;
         // (every chunk delivers the same arrays: they depend on the model and the parameters)
         const auto cp = result_copies(ctx, dev);
-        for (uint32_t k = 0; k < 8; k++) {
+        for (uint32_t k = 0; k < N_RESULT_ARRAYS; k++) {
             host[k] = nullptr;
             if (!cp[k].dev) continue;
             TRY(ensure_host_keep(ctx, *cp[k].host, est * cp[k].elem, T_total * cp[k].elem));
@@ -1436,6 +1484,7 @@ extern "C" int tkz_encode_batch_compact(tkz_ctx* ctx, const uint8_t* text, const
     if (params) P = *params;
     out->params = P;
     if (P.hf_flags) { ctx->err = "the compact result does not carry hf_compat (template / document offsets): use tkz_encode_batch"; return TKZ_ERR_INVALID_ARG; }
+    if (P.outputs & TKZ_OUT_WORD_IDS) { ctx->err = "the compact result does not carry word ids: use tkz_encode_batch"; return TKZ_ERR_INVALID_ARG; }
     // on the device: truncation only; no padding slot and no constant array is materialised or copied
     tkz_encode_params Q = P;
     Q.has_padding = 0;

@@ -65,6 +65,8 @@ constexpr int TW_REC_ID32 = 0;                    // u32 id (ids only)
 constexpr int TW_REC_WIDE = 1;                    // {u32 id, start | end << 8 | the word's position in the slice << 16}
 constexpr int TW_REC_ID16 = 2;                    // u16 id (ids only, 16-bit vocabulary)
 constexpr int TW_REC4 = 3;                        // u32: id | start << 16 | end << 24 (16-bit vocabulary, pre-token offsets)
+constexpr int TW_REC_WORD = 4;                    // {u32 id | k << 22, as TW_REC_WIDE}: k = the word's index in the slice's word list
+                                                  // (< 1024), for word ids (TKZ_OUT_WORD_IDS; ids below 2^22)
 
 // 32-byte slot = one L2 sector.  Short words (<= 15 bytes): k0..k3 = the normalised bytes, length in the top byte of k3
 // (so a used key is never all zero).  Medium words live in their own slot range: k0,k1 = 64-bit tag (top bit set),
@@ -115,6 +117,9 @@ struct SliceArgs {
     unsigned long long* n_words; unsigned int* n_uniq; unsigned int* n_uncached;
     ClassRanges cr;
     int has_iso;                                  // some byte is its own pre-token (punctuation split)
+    // TW_REC_WORD only: words that start in each slice, index of each document's first word in its slice's word list, the
+    // long words' indices in their slice's word list
+    uint32_t* slice_nword; uint32_t* doc_word_local; uint32_t* long_k;
 };
 
 // first document that starts at or after each tile (slice) start; entry n_tiles = n_docs + 1.  One thread per tile.
@@ -589,10 +594,12 @@ __device__ __forceinline__ WholeWarpOut tw_own_word(const DevModel& m, const Sli
     return out;
 }
 
-// one token into the stream at index i: of = start | end << 8, ph = the word's position in the slice << 16
+// one token into the stream at index i: of = start | end << 8, ph = the word's position in the slice << 16, k = the word's
+// index in the slice's word list (TW_REC_WORD)
 template <int REC>
-__device__ __forceinline__ void tw_put_token(void* tok, uint32_t i, uint32_t id, uint32_t of, uint32_t ph) {
+__device__ __forceinline__ void tw_put_token(void* tok, uint32_t i, uint32_t id, uint32_t of, uint32_t ph, uint32_t k = 0) {
     if (REC == TW_REC_WIDE) static_cast<uint2*>(tok)[i] = make_uint2(id, of | ph);
+    else if (REC == TW_REC_WORD) static_cast<uint2*>(tok)[i] = make_uint2(id | (k << 22), of | ph);
     else if (REC == TW_REC4) static_cast<uint32_t*>(tok)[i] = id | (of << 16);
     else if (REC == TW_REC_ID16) static_cast<uint16_t*>(tok)[i] = (uint16_t)id;
     else static_cast<uint32_t*>(tok)[i] = id;
@@ -610,7 +617,8 @@ __device__ __forceinline__ void tw_flush_pooled(const SliceArgs& a, const uint4*
         for (uint32_t i = lane & 3u; i < q.y; i += 4) {
             const unsigned long long r = __ldcg(a.upool + q.x + i);       // written in THIS launch by the word's owner: L2, not the read-only path
             const uint32_t of = ((uint32_t)(r >> 32) & 0xFFu) | (((uint32_t)(r >> 48) & 0xFFu) << 8);
-            tw_put_token<REC>(a.tok, q.z + i, (uint32_t)r, of, q.w);
+            if (REC == TW_REC_WORD) tw_put_token<REC>(a.tok, q.z + i, (uint32_t)r, of, q.w & 0xFFFF0000u, q.w & 0xFFFFu);   // (q.w = p << 16 | k)
+            else tw_put_token<REC>(a.tok, q.z + i, (uint32_t)r, of, q.w);
         }
     }
     __syncwarp();
@@ -916,17 +924,17 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             else { const uint32_t inc = warp_incl_scan(nt); ex = inc - nt; tot = __shfl_sync(FULL, inc, 31); }
             const uint32_t dst = tbase + run + ex;                  // stream position of the word's first token
             if (can_store && nt && !(flags & TW_POOLF)) {
-                // (the word's position in the slice goes into TW_REC_WIDE records only: it is read by the hf_compat mode of pass B
-                // that reports offsets relative to the document)
-                tw_put_token<REC>(a.tok, dst, v.a, v.b & 0xFFFFu, p << 16);
-                if (nt == 2) tw_put_token<REC>(a.tok, dst + 1, v.c, v.d & 0xFFFFu, p << 16);
+                // (the word's position in the slice goes into TW_REC_WIDE / TW_REC_WORD records only: it is read by the hf_compat
+                // mode of pass B that reports offsets relative to the document; k, the word's index, into TW_REC_WORD records)
+                tw_put_token<REC>(a.tok, dst, v.a, v.b & 0xFFFFu, p << 16, k);
+                if (nt == 2) tw_put_token<REC>(a.tok, dst + 1, v.c, v.d & 0xFFFFu, p << 16, k);
             }
             // words with three or more tokens: listed now, copied from the pool at the end of the slice
             const uint32_t pooled = __ballot_sync(FULL, can_store && nt && (flags & TW_POOLF));
             if (pooled) {
                 const uint32_t np = __popc(pooled);
                 if (n_pl + np > 32) { tw_flush_pooled<REC>(a, sh.plist, n_pl); n_pl = 0; }
-                if ((pooled >> lane) & 1u) sh.plist[n_pl + __popc(pooled & lt_mask)] = make_uint4(v.a, nt, dst, p << 16);
+                if ((pooled >> lane) & 1u) sh.plist[n_pl + __popc(pooled & lt_mask)] = make_uint4(v.a, nt, dst, (p << 16) | (REC == TW_REC_WORD ? k : 0u));
                 n_pl += np;
             }
             if (__any_sync(FULL, flags & (TW_ERRF | TW_LONGF))) {
@@ -935,7 +943,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
                 const uint32_t lm = __ballot_sync(FULL, (flags & TW_LONGF) != 0);
                 if (flags & TW_LONGF) {
                     const uint32_t j = n_long_here + __popc(lm & lt_mask);
-                    if (j < TW_MAX_SLICE_LONG) { sh.lbuf[j][0] = p; sh.lbuf[j][1] = v.a; sh.lbuf[j][2] = run + ex; }
+                    if (j < TW_MAX_SLICE_LONG) { sh.lbuf[j][0] = p | (REC == TW_REC_WORD ? k << 16 : 0u); sh.lbuf[j][1] = v.a; sh.lbuf[j][2] = run + ex; }
                 }
                 n_long_here += __popc(lm);
             }
@@ -953,9 +961,10 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             __syncwarp();
             if (lfirst + n_long_here > a.long_cap) { warp_abort = true; n_long_here = 0; }
             else if (lane < n_long_here) {
-                const uint32_t st = (uint32_t)(slice_base + sh.lbuf[lane][0]);
+                const uint32_t st = (uint32_t)(slice_base + (REC == TW_REC_WORD ? sh.lbuf[lane][0] & 0xFFFFu : sh.lbuf[lane][0]));
                 a.long_start[lfirst + lane] = st; a.long_end[lfirst + lane] = st + sh.lbuf[lane][1];
                 a.long_slice[lfirst + lane] = s; a.long_ins[lfirst + lane] = sh.lbuf[lane][2];
+                if (REC == TW_REC_WORD) a.long_k[lfirst + lane] = sh.lbuf[lane][0] >> 16;
             }
         }
         if (lane == 0) {
@@ -963,6 +972,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
             a.slice_ntok_inline[s] = can_store ? run : 0u;
             a.slice_ntok[s] = run;
             a.slice_long[s] = (lfirst << 3) | n_long_here;
+            if (REC == TW_REC_WORD) a.slice_nword[s] = nW;
         }
         __syncwarp();
         // ---- token prefix at every document start inside the slice
@@ -973,6 +983,7 @@ __global__ void __launch_bounds__(TW_THREADS, TW_BLOCKS_PER_SM) slice_words_kern
                 const uint32_t sg = q >> 5;
                 const uint32_t idx = sh.seg_wex[sg] + __popc(sh.seg_smask[sg] & ((1u << (q & 31u)) - 1u));
                 a.doc_tok_local[d] = idx < nW ? (uint32_t)sh.wlist[idx] : run;
+                if (REC == TW_REC_WORD) a.doc_word_local[d] = idx;
             }
         }
         __syncwarp();
@@ -1010,13 +1021,18 @@ struct SliceEmitArgs {
     unsigned long long* doc_tok_off;              // PLAIN: written here; !PLAIN: read (CSR after truncate / pad)
     unsigned long long* errw; uint32_t err_code;
     BigList big;
+    // TW_REC_WORD: exclusive scan of the words that start in each slice, global index of each document's first word, the long
+    // words' indices in their slice's word list
+    const uint32_t* slice_wordbase; const uint32_t* doc_word_base; const uint32_t* long_k;
 };
 
 // one token of the stream -> the arrays the call asked for.  OUTS = the TKZ_OUT_* mask when known at compile time
-// (ids only / ids + offsets + attention), 0 = read it from the parameters.
-template <uint32_t OUTS>
-__device__ __forceinline__ void te_put(const EmitParams& p, const EmitOut& o, unsigned long long dst, uint32_t id, uint32_t of, uint32_t hs) {
+// (ids only / ids + offsets + attention), 0 = read it from the parameters.  WID (TW_REC_WORD records): id carries the word's
+// index in its slice's word list in bits 22.., wb = the slice's first word relative to the document's
+template <uint32_t OUTS, bool WID = false>
+__device__ __forceinline__ void te_put(const EmitParams& p, const EmitOut& o, unsigned long long dst, uint32_t id, uint32_t of, uint32_t hs, uint32_t wb = 0) {
     const uint32_t outputs = OUTS ? OUTS : p.outputs;
+    if (WID) { o.word_ids[dst] = wb + (id >> 22); id &= 0x3FFFFFu; }
     uint32_t s = of & 0xFFu, e = (of >> 8) & 0xFFu, ty = 0u;
     if (p.hf_flags) {                                            // hf_compat (tkz_emit.cuh): document-relative offsets, the sequence's type id
         if (p.hf_flags & 2u) { const uint32_t b = hs + (of >> 16); s += b; e += b; }
@@ -1043,7 +1059,7 @@ __shared__ __align__(128) unsigned char te_smem[TW_WARPS][2 * TE_WIN + 16];   //
 
 template <int REC>
 struct TeWindows {
-    static constexpr uint32_t RB = REC == TW_REC_WIDE ? 8 : (REC == TW_REC_ID16 ? 2 : 4);   // bytes per record
+    static constexpr uint32_t RB = (REC == TW_REC_WIDE || REC == TW_REC_WORD) ? 8 : (REC == TW_REC_ID16 ? 2 : 4);   // bytes per record
     static constexpr uint32_t RPG = 16 / RB, RPW = TE_WIN / RB;                             // records per 16 bytes, per window
     uint32_t cur, clo, chi;              // the window being read and the records [clo, chi) it holds
     uint32_t nlo, nhi, npend;            // the other window: its records, whether its copy is in flight
@@ -1091,7 +1107,7 @@ struct TeWindows {
 // record q of a window -> (id, start | end << 8 [| position << 16]), the form te_put takes
 template <int REC>
 __device__ __forceinline__ void te_rec(const unsigned char* w, uint32_t q, uint32_t& id, uint32_t& of) {
-    if (REC == TW_REC_WIDE) { const uint2 r = reinterpret_cast<const uint2*>(w)[q]; id = r.x; of = r.y; }
+    if (REC == TW_REC_WIDE || REC == TW_REC_WORD) { const uint2 r = reinterpret_cast<const uint2*>(w)[q]; id = r.x; of = r.y; }
     else if (REC == TW_REC4) { const uint32_t r = reinterpret_cast<const uint32_t*>(w)[q]; id = r & 0xFFFFu; of = r >> 16; }
     else if (REC == TW_REC_ID16) { id = reinterpret_cast<const uint16_t*>(w)[q]; of = 0; }
     else { id = reinterpret_cast<const uint32_t*>(w)[q]; of = 0; }
@@ -1123,7 +1139,7 @@ __device__ __forceinline__ void te_store(const EmitParams& p, const EmitOut& o, 
     constexpr uint32_t U = 4;
     const uint32_t lane = lane_id();
     if (!VEC) {
-        for (uint32_t k = lane; k < n; k += 32) { uint32_t id, of; te_rec<REC>(w, q0 + k, id, of); te_put<OUTS>(p, o, d0 + k, id, of, hs); }
+        for (uint32_t k = lane; k < n; k += 32) { uint32_t id, of; te_rec<REC>(w, q0 + k, id, of); te_put<OUTS, REC == TW_REC_WORD>(p, o, d0 + k, id, of, hs); }
         return;
     }
     const uint32_t head = (uint32_t)d0 & (U - 1u);          // slots of the first group before d0
@@ -1154,9 +1170,10 @@ __host__ __device__ constexpr bool te_staged() { return PLAIN && (OUTS == 7u || 
 
 // copies the stream tokens [j0, j1) of a slice whose run starts at stream position src to dst0 + (j - j0): window by
 // window, or with TE_U loads in flight per lane for the forms that are not staged
+// (wb: see te_put; TW_REC_WORD records are never staged)
 template <bool STAGED, uint32_t OUTS, int REC>
 __device__ __forceinline__ void te_copy(TeWindows<REC>& w, const void* tok, const EmitParams& p, const EmitOut& o, uint32_t src, uint32_t j0, uint32_t j1,
-                                        unsigned long long dst0, uint32_t hs = 0) {
+                                        unsigned long long dst0, uint32_t hs = 0, uint32_t wb = 0) {
     if (!STAGED) {
         const uint32_t lane = lane_id();
         constexpr int TE_U = 4;                     // B200, c2b 1 GiB: pass B 1.42 ms with 2, 1.25 ms with 4 or 8 (8-byte records)
@@ -1167,13 +1184,13 @@ __device__ __forceinline__ void te_copy(TeWindows<REC>& w, const void* tok, cons
 #pragma unroll
             for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) {
                 const size_t i = (size_t)src + j + 32 * u;
-                if (REC == TW_REC_WIDE) { const uint2 r = __ldg(static_cast<const uint2*>(tok) + i); id[u] = r.x; of[u] = r.y; }
+                if (REC == TW_REC_WIDE || REC == TW_REC_WORD) { const uint2 r = __ldg(static_cast<const uint2*>(tok) + i); id[u] = r.x; of[u] = r.y; }
                 else if (REC == TW_REC4) { const uint32_t r = __ldg(static_cast<const uint32_t*>(tok) + i); id[u] = r & 0xFFFFu; of[u] = r >> 16; }
                 else if (REC == TW_REC_ID16) id[u] = __ldg(static_cast<const uint16_t*>(tok) + i);
                 else id[u] = __ldg(static_cast<const uint32_t*>(tok) + i);
             }
 #pragma unroll
-            for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) te_put<OUTS>(p, o, dst0 + (j + 32 * u - j0), id[u], of[u], hs);
+            for (int u = 0; u < TE_U; u++) if (j + 32 * u < j1) te_put<OUTS, REC == TW_REC_WORD>(p, o, dst0 + (j + 32 * u - j0), id[u], of[u], hs, wb);
         }
         return;
     }
@@ -1189,7 +1206,7 @@ __device__ __forceinline__ void te_copy(TeWindows<REC>& w, const void* tok, cons
 
 // PLAIN = no truncation and no padding: the output is the plain concatenation of all tokens in text order, so a token's
 // destination is its global index.  Otherwise the tokens of the slice are cut by the documents that meet the slice.
-// REC: the token stream's record kind, as pass A wrote it.
+// REC: the token stream's record kind, as pass A wrote it (TW_REC_WORD: !PLAIN, OUTS = 0 only).
 // Staged forms: 4 blocks of 8 warps per SM (64 registers, no spill).  At 5 blocks (48 registers) and 6 (40) they spill, and
 // pass B measured 1.11 and 1.17 ms against 0.99 (B200, c2b 1 GiB): the windows in flight hide the loads without more warps.
 template <bool PLAIN, uint32_t OUTS, int REC>
@@ -1250,12 +1267,15 @@ __global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PL
             if (base_next == base) continue;
             const uint32_t lf = lg >> 3, ln = lg & 7u;
             const uint32_t d_first = d_lo ? d_lo - 1 : 0;
+            constexpr bool WID = REC == TW_REC_WORD;
+            const uint32_t swb = WID ? __ldg(a.slice_wordbase + s) : 0u;                    // global index of the slice's first word
             for (uint32_t dc = d_first; dc < d_hi && dc < a.n_docs; dc += 31) {
                 // lane l holds the token start of document dc + l (32 values: 31 documents and the end of the last one)
                 const uint32_t dl = dc + lane;
                 const uint32_t my_ds = dl <= a.n_docs ? __ldg(a.doc_tok_start + dl) : 0xFFFFFFFFu;
                 const unsigned long long my_dto = dl < a.n_docs ? a.doc_tok_off[dl] : 0ull;
                 const uint32_t my_dbyte = (p.hf_flags & 2u) && dl < a.n_docs ? (uint32_t)a.doc_off[dl] : 0u;     // hf_compat: byte position of the document
+                const uint32_t my_wb = WID && dl < a.n_docs ? swb - __ldg(a.doc_word_base + dl) : 0u;           // (mod 2^32) the slice's first word in the document
                 const uint32_t nd_here = min(31u, min(d_hi, a.n_docs) - dc);
                 for (uint32_t e = 0; e < nd_here; e++) {
                     const uint32_t ds = __shfl_sync(FULL, my_ds, e), dn = __shfl_sync(FULL, my_ds, e + 1);
@@ -1270,7 +1290,8 @@ __global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PL
                     const unsigned long long dbase = dto + shift;                                    // destination of the document's token 0
                     const uint32_t dbyte = __shfl_sync(FULL, my_dbyte, e);
                     const uint32_t hs = s * TW_SLICE - dbyte;                                        // (mod 2^32) slice start relative to the document
-                    if (ln == 0) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs);
+                    const uint32_t wb = WID ? __shfl_sync(FULL, my_wb, e) : 0u;
+                    if (ln == 0) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, g0 - base, g1 - base, dbase + (g0 - ds), hs, wb);
                     else {
                         // slice-local real index r = g - base; pieces as in the PLAIN case, cut to [g0, g1)
                         uint32_t j = 0, r = 0;
@@ -1278,7 +1299,7 @@ __global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PL
                             const uint32_t jn = i < ln ? __ldg(a.long_ins + lf + i) : ntok;
                             {   // inline piece: stream tokens [j, jn) = real indices [r, r + jn - j)
                                 const uint32_t lo = max(g0 - base, r), hi2 = min(g1 - base, r + (jn - j));
-                                if (lo < hi2) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs);
+                                if (lo < hi2) te_copy<STAGED, OUTS, REC>(w, a.tok, p, o, src, j + (lo - r), j + (hi2 - r), dbase + (base + lo - ds), hs, wb);
                             }
                             r += jn - j; j = jn;
                             if (i < ln) {
@@ -1291,8 +1312,9 @@ __global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PL
                                     const unsigned long long dd = dbase + (base + lo - ds);
                                     bool queued = false;
                                     const uint32_t ls = (p.hf_flags & 2u) ? sp - dbyte : 0u;         // the long word's start within its document
-                                    if (c2 > EMIT_BIG) { if (lane == 0) queued = big_push(a.big, sp2, c2, dd, ls); queued = __shfl_sync(FULL, queued, 0); }
-                                    if (!queued) for (uint32_t q = lane; q < c2; q += 32) emit_real(p, o, dd + q, a.pool_id[sp2 + q], a.pool_s[sp2 + q] + ls, a.pool_e[sp2 + q] + ls);
+                                    const uint32_t wid = WID ? wb + __ldg(a.long_k + lf + i) : 0u;
+                                    if (c2 > EMIT_BIG) { if (lane == 0) queued = big_push<WID>(a.big, sp2, c2, dd, ls, wid); queued = __shfl_sync(FULL, queued, 0); }
+                                    if (!queued) for (uint32_t q = lane; q < c2; q += 32) emit_real<WID>(p, o, dd + q, a.pool_id[sp2 + q], a.pool_s[sp2 + q] + ls, a.pool_e[sp2 + q] + ls, wid);
                                 }
                                 r += cnt;
                             }
@@ -1306,13 +1328,16 @@ __global__ void __launch_bounds__(TW_THREADS, te_staged<PLAIN, OUTS>() ? 4 : (PL
 }
 
 // per document: global token index of its start, real token count, output slot count (feeds the scan -> CSR offsets)
+// (word ids: global index of its first word, from the word base of its slice; doc_word_base == nullptr: not asked for)
 __global__ void doc_finish2_kernel(const uint64_t* __restrict__ doc_off, uint32_t n_docs, const uint32_t* __restrict__ tile_tokbase,
                                    const uint32_t* __restrict__ doc_tok_local, EmitParams p, uint32_t* __restrict__ doc_tok_start,
-                                   uint32_t* __restrict__ doc_real, unsigned long long* __restrict__ doc_tok_off) {
+                                   uint32_t* __restrict__ doc_real, unsigned long long* __restrict__ doc_tok_off,
+                                   const uint32_t* __restrict__ slice_wordbase, const uint32_t* __restrict__ doc_word_local, uint32_t* __restrict__ doc_word_base) {
     const uint32_t d = blockIdx.x * blockDim.x + threadIdx.x;
     if (d > n_docs) return;
     const uint32_t s0 = tile_tokbase[(uint32_t)(doc_off[d] / TW_SLICE)] + doc_tok_local[d];
     doc_tok_start[d] = s0;
+    if (doc_word_base) doc_word_base[d] = slice_wordbase[(uint32_t)(doc_off[d] / TW_SLICE)] + doc_word_local[d];
     if (d < n_docs) {
         const uint32_t s1 = tile_tokbase[(uint32_t)(doc_off[d + 1] / TW_SLICE)] + doc_tok_local[d + 1];
         const unsigned long long tr = s1 - s0;
@@ -1335,7 +1360,8 @@ __device__ __forceinline__ void warp_fill_u32(uint32_t* p, unsigned long long n,
     if (done + lane < n) p[done + lane] = v;
 }
 
-// padding slots from per-document real counts (src/encoding.zig:407-414, 418-425), one warp per document
+// padding slots from per-document real counts (src/encoding.zig:407-414, 418-425), one warp per document.  WID: word ids
+template <bool WID>
 __global__ void __launch_bounds__(256) emit_pad_real_kernel(EmitParams p, EmitOut o, uint32_t n_docs, const uint32_t* __restrict__ doc_real,
                                                             const unsigned long long* __restrict__ doc_tok_off) {
     const uint32_t d = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -1347,8 +1373,8 @@ __global__ void __launch_bounds__(256) emit_pad_real_kernel(EmitParams p, EmitOu
         // hf_compat: the template's special tokens around the kept tokens (lanes 0-3 prefix, 8-11 suffix)
         const uint32_t lane = lane_id();
         const unsigned long long b0 = doc_tok_off[d] + ((p.has_pad && p.pad_left) ? olen - full : 0);
-        if (lane < p.n_pre) emit_special(p, o, b0 + lane, p.pre_id[lane], p.pre_type[lane]);
-        if (lane >= 8 && lane - 8 < p.n_suf) emit_special(p, o, b0 + p.n_pre + kept + (lane - 8), p.suf_id[lane - 8], p.suf_type[lane - 8]);
+        if (lane < p.n_pre) emit_special<WID>(p, o, b0 + lane, p.pre_id[lane], p.pre_type[lane]);
+        if (lane >= 8 && lane - 8 < p.n_suf) emit_special<WID>(p, o, b0 + p.n_pre + kept + (lane - 8), p.suf_id[lane - 8], p.suf_type[lane - 8]);
     }
     if (olen == full) return;
     const unsigned long long base = doc_tok_off[d] + (p.pad_left ? 0 : full);
@@ -1361,9 +1387,11 @@ __global__ void __launch_bounds__(256) emit_pad_real_kernel(EmitParams p, EmitOu
     if (p.outputs & 16u) warp_fill_u32(o.special + base, npad, 1u);
     if (p.outputs & 32u) { uint16_t* q = o.offsets16 + base; for (unsigned long long i = lane_id(); i < npad; i += 32) q[i] = 0; }
     if (p.outputs & 128u) { uint4* q = o.spans + base; for (unsigned long long i = lane_id(); i < npad; i += 32) q[i] = make_uint4(p.pad_id, 0u, 0u, 0x0400u); }
+    if (WID) warp_fill_u32(o.word_ids + base, npad, TKZ_NONE);
 }
 
 // hf_compat: only the template's special tokens (the padding slots were filled array-wide), one thread per document
+template <bool WID>
 __global__ void __launch_bounds__(256) emit_frame_kernel(EmitParams p, EmitOut o, uint32_t n_docs, const uint32_t* __restrict__ doc_real,
                                                          const unsigned long long* __restrict__ doc_tok_off) {
     const uint32_t d = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1371,8 +1399,8 @@ __global__ void __launch_bounds__(256) emit_frame_kernel(EmitParams p, EmitOut o
     unsigned long long kept;
     const unsigned long long olen = doc_out_len(p, doc_real[d], &kept);
     const unsigned long long b0 = doc_tok_off[d] + ((p.has_pad && p.pad_left) ? olen - kept - tpl_added(p) : 0);
-    for (uint32_t i = 0; i < p.n_pre; i++) emit_special(p, o, b0 + i, p.pre_id[i], p.pre_type[i]);
-    for (uint32_t i = 0; i < p.n_suf; i++) emit_special(p, o, b0 + p.n_pre + kept + i, p.suf_id[i], p.suf_type[i]);
+    for (uint32_t i = 0; i < p.n_pre; i++) emit_special<WID>(p, o, b0 + i, p.pre_id[i], p.pre_type[i]);
+    for (uint32_t i = 0; i < p.n_suf; i++) emit_special<WID>(p, o, b0 + p.n_pre + kept + i, p.suf_id[i], p.suf_type[i]);
 }
 
 // document of the first failing word (byte position in the error word) -> ctrl[4]

@@ -29,6 +29,8 @@ pub const OUT_ALL: u32 = 31;
 pub const OUT_OFFSETS_PACKED: u32 = 32; // one u16 per token (start | end << 8) when every pre-token is < 256 bytes
 pub const OUT_IDS_U16: u32 = 64;
 pub const OUT_SPAN_TOKENS: u32 = 128; // 16-byte SpanToken records // ids as u16 when every vocabulary id is < 65536
+pub const OUT_WORD_IDS: u32 = 256; // each token's pre-token index in its document, WORD_NONE for specials and padding (not in OUT_ALL)
+pub const WORD_NONE: u32 = 0xFFFFFFFF;
 
 pub const ModelDesc = extern struct {
     model_kind: i32,
@@ -91,6 +93,7 @@ pub const BatchResult = extern struct {
     span_tokens: ?[*]const u32, // 4 u32 per slot = SpanToken (src/token.zig:19-33)
     n_wide: u64, // offsets_packed: tokens whose u16 is 0xFFFF (pre-tokens of 256+ bytes)
     wide_tokens: ?[*]const u32, // {slot low, slot high, start, end} each, sorted by slot in host-buffer results
+    word_ids: ?[*]const u32, // OUT_WORD_IDS: n_tokens entries
 };
 
 /// tkz_compact_result: kept real tokens only; masks and padding slots are rebuilt on the host (tkz_compact_expand)
