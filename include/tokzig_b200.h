@@ -116,7 +116,8 @@ typedef struct tkz_model_desc {
 #define TKZ_OUT_WORD_IDS 256u
 
 /* Per-call knobs = the public fields Tokenizer.truncation / Tokenizer.padding (src/lib.zig:41-42,149-157;
- * src/types.zig:39-45,55-59).  stride / strategy / pad_token are ignored by the reference's encode. */
+ * src/types.zig:39-45,55-59).  strategy / pad_token are ignored by the reference's encode, and so is stride unless the call
+ * sets TKZ_HF_OVERFLOW. */
 typedef struct tkz_encode_params {
     int32_t has_truncation;
     uint64_t max_length;                /* Encoding.truncate  src/encoding.zig:363-380 */
@@ -145,9 +146,19 @@ typedef struct tkz_encode_params {
     uint32_t tpl_n_prefix, tpl_n_suffix;             /* <= TKZ_TPL_MAX each */
     uint32_t tpl_prefix_id[4], tpl_prefix_type[4], tpl_suffix_id[4], tpl_suffix_type[4];
     uint32_t tpl_seq_type;
+    uint64_t stride;                    /* TruncationParams.stride (src/types.zig:55-59): read only with TKZ_HF_OVERFLOW */
 } tkz_encode_params;
 #define TKZ_HF_TEMPLATE 1u
 #define TKZ_HF_DOC_OFFSETS 2u
+/* Overflowing windows (Hugging Face Encoding.overflowing with right-side truncation): a document of n real tokens with
+ * n > L = max_length - (tpl_n_prefix + tpl_n_suffix under TKZ_HF_TEMPLATE) becomes 1 + ceil((n - L) / (L - stride)) rows, row k
+ * holding tokens [k * (L - stride), min(k * (L - stride) + L, n)); a document with n <= L is one row, exactly as without the flag.
+ * Every row gets the template's special tokens and its own padding; offsets and word ids are those of the document; as in
+ * tokenizers 0.22, tpl_seq_type goes to the tokens of a document's first row and its overflowing rows' tokens have type id 0.  Rows come in
+ * document order (tkz_batch_result.n_rows / row_tok_off / doc_row_off).  TKZ_ERR_INVALID_ARG without has_truncation, when L is 0
+ * or stride >= L, with `fast` or TKZ_OUT_SPAN_TOKENS, in the compact results, and when a call would have 2^32 rows or more.
+ * TKZ_OUT_OFFSETS_PACKED is delivered as TKZ_OUT_OFFSETS. */
+#define TKZ_HF_OVERFLOW 4u
 #define TKZ_TPL_MAX 4u
 
 /* CSR batch encoding = n_docs Encodings (src/encoding.zig:231-243) back to back.  Document d owns slots
@@ -175,6 +186,11 @@ typedef struct tkz_batch_result {
     uint64_t n_wide;
     const uint32_t* wide_tokens;
     const uint32_t* word_ids;           /* n_tokens, see TKZ_OUT_WORD_IDS; 0xFFFFFFFF for special tokens and padding */
+    /* TKZ_HF_OVERFLOW: row r owns slots [row_tok_off[r], row_tok_off[r+1]) and document d rows [doc_row_off[d], doc_row_off[d+1]);
+     * doc_tok_off[d] == row_tok_off[doc_row_off[d]].  Without the flag n_rows is 0 and both pointers are NULL. */
+    uint64_t n_rows;
+    const uint64_t* row_tok_off;        /* n_rows + 1 */
+    const uint64_t* doc_row_off;        /* n_docs + 1 */
 } tkz_batch_result;
 
 /* counters of the last encode (FastTokenizer.arenaMemoryUsage analogue, src/lib.zig:451-453) */
@@ -311,6 +327,8 @@ tkz_ctx* tkzh_ctx(tkzh_tokenizer* t);
 
 /* public fields truncation / padding  src/lib.zig:41-42 */
 int tkzh_set_truncation(tkzh_tokenizer* t, int has, uint64_t max_length);
+/* truncation.stride: the overlap of consecutive rows when hf_compat includes TKZ_HF_OVERFLOW (0 by default) */
+int tkzh_set_truncation_stride(tkzh_tokenizer* t, uint64_t stride);
 int tkzh_set_padding(tkzh_tokenizer* t, int has, int has_length, uint64_t length, uint32_t pad_id, uint32_t pad_type_id,
                      int pad_left);
 /* hand-wiring normalizer_impl / pretokenizer_impl (src/lib.zig:37-38): op lists, see TKZH_NORM_* / TKZH_PT_*.
@@ -352,8 +370,9 @@ int tkzh_id_to_token(tkzh_tokenizer* t, uint32_t id, const uint8_t** token, uint
 int tkzh_model_id_to_token(tkzh_tokenizer* t, uint32_t id, const uint8_t** token, uint64_t* len);
 /* hf_compat switch of the host mirror (TKZ_HF_* flags; 0 = the reference's behaviour, the default): with TKZ_HF_TEMPLATE the
  * single-sequence template of the tokenizer.json post_processor (BertProcessing, TemplateProcessing  specials* $A specials*)
- * is applied, its special tokens only when tkzh_encode_batch is called with add_special_tokens != 0.  Returns 1 when such a
- * template was found at load time, 0 when there is none to apply. */
+ * is applied, its special tokens only when tkzh_encode_batch is called with add_special_tokens != 0; with TKZ_HF_OVERFLOW a
+ * truncated document returns all its windows as rows (tkzh_set_truncation_stride).  Returns 1 when such a template was found
+ * at load time, 0 when there is none to apply. */
 int tkzh_set_hf_compat(tkzh_tokenizer* t, uint32_t flags);
 /* the template found at load time (arrays of TKZ_TPL_MAX entries; any pointer may be NULL): 1 and the outputs filled, or 0 */
 int tkzh_hf_template(tkzh_tokenizer* t, uint32_t* n_prefix, uint32_t* prefix_id, uint32_t* prefix_type, uint32_t* n_suffix,

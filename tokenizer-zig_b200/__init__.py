@@ -91,10 +91,11 @@ class EncodeParams(C.Structure):
         ("tpl_suffix_id", C.c_uint32 * 4),
         ("tpl_suffix_type", C.c_uint32 * 4),
         ("tpl_seq_type", C.c_uint32),
+        ("stride", C.c_uint64),
     ]
 
 
-HF_TEMPLATE, HF_DOC_OFFSETS = 1, 2
+HF_TEMPLATE, HF_DOC_OFFSETS, HF_OVERFLOW = 1, 2, 4
 
 
 class BatchResult(C.Structure):
@@ -115,6 +116,9 @@ class BatchResult(C.Structure):
         ("n_wide", C.c_uint64),
         ("wide_tokens", C.c_void_p),
         ("word_ids", C.c_void_p),
+        ("n_rows", C.c_uint64),
+        ("row_tok_off", C.c_void_p),
+        ("doc_row_off", C.c_void_p),
     ]
 
 
@@ -153,7 +157,7 @@ EXPORTED_SYMBOLS = [
     "tkz_ctx_numa_node", "tkzm_create", "tkzm_destroy", "tkzm_size", "tkzm_ctx", "tkzm_last_error", "tkzm_model_upload", "tkzm_shard_bounds",
     "tkzm_document_costs", "tkzm_encode_batch_compact",
     "tkz_encode_batch_device", "tkz_encode_batch_compact", "tkz_compact_slots", "tkz_compact_expand", "tkz_decode_upload", "tkz_decode_batch",
-    "tkzh_from_json", "tkzh_from_file", "tkzh_free", "tkzh_last_error", "tkzh_ctx", "tkzh_set_truncation", "tkzh_set_padding",
+    "tkzh_from_json", "tkzh_from_file", "tkzh_free", "tkzh_last_error", "tkzh_ctx", "tkzh_set_truncation", "tkzh_set_truncation_stride", "tkzh_set_padding",
     "tkzh_set_normalizer", "tkzh_set_pretokenizer", "tkzh_encode_batch", "tkzh_encode_batch_fast", "tkzh_decode", "tkzh_decode_batch", "tkzh_get_vocab_size", "tkzh_token_to_id",
     "tkzh_id_to_token", "tkzh_model_id_to_token", "tkzh_add_special_tokens", "tkzh_model_vocab_count", "tkzh_merge_count", "tkzh_has_normalizer",
     "tkzh_has_pretokenizer", "tkzh_has_post_processor", "tkzh_set_hf_compat", "tkzh_hf_template", "tkzh_added_token_count", "tkzh_added_token", "tkzh_model_desc",
@@ -205,6 +209,7 @@ def lib():
     L.tkzh_ctx.argtypes = [vp]
     L.tkzh_ctx.restype = vp
     L.tkzh_set_truncation.argtypes = [vp, i32, u64]
+    L.tkzh_set_truncation_stride.argtypes = [vp, u64]
     L.tkzh_set_hf_compat.argtypes = [vp, C.c_uint32]
     L.tkzh_set_hf_compat.restype = C.c_int
     L.tkzh_hf_template.argtypes = [vp] + [vp] * 7
@@ -283,6 +288,8 @@ class BatchEncoding:
     wide_tokens: Optional[np.ndarray] = None        # (n_wide, 4) u32: slot low, slot high, start, end -- tokens of pre-tokens of 256+ bytes
     span_tokens: Optional[np.ndarray] = None        # (n, 4) u32: id, start, end, type_id | flags << 8 (OUT_SPAN_TOKENS)
     word_ids: Optional[np.ndarray] = None           # u32 per slot: pre-token index in the document, WORD_NONE for specials / padding (OUT_WORD_IDS)
+    row_tok_off: Optional[np.ndarray] = None        # HF_OVERFLOW: row r owns slots [row_tok_off[r], row_tok_off[r+1])
+    doc_row_off: Optional[np.ndarray] = None        # HF_OVERFLOW: document d owns rows [doc_row_off[d], doc_row_off[d+1])
 
     def __len__(self):
         return len(self.doc_tok_off) - 1
@@ -302,6 +309,13 @@ class BatchEncoding:
     def doc_slice(self, i):
         return slice(int(self.doc_tok_off[i]), int(self.doc_tok_off[i + 1]))
 
+    @property
+    def overflow_to_sample_mapping(self) -> Optional[np.ndarray]:
+        """HF_OVERFLOW: the document of every row (transformers' overflow_to_sample_mapping)"""
+        if self.doc_row_off is None:
+            return None
+        return np.repeat(np.arange(len(self.doc_row_off) - 1, dtype=np.int64), np.diff(self.doc_row_off.astype(np.int64)))
+
 
 def _result_to_batch(r: BatchResult) -> BatchEncoding:
     T, n = int(r.n_tokens), int(r.n_docs)
@@ -318,6 +332,8 @@ def _result_to_batch(r: BatchResult) -> BatchEncoding:
         wide_tokens=_copy(r.wide_tokens, 4 * int(r.n_wide), np.uint32).reshape(-1, 4) if (r.wide_tokens and r.n_wide) else None,
         span_tokens=_copy(r.span_tokens, 4 * T, np.uint32).reshape(-1, 4) if r.span_tokens else None,
         word_ids=_copy(r.word_ids, T, np.uint32) if r.word_ids else None,
+        row_tok_off=_copy(r.row_tok_off, int(r.n_rows) + 1, np.uint64) if r.row_tok_off else None,
+        doc_row_off=_copy(r.doc_row_off, n + 1, np.uint64) if r.doc_row_off else None,
     )
 
 
@@ -425,7 +441,7 @@ class Tokenizer:
     def __init__(self, handle, L):
         self._h = handle
         self._L = L
-        self.truncation: Optional[dict] = None     # {"max_length": 512}          src/types.zig:55-59
+        self.truncation: Optional[dict] = None     # {"max_length": 512, "stride": 0}  src/types.zig:55-59 (stride: HF_OVERFLOW)
         self.padding: Optional[dict] = None        # {"length":..,"pad_id":..,"pad_type_id":..,"direction":"right"}  src/types.zig:39-45
 
     @classmethod
@@ -481,7 +497,7 @@ class Tokenizer:
     def set_hf_compat(self, flags: int) -> bool:
         """hf_compat (beyond the reference, off by default): HF_TEMPLATE applies the post_processor's single-sequence template
         (its special tokens only when encode is called with add_special_tokens), HF_DOC_OFFSETS reports document-relative
-        offsets.  Returns whether the tokenizer.json carried a template this mode can apply."""
+        offsets, HF_OVERFLOW returns every window of a truncated document as a row (truncation["stride"] tokens of overlap).  Returns whether the tokenizer.json carried a template this mode can apply."""
         rc = self._L.tkzh_set_hf_compat(self._h, int(flags))
         if rc < 0:
             raise TokzigError(rc, "tkzh_set_hf_compat", -1)
@@ -499,8 +515,10 @@ class Tokenizer:
     def _push_params(self):
         if self.truncation is None:
             self._L.tkzh_set_truncation(self._h, 0, 0)
+            self._L.tkzh_set_truncation_stride(self._h, 0)
         else:
             self._L.tkzh_set_truncation(self._h, 1, int(self.truncation.get("max_length", 512)))
+            self._L.tkzh_set_truncation_stride(self._h, int(self.truncation.get("stride", 0)))
         if self.padding is None:
             self._L.tkzh_set_padding(self._h, 0, 0, 0, 0, 0, 0)
         else:
@@ -525,6 +543,7 @@ class Tokenizer:
         p = EncodeParams()
         if self.truncation is not None:
             p.has_truncation, p.max_length = 1, int(self.truncation.get("max_length", 512))
+            p.stride = int(self.truncation.get("stride", 0))
         if self.padding is not None and self.padding.get("length") is not None:
             p.has_padding, p.pad_length = 1, int(self.padding["length"])
             p.pad_id, p.pad_type_id = int(self.padding.get("pad_id", 0)), int(self.padding.get("pad_type_id", 0))

@@ -25,6 +25,7 @@
 #include "tkz_decode.cuh"
 #include "tkz_emit.cuh"
 #include "tkz_fast.cuh"
+#include "tkz_overflow.cuh"
 #include "tkz_slices.cuh"
 #include "tkz_scan.cuh"
 #include "tkz_split.cuh"
@@ -60,8 +61,9 @@ struct tkz_ctx {
     // arenas (grow-only; replace src/arena.zig)
     DevBuf a_text, a_doc_off, a_norm_text, a_norm_doc_off, a_chunk, a_tiles, a_word_start, a_word_end, a_word_doc, a_doc_word_off,
         a_word_ntok, a_pool_id, a_pool_s, a_pool_e, a_pool_rk, a_scan_tmp, a_ctrl;
-    // output arrays, double-buffered so that the D2H copy of one chunk overlaps the kernels of the next (tkz_encode_batch)
-    struct OutSet { DevBuf doc_tok_off, ids, off, attn, type, special, off16, ids16, spans, wide, wid; } outs[2];
+    // output arrays, double-buffered so that the D2H copy of one chunk overlaps the kernels of the next (tkz_encode_batch); a
+    // third set stages the untruncated tokens that TKZ_HF_OVERFLOW cuts into rows (tkz_overflow.cuh)
+    struct OutSet { DevBuf doc_tok_off, ids, off, attn, type, special, off16, ids16, spans, wide, wid, row_tok_off, doc_row_off; } outs[3];
     int out_sel = 0;
     OutSet& O() { return outs[out_sel]; }
     DevBuf in_text[2], in_doc_off[2];
@@ -72,7 +74,8 @@ struct tkz_ctx {
     // slice pipeline arenas (tkz_slices.cuh)
     DevBuf a_long_start, a_long_end, a_long_ntok, a_long_slice, a_long_ins, a_tile_ntok, a_tile_ntok_inline, a_tile_tok_off, a_tile_long,
         a_doc_tok_local, a_doc_tok_start, a_doc_real, a_upool, a_tile_doc_lo, a_g_first, a_g_win, a_g_flag, a_big,
-        a_slice_nword, a_doc_word_local, a_doc_word_base, a_long_k;        // word ids (TKZ_OUT_WORD_IDS)
+        a_slice_nword, a_doc_word_local, a_doc_word_base, a_long_k,        // word ids (TKZ_OUT_WORD_IDS)
+        a_row_real, a_row_doc;                                             // overflowing windows (TKZ_HF_OVERFLOW)
     bool use_dedup = true;                // TKZ_NO_DEDUP=1: per-occurrence pipeline even with a pre-tokenizer (A/B switch of the parity tests)
     DevBuf a_wtable, a_lscratch, a_tok_id;
     bool has_iso = false;                 // the class table isolates some byte (punctuation split)
@@ -94,7 +97,7 @@ struct tkz_ctx {
     uint64_t tw_uniq_hist = 0;            // most unique words seen in one batch: sizes the next batch's word table
     uint64_t tw_upool_hist = 0;           // most token records used by one batch
     double tw_tok_per_byte = 0.0;         // densest batch so far: sizes the token stream
-    HostBuf h_ctrl, h_doc_tok_off, h_ids, h_off, h_attn, h_type, h_special, h_off16, h_ids16, h_spans, h_wide, h_wid;
+    HostBuf h_ctrl, h_doc_tok_off, h_ids, h_off, h_attn, h_type, h_special, h_off16, h_ids16, h_spans, h_wide, h_wid, h_row_tok_off, h_doc_row_off;
     DevBuf a_fast_heap, a_word_aux;       // FastTokenizer mode (tkz_fast.cuh)
     bool ids16_ok = false;                // every id the model can emit is below 65536 (TKZ_OUT_IDS_U16)
     uint32_t max_id = 0;                  // largest id the model can emit (word ids need it below 2^22: TW_REC_WORD)
@@ -317,15 +320,15 @@ extern "C" void tkz_ctx_destroy(tkz_ctx* ctx) {
                       &ctx->in_doc_off[1], &ctx->a_ctrl, &ctx->a_long_start, &ctx->a_long_end, &ctx->a_long_ntok, &ctx->a_long_slice, &ctx->a_long_ins,
                       &ctx->a_tile_ntok, &ctx->a_tile_ntok_inline, &ctx->a_tile_tok_off, &ctx->a_tile_long, &ctx->a_doc_tok_local,
                       &ctx->a_doc_tok_start, &ctx->a_doc_real, &ctx->a_upool, &ctx->a_tile_doc_lo, &ctx->a_g_first, &ctx->a_g_win, &ctx->a_g_flag, &ctx->a_big,
-                      &ctx->a_slice_nword, &ctx->a_doc_word_local, &ctx->a_doc_word_base, &ctx->a_long_k,
+                      &ctx->a_slice_nword, &ctx->a_doc_word_local, &ctx->a_doc_word_base, &ctx->a_long_k, &ctx->a_row_real, &ctx->a_row_doc,
                       &ctx->a_wtable, &ctx->a_lscratch, &ctx->a_tok_id, &ctx->a_fast_heap, &ctx->a_word_aux,
                       &ctx->a_huge_w, &ctx->a_huge_base, &ctx->a_huge_done, &ctx->a_grid_state, &ctx->a_grid_words,
                       &ctx->t_dec_bytes, &ctx->t_dec_off, &ctx->t_dec_special, &ctx->a_dec_ids, &ctx->a_dec_seq_off, &ctx->a_dec_len, &ctx->a_dec_raw,
                       &ctx->a_dec_out, &ctx->a_dec_olen, &ctx->a_dec_boff};
-    for (auto& os : ctx->outs) for (DevBuf* b : {&os.doc_tok_off, &os.ids, &os.off, &os.attn, &os.type, &os.special, &os.off16, &os.ids16, &os.spans, &os.wide, &os.wid}) release(*b);
+    for (auto& os : ctx->outs) for (DevBuf* b : {&os.doc_tok_off, &os.ids, &os.off, &os.attn, &os.type, &os.special, &os.off16, &os.ids16, &os.spans, &os.wide, &os.wid, &os.row_tok_off, &os.doc_row_off}) release(*b);
     for (DevBuf* b : bufs) release(*b);
     HostBuf* hb[] = {&ctx->h_ctrl, &ctx->h_doc_tok_off, &ctx->h_ids, &ctx->h_off, &ctx->h_attn, &ctx->h_type, &ctx->h_special, &ctx->h_off16, &ctx->h_ids16, &ctx->h_spans, &ctx->h_wide, &ctx->h_wid,
-                     &ctx->h_doc_stage[0], &ctx->h_doc_stage[1], &ctx->h_dec_bytes, &ctx->h_dec_off};
+                     &ctx->h_row_tok_off, &ctx->h_doc_row_off, &ctx->h_doc_stage[0], &ctx->h_doc_stage[1], &ctx->h_dec_bytes, &ctx->h_dec_off};
     for (HostBuf* b : hb) release_host(*b);
     if (ctx->s_h2d) cudaStreamDestroy(ctx->s_h2d);
     if (ctx->s_d2h) cudaStreamDestroy(ctx->s_d2h);
@@ -1173,6 +1176,70 @@ int encode_words(tkz_ctx* ctx, const DevModel& m, const uint8_t* d_text, const u
     return TKZ_OK;
 }
 
+// TKZ_HF_OVERFLOW (tkz_overflow.cuh): what a pipeline left in the staging output set (*out: every document's real tokens, no
+// truncation, padding or template) becomes rows of the call's output set, one per window.  P = the call's parameters.
+int encode_overflow(tkz_ctx* ctx, const tkz_encode_params& P, uint64_t launches, tkz_batch_result* out) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long* ctrl = (unsigned long long*)ctx->a_ctrl.p;
+    unsigned long long* hctrl = (unsigned long long*)ctx->h_ctrl.p;
+    const tkz_batch_result stage = *out;
+    const uint32_t nd = (uint32_t)stage.n_docs;
+    const unsigned long long* stage_off = (const unsigned long long*)stage.doc_tok_off;
+    const EmitParams ep = emit_params(P);
+    const uint64_t L = P.max_length - ((P.hf_flags & TKZ_HF_TEMPLATE) ? P.tpl_n_prefix + P.tpl_n_suffix : 0u), step = L - P.stride;
+    auto& O = ctx->O();
+    // ---- rows per document -> doc_row_off
+    TRY(ensure(ctx, O.doc_row_off, ((size_t)nd + 2) * 8));
+    TRY(ensure(ctx, ctx->a_scan_tmp, scan_tmp_elems(nd) * 8));
+    unsigned long long* doc_row_off = (unsigned long long*)O.doc_row_off.p;
+    if (nd) { ovf_doc_rows_kernel<<<(nd + 255) / 256, 256, 0, st>>>(stage_off, nd, L, step, doc_row_off, ctrl + 24); launches++; }
+    launches += exclusive_scan<unsigned long long>(doc_row_off, nd, doc_row_off, (unsigned long long*)ctx->a_scan_tmp.p, st);
+    TRY(readback(ctx, hctrl + 48, doc_row_off + nd, 8));
+    TRY(readback(ctx, hctrl + 49, ctrl + 24, 8));
+    CK(cudaStreamSynchronize(st));
+    const uint64_t R = hctrl[48], rows_real = hctrl[49];
+    // (the epilogue kernels index documents -- rows here -- with a u32)
+    if (R >= (1ull << 32)) { ctx->err = "overflowing windows: 2^32 rows or more in one call"; return TKZ_ERR_INVALID_ARG; }
+    const uint32_t nr = (uint32_t)R;
+    // ---- each row's document, window length and slots -> row_tok_off
+    TRY(ensure(ctx, O.row_tok_off, (R + 2) * 8));
+    TRY(ensure(ctx, ctx->a_row_real, (R + 2) * 4));
+    TRY(ensure(ctx, ctx->a_row_doc, (R + 2) * 4));
+    TRY(ensure(ctx, ctx->a_scan_tmp, scan_tmp_elems(R) * 8));
+    unsigned long long* row_tok_off = (unsigned long long*)O.row_tok_off.p;
+    const uint32_t* row_real = (const uint32_t*)ctx->a_row_real.p;
+    const uint32_t* row_doc = (const uint32_t*)ctx->a_row_doc.p;
+    if (nr) {
+        ovf_row_len_kernel<<<(nr + 255) / 256, 256, 0, st>>>(ep, stage_off, doc_row_off, nd, nr, L, step, row_tok_off, (uint32_t*)row_real, (uint32_t*)row_doc);
+        launches++;
+    }
+    launches += exclusive_scan<unsigned long long>(row_tok_off, R, row_tok_off, (unsigned long long*)ctx->a_scan_tmp.p, st);
+    TRY(readback(ctx, hctrl + 50, row_tok_off + R, 8));
+    CK(cudaStreamSynchronize(st));
+    const uint64_t T = hctrl[50];
+    // ---- the rows: windows, then the template's special tokens and the padding of the shared epilogue
+    TRY(ensure(ctx, O.doc_tok_off, ((size_t)nd + 1) * 8));
+    EmitOut eo;
+    TRY(alloc_outputs(ctx, ep, T, 0, eo));
+    const bool filled = pad_prologue(ctx, ep, eo, nr, T, rows_real, launches);
+    const OvfStage src{stage.ids, stage.ids16, (const uint2*)stage.offsets, stage.word_ids};
+    if (nr) {
+        const unsigned g = (unsigned)(((uint64_t)nr * 32 + 255) / 256);
+        if (ep.outputs & TKZ_OUT_WORD_IDS) ovf_copy_kernel<true><<<g, 256, 0, st>>>(ep, eo, src, nr, step, stage_off, doc_row_off, row_tok_off, row_real, row_doc);
+        else ovf_copy_kernel<false><<<g, 256, 0, st>>>(ep, eo, src, nr, step, stage_off, doc_row_off, row_tok_off, row_real, row_doc);
+        launches++;
+    }
+    unsigned long long* doc_tok_off = (unsigned long long*)O.doc_tok_off.p;
+    ovf_doc_off_kernel<<<(nd + 1 + 255) / 256, 256, 0, st>>>(doc_row_off, row_tok_off, nd, doc_tok_off); launches++;
+    pad_epilogue(ctx, ep, eo, nr, row_real, row_tok_off, filled, launches);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->ev[4], st));
+    CK(cudaStreamSynchronize(st));
+    finish(ctx, ep, eo, doc_tok_off, nd, T, stage.n_real_tokens, 0, launches, out);
+    out->n_rows = R; out->row_tok_off = (const uint64_t*)row_tok_off; out->doc_row_off = (const uint64_t*)doc_row_off;
+    return TKZ_OK;
+}
+
 int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_doc_off, uint64_t n_docs, uint64_t N,
                        const tkz_encode_params* params, tkz_batch_result* out) {
     memset(out, 0, sizeof *out);
@@ -1197,7 +1264,7 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
     }
     if (P.hf_flags) {
         // hf_compat (beyond the reference, opt-in)
-        if (P.hf_flags & ~(uint32_t)(TKZ_HF_TEMPLATE | TKZ_HF_DOC_OFFSETS)) { ctx->err = "unknown hf_flags bit"; return TKZ_ERR_INVALID_ARG; }
+        if (P.hf_flags & ~(uint32_t)(TKZ_HF_TEMPLATE | TKZ_HF_DOC_OFFSETS | TKZ_HF_OVERFLOW)) { ctx->err = "unknown hf_flags bit"; return TKZ_ERR_INVALID_ARG; }
         if (P.fast) { ctx->err = "hf_flags cannot be combined with the FastTokenizer mode"; return TKZ_ERR_INVALID_ARG; }
         if (P.tpl_n_prefix > TKZ_TPL_MAX || P.tpl_n_suffix > TKZ_TPL_MAX) { ctx->err = "at most TKZ_TPL_MAX special tokens on either side of the sequence"; return TKZ_ERR_INVALID_ARG; }
         if (!(P.hf_flags & TKZ_HF_TEMPLATE)) { P.tpl_n_prefix = P.tpl_n_suffix = 0; P.tpl_seq_type = 0; }
@@ -1206,6 +1273,14 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
                 if ((i < P.tpl_n_prefix && P.tpl_prefix_id[i] > 0xFFFFu) || (i < P.tpl_n_suffix && P.tpl_suffix_id[i] > 0xFFFFu)) { ctx->err = "template id above 65535 with TKZ_OUT_IDS_U16"; return TKZ_ERR_INVALID_ARG; }
         // document-relative offsets do not fit the one-u16-per-token form
         if ((P.hf_flags & TKZ_HF_DOC_OFFSETS) && (P.outputs & TKZ_OUT_OFFSETS_PACKED)) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
+        if (P.hf_flags & TKZ_HF_OVERFLOW) {
+            const uint64_t added = (P.hf_flags & TKZ_HF_TEMPLATE) ? P.tpl_n_prefix + P.tpl_n_suffix : 0u;
+            if (!P.has_truncation) { ctx->err = "overflowing windows need truncation"; return TKZ_ERR_INVALID_ARG; }
+            if (P.max_length <= added || P.stride >= P.max_length - added) { ctx->err = "overflowing windows need stride < max_length minus the template's tokens"; return TKZ_ERR_INVALID_ARG; }
+            if (P.outputs & TKZ_OUT_SPAN_TOKENS) { ctx->err = "overflowing windows do not carry span tokens"; return TKZ_ERR_INVALID_ARG; }
+            // (the windows are copied with their 32-bit offsets)
+            if (P.outputs & TKZ_OUT_OFFSETS_PACKED) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
+        }
     }
     if (P.outputs & TKZ_OUT_WORD_IDS) {
         if (P.fast) { ctx->err = "word ids cannot be combined with the FastTokenizer mode"; return TKZ_ERR_INVALID_ARG; }
@@ -1213,6 +1288,14 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
         if (ctx->max_id >= (1u << 22)) { ctx->err = "word ids need every id of the model below 2^22"; return TKZ_ERR_INVALID_ARG; }
     }
     if ((P.outputs & TKZ_OUT_IDS_U16) && (!ctx->ids16_ok || (P.has_padding && P.pad_id > 0xFFFFu))) P.outputs &= ~TKZ_OUT_IDS_U16;
+    // overflowing windows: the pipelines encode into the staging set with no truncation, padding or template tokens, and ask
+    // only for the arrays that differ per token (the document-offset shift stays theirs)
+    const bool overflow = (P.hf_flags & TKZ_HF_OVERFLOW) != 0;
+    tkz_encode_params S = P;
+    if (overflow) {
+        S.has_truncation = 0; S.has_padding = 0; S.hf_flags = P.hf_flags & TKZ_HF_DOC_OFFSETS;
+        S.outputs = TKZ_OUT_IDS | (P.outputs & (TKZ_OUT_IDS_U16 | TKZ_OUT_OFFSETS | TKZ_OUT_WORD_IDS));
+    }
     const uint32_t nd = (uint32_t)n_docs;
     DevModel m = ctx->dm;
 
@@ -1250,15 +1333,21 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
     // ---- slice pipeline (tkz_slices.cuh) whenever there is a pre-tokenizer; TKZ_NO_DEDUP=1 keeps the per-occurrence
     //      pipeline for A/B tests
     ctx->stats.path = 0;
+    const int out_sel = ctx->out_sel;
+    if (overflow) ctx->out_sel = 2;
+    int rc;
     if (m.has_pretok && ctx->use_dedup && !P.fast) {
         const ClassRanges& cr = ctx->dm.norm_has_drop ? ctx->cr_post : ctx->cr;      // (K0 ran: the text is already normalised)
-        int rc = encode_slices(ctx, m, cr, d_text, d_doc_off, nd, N, P, false, out, launches);
-        if (rc != TKZ_RETRY_WORST) return rc;
-        ctx->retried = true;
-        ctrl_reset_kernel<<<1, 1, 0, st>>>(ctrl); launches++;
-        return encode_slices(ctx, m, cr, d_text, d_doc_off, nd, N, P, true, out, launches);
-    }
-    return encode_words(ctx, m, d_text, d_doc_off, nd, N, P, out, launches);
+        rc = encode_slices(ctx, m, cr, d_text, d_doc_off, nd, N, S, false, out, launches);
+        if (rc == TKZ_RETRY_WORST) {
+            ctx->retried = true;
+            ctrl_reset_kernel<<<1, 1, 0, st>>>(ctrl); launches++;
+            rc = encode_slices(ctx, m, cr, d_text, d_doc_off, nd, N, S, true, out, launches);
+        }
+    } else rc = encode_words(ctx, m, d_text, d_doc_off, nd, N, S, out, launches);
+    ctx->out_sel = out_sel;
+    if (rc != TKZ_OK || !overflow) return rc;
+    return encode_overflow(ctx, P, launches, out);
 }
 
 }  // namespace
@@ -1314,6 +1403,7 @@ int encode_host_single(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_of
     int rc = encode_device_impl(ctx, (const uint8_t*)ctx->a_text.p, (const uint64_t*)ctx->a_doc_off.p, n_docs, N, params, &dev);
     *out = dev;
     set_result(out, dev.n_docs, dev.n_tokens, dev.n_real_tokens, nullptr, {}, 0, nullptr);    // (no device pointer leaves)
+    out->row_tok_off = out->doc_row_off = nullptr;
     if (rc != TKZ_OK) return rc;
     const uint64_t T = dev.n_tokens;
     cudaStream_t st = ctx->stream;
@@ -1330,6 +1420,13 @@ int encode_host_single(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_of
     if (dev.n_wide) {
         TRY(ensure_host(ctx, ctx->h_wide, dev.n_wide * 16));
         CK(cudaMemcpyAsync(ctx->h_wide.p, dev.wide_tokens, dev.n_wide * 16, cudaMemcpyDeviceToHost, st));
+    }
+    if (dev.n_rows) {
+        TRY(ensure_host(ctx, ctx->h_row_tok_off, (dev.n_rows + 1) * 8));
+        TRY(ensure_host(ctx, ctx->h_doc_row_off, (n_docs + 1) * 8));
+        CK(cudaMemcpyAsync(ctx->h_row_tok_off.p, dev.row_tok_off, (dev.n_rows + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(ctx->h_doc_row_off.p, dev.doc_row_off, (n_docs + 1) * 8, cudaMemcpyDeviceToHost, st));
+        out->row_tok_off = (const uint64_t*)ctx->h_row_tok_off.p; out->doc_row_off = (const uint64_t*)ctx->h_doc_row_off.p;
     }
     CK(cudaStreamSynchronize(st));
     if (dev.n_wide) wide_finish((WideRec*)ctx->h_wide.p, dev.n_wide, {});
@@ -1364,8 +1461,14 @@ int encode_host_chunked(tkz_ctx* ctx, const uint8_t* text, const uint64_t* doc_o
     if (params_in) P = *params_in;
     if (P.outputs == 0) P.outputs = TKZ_OUT_ALL;
     P.outputs |= TKZ_OUT_IDS;
+    // overflowing windows: a chunk never splits a document, so it never splits a document's rows either; row offsets are shifted
+    // by the chunk's slot base and document-row offsets by its row base, like doc_tok_off.  (Offsets come as 32-bit pairs.)
+    const bool overflow = (P.hf_flags & TKZ_HF_OVERFLOW) != 0;
+    if (overflow && (P.outputs & TKZ_OUT_OFFSETS_PACKED)) P.outputs = (P.outputs & ~TKZ_OUT_OFFSETS_PACKED) | TKZ_OUT_OFFSETS;
     TRY(ensure_host(ctx, ctx->h_doc_tok_off, (n_docs + 1) * 8));
     uint64_t* h_dto = (uint64_t*)ctx->h_doc_tok_off.p;
+    if (overflow) TRY(ensure_host(ctx, ctx->h_doc_row_off, (n_docs + 1) * 8));
+    uint64_t* h_dro = (uint64_t*)ctx->h_doc_row_off.p;
     auto stage_in = [&](size_t i) -> int {
         const int b = (int)(i & 1);
         const uint64_t d0 = cb[i], d1 = cb[i + 1], base = doc_off[d0], nb = doc_off[d1] - base, nd = d1 - d0;
@@ -1384,7 +1487,7 @@ restart:
     cb.resize(2); chunk_target = ctx->chunk_bytes; ctx->kept_valid = false; ctx->call_uniq = 0;
     uint64_t W_total = 0; std::vector<std::array<uint64_t, 3>> wide_parts;
     TRY(stage_in(0));
-    uint64_t T_total = 0, T_real = 0;
+    uint64_t T_total = 0, T_real = 0, R_total = 0;
     float ms_kernels = 0.f;
     for (size_t i = 0; cb[i] < n_docs; i++) {
         const int b = (int)(i & 1);
@@ -1426,10 +1529,16 @@ restart:
         // kernel-bound chunk (its device time exceeds what ~45 GB/s of PCIe needs for its text): larger chunks from now on
         if ((double)ctx->stats.ms_total * 1e-3 > (double)nb / 45e9 && chunk_target < chunk_max) chunk_target *= 2;
         const uint64_t T = dev.n_tokens;
-        // size the host arrays from the first chunk's token density
+        // size the host arrays from the first chunk's density of slots (rows: of rows)
         uint64_t est = T_total + T;
         if (i == 0 && nb) est = (uint64_t)((double)T * ((double)N / (double)nb) * 1.03) + 4096;
         if (est < T_total + T) est = T_total + T;
+        const uint64_t R = dev.n_rows;
+        if (overflow) {
+            uint64_t est_rows = R_total + R + 1;
+            if (i == 0 && nb) est_rows = std::max<uint64_t>(est_rows, (uint64_t)((double)R * ((double)N / (double)nb) * 1.03) + 4096);
+            TRY(ensure_host_keep(ctx, ctx->h_row_tok_off, est_rows * 8, R_total * 8));
+        }
         // (every chunk delivers the same arrays: they depend on the model and the parameters)
         const auto cp = result_copies(ctx, dev);
         for (uint32_t k = 0; k < N_RESULT_ARRAYS; k++) {
@@ -1448,8 +1557,14 @@ restart:
         // chunk-relative CSR offsets -> call-relative on the device (same stream as the copy; the chunk's kernels have finished)
         if (T_total) add_base_u64_kernel<<<(unsigned)((nd + 1 + 255) / 256), 256, 0, ctx->s_d2h>>>((unsigned long long*)dev.doc_tok_off, nd + 1, T_total);
         CK(cudaMemcpyAsync(h_dto + d0, dev.doc_tok_off, (nd + 1) * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        if (overflow) {
+            if (T_total) add_base_u64_kernel<<<(unsigned)((R + 1 + 255) / 256), 256, 0, ctx->s_d2h>>>((unsigned long long*)dev.row_tok_off, R + 1, T_total);
+            if (R_total) add_base_u64_kernel<<<(unsigned)((nd + 1 + 255) / 256), 256, 0, ctx->s_d2h>>>((unsigned long long*)dev.doc_row_off, nd + 1, R_total);
+            CK(cudaMemcpyAsync((uint64_t*)ctx->h_row_tok_off.p + R_total, dev.row_tok_off, (R + 1) * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+            CK(cudaMemcpyAsync(h_dro + d0, dev.doc_row_off, (nd + 1) * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        }
         CK(cudaEventRecord(ctx->ev_d2h[b], ctx->s_d2h));
-        T_total += T; T_real += dev.n_real_tokens;
+        T_total += T; T_real += dev.n_real_tokens; R_total += R;
     }
     CK(cudaStreamSynchronize(ctx->s_d2h));
     CK(cudaStreamSynchronize(ctx->s_h2d));
@@ -1458,6 +1573,10 @@ restart:
     ctx->out_sel = 0;
     ctx->stats.ms_call_kernels = ms_kernels;
     set_result(out, n_docs, T_total, T_real, h_dto, host, W_total, ctx->h_wide.p);
+    if (overflow) {
+        ((uint64_t*)ctx->h_row_tok_off.p)[R_total] = T_total; h_dro[n_docs] = R_total;
+        out->n_rows = R_total; out->row_tok_off = (const uint64_t*)ctx->h_row_tok_off.p; out->doc_row_off = h_dro;
+    }
     return TKZ_OK;
 }
 

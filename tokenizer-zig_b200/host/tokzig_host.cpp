@@ -73,7 +73,7 @@ struct tkzh_tokenizer {
     int decoder_kind = 0;
     std::vector<AddedToken> added_tokens;
     SideVocab added_vocab;
-    bool has_trunc = false; uint64_t max_length = 512;
+    bool has_trunc = false; uint64_t max_length = 512; uint64_t stride = 0;
     bool has_pad = false; bool pad_has_length = false; uint64_t pad_length = 0; uint32_t pad_id = 0, pad_type_id = 0; bool pad_left = false;
     // flattened
     std::vector<uint8_t> vocab_bytes; std::vector<uint64_t> vocab_off;
@@ -354,6 +354,10 @@ extern "C" int tkzh_set_truncation(tkzh_tokenizer* t, int has, uint64_t max_leng
     if (!t) return TKZ_ERR_INVALID_ARG;
     t->has_trunc = has != 0; t->max_length = max_length; return TKZ_OK;
 }
+extern "C" int tkzh_set_truncation_stride(tkzh_tokenizer* t, uint64_t stride) {
+    if (!t) return TKZ_ERR_INVALID_ARG;
+    t->stride = stride; return TKZ_OK;
+}
 extern "C" int tkzh_set_padding(tkzh_tokenizer* t, int has, int has_length, uint64_t length, uint32_t pad_id, uint32_t pad_type_id, int pad_left) {
     if (!t) return TKZ_ERR_INVALID_ARG;
     t->has_pad = has != 0; t->pad_has_length = has_length != 0; t->pad_length = length; t->pad_id = pad_id; t->pad_type_id = pad_type_id; t->pad_left = pad_left != 0;
@@ -385,7 +389,8 @@ extern "C" int tkzh_encode_batch(tkzh_tokenizer* t, const uint8_t* text, const u
     p.has_truncation = t->has_trunc; p.max_length = t->max_length;                // lib.zig:150-152
     p.has_padding = t->has_pad && t->pad_has_length; p.pad_length = t->pad_length; // lib.zig:155-157, encoding.zig:386
     p.pad_id = t->pad_id; p.pad_type_id = t->pad_type_id; p.pad_left = t->pad_left; p.outputs = outputs;
-    p.hf_flags = t->hf_flags & TKZ_HF_DOC_OFFSETS;
+    p.hf_flags = t->hf_flags & (TKZ_HF_DOC_OFFSETS | TKZ_HF_OVERFLOW);
+    p.stride = t->stride;
     if ((t->hf_flags & TKZ_HF_TEMPLATE) && t->has_template) {
         p.hf_flags |= TKZ_HF_TEMPLATE; p.tpl_seq_type = t->tpl_seq_type;
         if (add_special_tokens) {
@@ -519,7 +524,7 @@ extern "C" int tkzh_hf_template(tkzh_tokenizer* t, uint32_t* n_prefix, uint32_t*
 }
 extern "C" int tkzh_set_hf_compat(tkzh_tokenizer* t, uint32_t flags) {
     if (!t) return TKZ_ERR_INVALID_ARG;
-    t->hf_flags = flags & (TKZ_HF_TEMPLATE | TKZ_HF_DOC_OFFSETS);
+    t->hf_flags = flags & (TKZ_HF_TEMPLATE | TKZ_HF_DOC_OFFSETS | TKZ_HF_OVERFLOW);
     return t->has_template ? 1 : 0;
 }
 extern "C" uint64_t tkzh_added_token_count(tkzh_tokenizer* t) { return t->added_tokens.size(); }

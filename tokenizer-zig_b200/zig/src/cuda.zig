@@ -65,7 +65,7 @@ pub const EncodeParams = extern struct {
     fast_max_sequence_length: u32 = 0, // 0 = 8192
     fast_max_tokens: u32 = 0, // 0 = 512
     // hf_compat (beyond the reference, opt-in; 0 = reference behaviour): single-sequence template + document-relative offsets
-    hf_flags: u32 = 0, // HF_TEMPLATE | HF_DOC_OFFSETS
+    hf_flags: u32 = 0, // HF_TEMPLATE | HF_DOC_OFFSETS | HF_OVERFLOW
     tpl_n_prefix: u32 = 0,
     tpl_n_suffix: u32 = 0,
     tpl_prefix_id: [4]u32 = .{ 0, 0, 0, 0 },
@@ -73,9 +73,11 @@ pub const EncodeParams = extern struct {
     tpl_suffix_id: [4]u32 = .{ 0, 0, 0, 0 },
     tpl_suffix_type: [4]u32 = .{ 0, 0, 0, 0 },
     tpl_seq_type: u32 = 0,
+    stride: u64 = 0, // TruncationParams.stride: overlap of consecutive rows, read only with HF_OVERFLOW
 };
 pub const HF_TEMPLATE: u32 = 1;
 pub const HF_DOC_OFFSETS: u32 = 2;
+pub const HF_OVERFLOW: u32 = 4; // every window of a truncated document as a row of its own
 
 pub const BatchResult = extern struct {
     n_docs: u64,
@@ -94,6 +96,9 @@ pub const BatchResult = extern struct {
     n_wide: u64, // offsets_packed: tokens whose u16 is 0xFFFF (pre-tokens of 256+ bytes)
     wide_tokens: ?[*]const u32, // {slot low, slot high, start, end} each, sorted by slot in host-buffer results
     word_ids: ?[*]const u32, // OUT_WORD_IDS: n_tokens entries
+    n_rows: u64, // HF_OVERFLOW: rows of the call; 0 without it
+    row_tok_off: ?[*]const u64, // HF_OVERFLOW: n_rows + 1, row r owns slots [row_tok_off[r], row_tok_off[r+1])
+    doc_row_off: ?[*]const u64, // HF_OVERFLOW: n_docs + 1, document d owns rows [doc_row_off[d], doc_row_off[d+1])
 };
 
 /// tkz_compact_result: kept real tokens only; masks and padding slots are rebuilt on the host (tkz_compact_expand)
@@ -106,7 +111,7 @@ pub const CompactResult = extern struct {
     ids16: ?[*]const u16,
     offsets_packed: ?[*]const u16, // 0xFFFF = look the token up in wide_tokens; null when the call fell back to `offsets`
     offsets: ?[*]const u32,
-    params: EncodeParams,
+    params: EncodeParams, // (its stride moves the fields below)
     err_doc: i64,
     n_wide: u64,
     wide_tokens: ?[*]const u32, // {kept index low, high, start, end}, sorted by kept index
