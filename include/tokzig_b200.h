@@ -99,7 +99,7 @@ typedef struct tkz_model_desc {
  * or more get the value 0xFFFF (no real token has start = end = 255) and their offsets travel in a side list
  * (tkz_batch_result.n_wide / wide_tokens).  A batch where those tokens are many (above an eighth of all tokens or 4 M), a
  * tokenizer without pre-tokenizer, and TKZ_HF_DOC_OFFSETS fall back to TKZ_OUT_OFFSETS for the whole call: exactly one of
- * offsets / offsets_packed is then non-NULL. */
+ * offsets / offsets_packed is then non-NULL.  Padding slots and the template's special tokens (TKZ_HF_TEMPLATE) are 0. */
 #define TKZ_OUT_OFFSETS_PACKED 32u
 /* Ids as u16 in tkz_batch_result.ids16 instead of u32 in ids: honoured when every id of the uploaded vocabulary is below
  * 65536 (GPT-2- and BERT-sized vocabularies), ignored otherwise: exactly one of ids / ids16 is non-NULL. */
@@ -176,7 +176,7 @@ typedef struct tkz_batch_result {
     const uint32_t* type_ids;
     const uint32_t* special_tokens_mask;
     int64_t err_doc;                    /* document index of the first error, -1 if none */
-    const uint16_t* offsets_packed;     /* n_tokens x (start | end << 8), see TKZ_OUT_OFFSETS_PACKED; padding slots are 0 */
+    const uint16_t* offsets_packed;     /* n_tokens x (start | end << 8), see TKZ_OUT_OFFSETS_PACKED; padding and template slots are 0 */
     const uint16_t* ids16;              /* n_tokens, see TKZ_OUT_IDS_U16 */
     const uint32_t* span_tokens;        /* 4 u32 per slot, see TKZ_OUT_SPAN_TOKENS */
     /* TKZ_OUT_OFFSETS_PACKED, tokens of pre-tokens of 256 bytes or more: their u16 is 0xFFFF and their offsets are here,

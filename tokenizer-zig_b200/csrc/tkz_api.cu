@@ -1262,6 +1262,8 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
         if (P.fast_max_sequence_length < 4 || P.fast_max_sequence_length > 65535) { ctx->err = "fast_max_sequence_length must be 4 .. 65535 (16-bit symbol indices, arena.zig:17-42)"; return TKZ_ERR_INVALID_ARG; }
         P.has_truncation = 1; P.max_length = P.fast_max_tokens; P.has_padding = 0;
     }
+    // (before the template's ids are checked against the u16 form: a vocabulary with larger ids ignores it)
+    if ((P.outputs & TKZ_OUT_IDS_U16) && (!ctx->ids16_ok || (P.has_padding && P.pad_id > 0xFFFFu))) P.outputs &= ~TKZ_OUT_IDS_U16;
     if (P.hf_flags) {
         // hf_compat (beyond the reference, opt-in)
         if (P.hf_flags & ~(uint32_t)(TKZ_HF_TEMPLATE | TKZ_HF_DOC_OFFSETS | TKZ_HF_OVERFLOW)) { ctx->err = "unknown hf_flags bit"; return TKZ_ERR_INVALID_ARG; }
@@ -1287,7 +1289,6 @@ int encode_device_impl(tkz_ctx* ctx, const uint8_t* d_text, const uint64_t* d_do
         // (the slice pipeline's token records keep the word's index in the slice above a 22-bit id)
         if (ctx->max_id >= (1u << 22)) { ctx->err = "word ids need every id of the model below 2^22"; return TKZ_ERR_INVALID_ARG; }
     }
-    if ((P.outputs & TKZ_OUT_IDS_U16) && (!ctx->ids16_ok || (P.has_padding && P.pad_id > 0xFFFFu))) P.outputs &= ~TKZ_OUT_IDS_U16;
     // overflowing windows: the pipelines encode into the staging set with no truncation, padding or template tokens, and ask
     // only for the arrays that differ per token (the document-offset shift stays theirs)
     const bool overflow = (P.hf_flags & TKZ_HF_OVERFLOW) != 0;

@@ -97,6 +97,7 @@ template <bool WID = false>
 __device__ __forceinline__ void emit_special(const EmitParams& p, const EmitOut& o, unsigned long long dst, uint32_t id, uint32_t ty) {
     emit_id(p, o, dst, id);
     if (p.outputs & 2u) reinterpret_cast<uint2*>(o.offsets)[dst] = make_uint2(0u, 0u);
+    if (p.outputs & 32u) o.offsets16[dst] = 0;
     if (p.outputs & 4u) o.attention[dst] = 1u;
     if (p.outputs & 8u) o.type_ids[dst] = ty;
     if (p.outputs & 16u) o.special[dst] = 1u;
